@@ -442,6 +442,25 @@ int ledb200_stack_pad(const void* img, int32_t img_dtype, int32_t h, int32_t w, 
                       const float* std3, float pad_val, float* out, int32_t Hp, int32_t Wp, const void* label,
                       int32_t label_dtype, int64_t* label_out, int32_t seg_pad_val, void* stream);
 
+/* ledb200_tta_merge: SegTTAModel.merge_preds (mmseg/models/segmentors/seg_tta.py) over V views of N images in ONE launch.
+ *   views (HOST array, 1 <= V <= 32, in the augmentation list order): image n of view v is the fp32 [K,H,W] plane stack at
+ *   logits + n * image_stride (elements); pad_lrtb / flip (0 none, 1 horizontal, 2 vertical) are that view's padding to
+ *   remove and flip to undo.  Per output pixel of [oh, ow] and per view, the value of class k is exactly what
+ *   ledb200_postprocess writes to out_logits for that view (same source taps and lerp); then mode 0 (out_channels > 1):
+ *   softmax over K, mode 1 (out_channels == 1): sigmoid per class, summed over the views in order in fp32 registers
+ *   (shared memory for K > 32) and divided by V.  pred: mode 0 argmax over K (first max) [N,oh,ow] U8 or I64; mode 1
+ *   (merged > threshold) as F32 [N,K,oh,ow].  probs_opt (nullable): the merged fp32 [N,K,oh,ow].  1 <= K <= 255. */
+typedef struct {
+  const float* logits;
+  int64_t image_stride;
+  int32_t H, W;
+  int32_t pad_lrtb[4];
+  int32_t flip;
+} ledb200_tta_view;
+int ledb200_tta_merge(const ledb200_tta_view* views, int32_t V, int32_t N, int32_t K, int32_t oh, int32_t ow,
+                      int32_t align_corners, int32_t mode, float threshold, void* pred, int32_t pred_dtype,
+                      float* probs_opt, void* stream);
+
 /* ---- layer-level operators for module compositions outside the R0 plan (the LED wiring, led_variant.py) ---------------
  * A conv layer handle is ONE mmcv ConvModule (mmcv/cnn/bricks/conv_module.py; conv k = 1 | 3, stride 1 | 2, padding k/2)
  * whose BatchNorm the caller folded into `weight` (OIHW, HOST fp32) / `bias` (nullable); `pre_scale` / `pre_shift`

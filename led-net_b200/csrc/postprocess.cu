@@ -13,10 +13,15 @@
 //  * slide_merge : the same for ALL crops at once (they ran as one batch of the engine): per output pixel the crops that
 //      cover it are summed in the reference's grid order (fp32, starting from 0: bit-identical to the sequential
 //      `preds +=`), divided by their number, and optionally arg-maxed - no full-size read-modify-write per crop.
+//  * tta_merge : SegTTAModel.merge_preds (mmseg/models/segmentors/seg_tta.py) for every view of a batch at once: per output
+//      pixel each view is sampled through postprocess_kernel's own geometry (un-pad, un-flip, resize), soft-maxed (or
+//      sigmoid-ed) over K and summed in view order in registers; then / V and argmax (or > threshold).  Only the labels
+//      (and, on request, the merged probabilities) reach memory.
 //  * stack_pad : SegDataPreProcessor.forward + stack_batch for one sample (mmseg/models/data_preprocessor.py:112-149,
 //      mmseg/utils/misc.py:30-128): BGR<->RGB swap, float, (x - mean) / std, right / bottom padding with `pad_val`
 //      (applied AFTER the normalisation, as the reference does), label map padded with `seg_pad_val`.
 // All tensors are the reference's NCHW fp32; one thread per output pixel, consecutive threads on consecutive x.
+#include <type_traits>
 #include <vector>
 
 #include "kernels.h"
@@ -24,13 +29,37 @@
 namespace ledb {
 namespace {
 
+// The geometry of one post-processed view: stored [K, H, W] logits, the padding to remove, the flip to undo and the
+// ATen resize scales from the cropped extent [ch, cw] to the output size.  Shared by postprocess_kernel and
+// tta_merge_kernel, so a merged view samples exactly the values ledb200_postprocess writes for it.
+struct ViewGeom {
+  int H, W;
+  int pl, pt;            // left / top padding (right / bottom only shorten the cropped extent)
+  int ch, cw;            // cropped extent
+  int flip;              // 0 none, 1 horizontal, 2 vertical
+  float sy, sx;          // ATen scales
+};
+
+// false when the padding is negative or removes the whole image
+bool make_geom(int H, int W, const int32_t* pad_lrtb, int flip, int oh, int ow, int align_corners, ViewGeom& g) {
+  const int pl = pad_lrtb ? pad_lrtb[0] : 0, pr = pad_lrtb ? pad_lrtb[1] : 0;
+  const int pt = pad_lrtb ? pad_lrtb[2] : 0, pb = pad_lrtb ? pad_lrtb[3] : 0;
+  g.H = H; g.W = W; g.pl = pl; g.pt = pt; g.ch = H - pt - pb; g.cw = W - pl - pr; g.flip = flip;
+  if (pl < 0 || pr < 0 || pt < 0 || pb < 0 || g.ch < 1 || g.cw < 1) return false;
+  if (align_corners) {
+    g.sy = oh > 1 ? (float)(g.ch - 1) / (float)(oh - 1) : 0.f;
+    g.sx = ow > 1 ? (float)(g.cw - 1) / (float)(ow - 1) : 0.f;
+  } else {
+    g.sy = (float)g.ch / (float)oh; g.sx = (float)g.cw / (float)ow;
+  }
+  return true;
+}
+
 struct PostArgs {
   const float* logits;   // [K, H, W] of one image
-  int K, H, W;
-  int pl, pr, pt, pb;    // padding to remove
-  int flip;              // 0 none, 1 horizontal, 2 vertical
+  int K;
+  ViewGeom g;
   int oh, ow, align_corners;
-  float sy, sx;          // ATen scales
   float threshold;       // C == 1
   void* pred; int pred_dtype;
   float* out_logits;     // optional [K, oh, ow]
@@ -48,35 +77,191 @@ __device__ __forceinline__ void src_index(int dst, float scale, int in_size, int
   }
 }
 
+// the four source taps of output pixel (oy, ox) in the stored logits, and the lerp weights
+struct Taps {
+  int64_t o00, o01, o10, o11;
+  float ly, lx;
+};
+
+__device__ __forceinline__ Taps view_taps(const ViewGeom& g, int oy, int ox, int align_corners) {
+  int y0, y1, x0, x1;
+  Taps t;
+  src_index(oy, g.sy, g.ch, align_corners, y0, y1, t.ly);
+  src_index(ox, g.sx, g.cw, align_corners, x0, x1, t.lx);
+  // cropped (and flipped) coordinates -> coordinates of the stored logits
+  if (g.flip == 1) { x0 = g.cw - 1 - x0; x1 = g.cw - 1 - x1; }
+  if (g.flip == 2) { y0 = g.ch - 1 - y0; y1 = g.ch - 1 - y1; }
+  t.o00 = (int64_t)(y0 + g.pt) * g.W + x0 + g.pl; t.o01 = (int64_t)(y0 + g.pt) * g.W + x1 + g.pl;
+  t.o10 = (int64_t)(y1 + g.pt) * g.W + x0 + g.pl; t.o11 = (int64_t)(y1 + g.pt) * g.W + x1 + g.pl;
+  return t;
+}
+
+// postprocess_result's value of one class plane `p` at the taps (sigmoid applied when K == 1, base.py:190)
+__device__ __forceinline__ float view_value(const float* p, const Taps& t, int K) {
+  const float hy = 1.f - t.ly, hx = 1.f - t.lx;
+  // ATen upsample_bilinear2d: h0lambda * (w0lambda * v00 + w1lambda * v01) + h1lambda * (w0lambda * v10 + w1lambda * v11)
+  float v = hy * (hx * __ldg(p + t.o00) + t.lx * __ldg(p + t.o01)) + t.ly * (hx * __ldg(p + t.o10) + t.lx * __ldg(p + t.o11));
+  if (K == 1) v = 1.f / (1.f + __expf(-v));
+  return v;
+}
+
 template <typename TP>
 __global__ void __launch_bounds__(256) postprocess_kernel(PostArgs a) {
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= (int64_t)a.oh * a.ow) return;
   const int ox = (int)(idx % a.ow), oy = (int)(idx / a.ow);
-  const int ch = a.H - a.pt - a.pb, cw = a.W - a.pl - a.pr;       // cropped extent
-  int y0, y1, x0, x1;
-  float ly, lx;
-  src_index(oy, a.sy, ch, a.align_corners, y0, y1, ly);
-  src_index(ox, a.sx, cw, a.align_corners, x0, x1, lx);
-  // cropped (and flipped) coordinates -> coordinates of the stored logits
-  if (a.flip == 1) { x0 = cw - 1 - x0; x1 = cw - 1 - x1; }
-  if (a.flip == 2) { y0 = ch - 1 - y0; y1 = ch - 1 - y1; }
-  const int64_t o00 = (int64_t)(y0 + a.pt) * a.W + x0 + a.pl, o01 = (int64_t)(y0 + a.pt) * a.W + x1 + a.pl;
-  const int64_t o10 = (int64_t)(y1 + a.pt) * a.W + x0 + a.pl, o11 = (int64_t)(y1 + a.pt) * a.W + x1 + a.pl;
-  const float hy = 1.f - ly, hx = 1.f - lx;
+  const Taps t = view_taps(a.g, oy, ox, a.align_corners);
   float best = -INFINITY;
   int bi = 0;
   float v = 0.f;
   for (int k = 0; k < a.K; ++k) {
-    const float* p = a.logits + (int64_t)k * a.H * a.W;
-    // ATen upsample_bilinear2d: h0lambda * (w0lambda * v00 + w1lambda * v01) + h1lambda * (w0lambda * v10 + w1lambda * v11)
-    v = hy * (hx * __ldg(p + o00) + lx * __ldg(p + o01)) + ly * (hx * __ldg(p + o10) + lx * __ldg(p + o11));
-    if (a.K == 1) v = 1.f / (1.f + __expf(-v));
+    v = view_value(a.logits + (int64_t)k * a.g.H * a.g.W, t, a.K);
     if (a.out_logits) a.out_logits[(int64_t)k * a.oh * a.ow + idx] = v;
     if (v > best) { best = v; bi = k; }                           // strict >: torch.argmax's first-max rule
   }
   TP* pred = reinterpret_cast<TP*>(a.pred);
   if (pred) pred[idx] = (TP)(a.K == 1 ? (v > a.threshold ? 1 : 0) : bi);
+}
+
+// ---- tta_merge: SegTTAModel.merge_preds over every view of a batch -----------------------------------------------
+constexpr int kMaxViews = 32;
+struct TtaView {
+  const float* logits;   // image n at logits + n * image_stride
+  int64_t image_stride;
+  ViewGeom g;
+};
+struct TtaArgs {
+  TtaView v[kMaxViews];
+  int V, N, K, oh, ow, align_corners;
+  float threshold;       // sigmoid mode
+  void* pred;            // softmax mode: labels [N, oh, ow]; sigmoid mode: float mask [N, K, oh, ow]
+  float* probs;          // optional merged [N, K, oh, ow]
+};
+
+__device__ __forceinline__ float sigmoid_ref(float v) { return 1.f / (1.f + expf(-v)); }
+
+// Both paths: TP == float selects the sigmoid mode (out_channels == 1), whose prediction is the float mask
+// (logits > threshold).to(logits) of [N, K, oh, ow]; otherwise TP is the label type of argmax(dim=0).
+
+// Register path, K <= KT: one thread per output pixel, the per-class accumulator and the view's values in registers.
+// EXACT: K == KT (no per-class guards).
+template <int KT, bool EXACT, typename TP>
+__global__ void __launch_bounds__(256) tta_merge_kernel(const __grid_constant__ TtaArgs a) {
+  constexpr bool kSigmoid = std::is_same<TP, float>::value;
+  const int K = EXACT ? KT : a.K;
+  const int64_t OHW = (int64_t)a.oh * a.ow;
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (int64_t)a.N * OHW) return;
+  const int n = (int)(idx / OHW);
+  const int64_t pix = idx % OHW;
+  const int oy = (int)(pix / a.ow), ox = (int)(pix % a.ow);
+  float acc[KT];
+#pragma unroll
+  for (int k = 0; k < KT; ++k) acc[k] = 0.f;                     // logits = zeros_like(views[0])
+  for (int i = 0; i < a.V; ++i) {
+    const TtaView& vw = a.v[i];
+    const Taps t = view_taps(vw.g, oy, ox, a.align_corners);
+    const float* base = vw.logits + (int64_t)n * vw.image_stride;
+    const int64_t plane = (int64_t)vw.g.H * vw.g.W;
+    float v[KT];
+    float m = -INFINITY;
+#pragma unroll
+    for (int k = 0; k < KT; ++k)
+      if (EXACT || k < K) { v[k] = view_value(base + k * plane, t, K); m = fmaxf(m, v[k]); }
+    if constexpr (kSigmoid) {
+#pragma unroll
+      for (int k = 0; k < KT; ++k)
+        if (EXACT || k < K) acc[k] += sigmoid_ref(v[k]);          // logits += seg_logit.sigmoid()
+    } else {
+      float s = 0.f;
+#pragma unroll
+      for (int k = 0; k < KT; ++k)
+        if (EXACT || k < K) { v[k] = expf(v[k] - m); s += v[k]; }
+#pragma unroll
+      for (int k = 0; k < KT; ++k)
+        if (EXACT || k < K) acc[k] += v[k] / s;                   // logits += seg_logit.softmax(dim=0)
+    }
+  }
+  float best = -INFINITY;
+  int bi = 0;
+#pragma unroll
+  for (int k = 0; k < KT; ++k) {
+    if (EXACT || k < K) {
+      const float mk = acc[k] / (float)a.V;                       // logits /= len(views)
+      const int64_t o = ((int64_t)n * K + k) * OHW + pix;
+      if (a.probs) a.probs[o] = mk;
+      if constexpr (kSigmoid) {
+        if (a.pred) reinterpret_cast<float*>(a.pred)[o] = mk > a.threshold ? 1.f : 0.f;
+      }
+      if (mk > best) { best = mk; bi = k; }                       // strict >: torch.argmax's first-max rule
+    }
+  }
+  if constexpr (!kSigmoid) {
+    if (a.pred) reinterpret_cast<TP*>(a.pred)[idx] = (TP)bi;
+  }
+}
+
+// General path, 32 < K <= 255: the accumulator of thread t lives in shared memory at acc[k * 32 + t] (one warp per
+// block, K * 128 bytes); each view's values are recomputed per pass from the same taps instead of held.
+template <typename TP>
+__global__ void __launch_bounds__(32) tta_merge_general_kernel(const __grid_constant__ TtaArgs a) {
+  extern __shared__ float tta_acc[];
+  float* acc = tta_acc + threadIdx.x;
+  const int K = a.K;
+  const int64_t OHW = (int64_t)a.oh * a.ow;
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (int64_t)a.N * OHW) return;
+  const int n = (int)(idx / OHW);
+  const int64_t pix = idx % OHW;
+  const int oy = (int)(pix / a.ow), ox = (int)(pix % a.ow);
+  for (int k = 0; k < K; ++k) acc[k * 32] = 0.f;
+  for (int i = 0; i < a.V; ++i) {
+    const TtaView& vw = a.v[i];
+    const Taps t = view_taps(vw.g, oy, ox, a.align_corners);
+    const float* base = vw.logits + (int64_t)n * vw.image_stride;
+    const int64_t plane = (int64_t)vw.g.H * vw.g.W;
+    if constexpr (std::is_same<TP, float>::value) {
+      for (int k = 0; k < K; ++k) acc[k * 32] += sigmoid_ref(view_value(base + k * plane, t, K));
+    } else {
+      float m = -INFINITY, s = 0.f;
+      for (int k = 0; k < K; ++k) m = fmaxf(m, view_value(base + k * plane, t, K));
+      for (int k = 0; k < K; ++k) s += expf(view_value(base + k * plane, t, K) - m);
+      for (int k = 0; k < K; ++k) acc[k * 32] += expf(view_value(base + k * plane, t, K) - m) / s;
+    }
+  }
+  const float V = (float)a.V;
+  float best = -INFINITY;
+  int bi = 0;
+  for (int k = 0; k < K; ++k) {
+    const float mk = acc[k * 32] / V;
+    const int64_t o = ((int64_t)n * K + k) * OHW + pix;
+    if (a.probs) a.probs[o] = mk;
+    if constexpr (std::is_same<TP, float>::value) {
+      if (a.pred) reinterpret_cast<float*>(a.pred)[o] = mk > a.threshold ? 1.f : 0.f;
+    }
+    if (mk > best) { best = mk; bi = k; }
+  }
+  if constexpr (!std::is_same<TP, float>::value) {
+    if (a.pred) reinterpret_cast<TP*>(a.pred)[idx] = (TP)bi;
+  }
+}
+
+template <typename TP>
+int launch_tta_merge(const TtaArgs& a, cudaStream_t st) {
+  const unsigned grid = (unsigned)ceil_div64((int64_t)a.N * a.oh * a.ow, 256);
+  switch (a.K) {
+    case 2: tta_merge_kernel<2, true, TP><<<grid, 256, 0, st>>>(a); break;       // Apple-Branch
+    case 19: tta_merge_kernel<19, true, TP><<<grid, 256, 0, st>>>(a); break;     // Cityscapes
+    default:
+      if (a.K <= 8) tta_merge_kernel<8, false, TP><<<grid, 256, 0, st>>>(a);
+      else if (a.K <= 16) tta_merge_kernel<16, false, TP><<<grid, 256, 0, st>>>(a);
+      else if (a.K <= 32) tta_merge_kernel<32, false, TP><<<grid, 256, 0, st>>>(a);
+      else
+        tta_merge_general_kernel<TP><<<(unsigned)ceil_div64((int64_t)a.N * a.oh * a.ow, 32), 32,
+                                       (size_t)a.K * 32 * sizeof(float), st>>>(a);
+  }
+  LEDB_LAUNCH_OK("tta_merge_kernel");
+  return LEDB200_OK;
 }
 
 __global__ void __launch_bounds__(256) slide_accumulate_kernel(float* preds, float* count, const float* crop, int N, int K,
@@ -195,19 +380,10 @@ int ledb200_postprocess(const float* logits, int32_t K, int32_t H, int32_t W, co
   if (pred && pred_dtype != LEDB200_U8 && pred_dtype != LEDB200_I64 && pred_dtype != LEDB200_F32)
     return fail(LEDB200_EINVAL, "postprocess: pred dtype must be U8, I64 or F32");
   PostArgs a;
-  a.logits = logits; a.K = K; a.H = H; a.W = W;
-  a.pl = padding_lrtb ? padding_lrtb[0] : 0; a.pr = padding_lrtb ? padding_lrtb[1] : 0;
-  a.pt = padding_lrtb ? padding_lrtb[2] : 0; a.pb = padding_lrtb ? padding_lrtb[3] : 0;
-  const int ch = H - a.pt - a.pb, cw = W - a.pl - a.pr;
-  if (a.pl < 0 || a.pr < 0 || a.pt < 0 || a.pb < 0 || ch < 1 || cw < 1)
+  a.logits = logits; a.K = K;
+  a.oh = out_h; a.ow = out_w; a.align_corners = align_corners ? 1 : 0;
+  if (!make_geom(H, W, padding_lrtb, flip, out_h, out_w, a.align_corners, a.g))
     return fail(LEDB200_EINVAL, "postprocess: padding removes the whole image");
-  a.flip = flip; a.oh = out_h; a.ow = out_w; a.align_corners = align_corners ? 1 : 0;
-  if (a.align_corners) {
-    a.sy = out_h > 1 ? (float)(ch - 1) / (float)(out_h - 1) : 0.f;
-    a.sx = out_w > 1 ? (float)(cw - 1) / (float)(out_w - 1) : 0.f;
-  } else {
-    a.sy = (float)ch / (float)out_h; a.sx = (float)cw / (float)out_w;
-  }
   a.threshold = threshold; a.pred = pred; a.pred_dtype = pred_dtype; a.out_logits = out_logits;
   const unsigned grid = (unsigned)ceil_div64((int64_t)out_h * out_w, 256);
   cudaStream_t st = (cudaStream_t)stream;
@@ -302,6 +478,38 @@ int ledb200_stack_pad(const void* img, int32_t img_dtype, int32_t h, int32_t w, 
   }
   LEDB_LAUNCH_OK("stack_pad_kernel");
   return LEDB200_OK;
+}
+
+int ledb200_tta_merge(const ledb200_tta_view* views, int32_t V, int32_t N, int32_t K, int32_t oh, int32_t ow,
+                      int32_t align_corners, int32_t mode, float threshold, void* pred, int32_t pred_dtype,
+                      float* probs_opt, void* stream) {
+  if (!views || (!pred && !probs_opt)) return fail(LEDB200_EINVAL, "tta_merge: null buffer");
+  if (V < 1 || V > kMaxViews) return fail(LEDB200_EINVAL, "tta_merge: between 1 and 32 views per call");
+  if (K < 1 || K > 255) return fail(LEDB200_EINVAL, "tta_merge: K must lie in [1, 255]");
+  if (N < 1 || oh < 1 || ow < 1) return fail(LEDB200_EINVAL, "tta_merge: empty tensor");
+  if (mode != 0 && mode != 1) return fail(LEDB200_EINVAL, "tta_merge: mode must be 0 (softmax) or 1 (sigmoid)");
+  if (pred && mode == 0 && pred_dtype != LEDB200_U8 && pred_dtype != LEDB200_I64)
+    return fail(LEDB200_EINVAL, "tta_merge: softmax-mode pred dtype must be U8 or I64");
+  if (pred && mode == 1 && pred_dtype != LEDB200_F32)
+    return fail(LEDB200_EINVAL, "tta_merge: sigmoid-mode pred (the float mask) must be F32");
+  TtaArgs a;
+  a.V = V; a.N = N; a.K = K; a.oh = oh; a.ow = ow; a.align_corners = align_corners ? 1 : 0;
+  a.threshold = threshold; a.pred = pred; a.probs = probs_opt;
+  for (int i = 0; i < V; ++i) {
+    const ledb200_tta_view& v = views[i];
+    if (!v.logits) return fail(LEDB200_EINVAL, "tta_merge: null view logits");
+    if (v.H < 1 || v.W < 1) return fail(LEDB200_EINVAL, "tta_merge: empty view");
+    if (v.flip < 0 || v.flip > 2) return fail(LEDB200_EINVAL, "tta_merge: flip must be 0 (none), 1 (horizontal) or 2 (vertical)");
+    if (N > 1 && v.image_stride < (int64_t)K * v.H * v.W)
+      return fail(LEDB200_EINVAL, "tta_merge: image_stride smaller than one image's [K, H, W] logits");
+    a.v[i].logits = v.logits; a.v[i].image_stride = v.image_stride;
+    if (!make_geom(v.H, v.W, v.pad_lrtb, v.flip, oh, ow, a.align_corners, a.v[i].g))
+      return fail(LEDB200_EINVAL, "tta_merge: a view's padding removes the whole image");
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (mode == 1) return launch_tta_merge<float>(a, st);
+  if (pred_dtype == LEDB200_I64) return launch_tta_merge<int64_t>(a, st);
+  return launch_tta_merge<uint8_t>(a, st);
 }
 
 }  // extern "C"

@@ -36,6 +36,7 @@ SYMBOLS = [
     'ledb200_mfaf_param_floats', 'ledb200_mfaf_workspace_bytes', 'ledb200_mfaf_forward',
     'ledb200_getb_param_floats', 'ledb200_getb_create', 'ledb200_getb_destroy', 'ledb200_getb_forward',
     'ledb200_postprocess', 'ledb200_slide_accumulate', 'ledb200_slide_finalize', 'ledb200_slide_merge', 'ledb200_stack_pad',
+    'ledb200_tta_merge',
     'ledb200_seam_param_floats', 'ledb200_seam_workspace_bytes', 'ledb200_seam_forward',
     'ledb200_conv_layer_create', 'ledb200_conv_layer_forward', 'ledb200_conv_layer_destroy',
     'ledb200_avgpool2d', 'ledb200_resize_bilinear', 'ledb200_add_relu', 'ledb200_conv_layer_forward_image',
@@ -53,6 +54,12 @@ class Cfg(C.Structure):
                 ('align_corners', C.c_int32), ('dtype', C.c_int32), ('device', C.c_int32),
                 ('variant', C.c_int32), ('conv_backend', C.c_int32), ('mean', C.c_float * 3),
                 ('std', C.c_float * 3), ('bgr_to_rgb', C.c_int32), ('reserved', C.c_int32 * 7)]
+
+
+class TtaView(C.Structure):
+    """ledb200_tta_view: image n of the view at logits + n * image_stride (fp32 elements); padding / flip to undo."""
+    _fields_ = [('logits', C.c_void_p), ('image_stride', C.c_int64), ('H', C.c_int32), ('W', C.c_int32),
+                ('pad_lrtb', C.c_int32 * 4), ('flip', C.c_int32)]
 
 
 _lib = None
@@ -156,6 +163,7 @@ def get():
     lib.ledb200_slide_finalize.argtypes = [vp, vp] + [i32] * 4 + [vp, i32, vp]
     lib.ledb200_slide_merge.argtypes = [vp, i32, vp, vp] + [i32] * 6 + [vp, vp, i32, vp]
     lib.ledb200_stack_pad.argtypes = [vp, i32, i32, i32, i32, vp, vp, f32, vp, i32, i32, vp, i32, vp, i32, vp]
+    lib.ledb200_tta_merge.argtypes = [C.POINTER(TtaView)] + [i32] * 7 + [f32, vp, i32, vp, vp]
     lib.ledb200_conv_layer_create.argtypes = [vp, vp, vp, vp] + [i32] * 5 + [C.POINTER(vp)]
     lib.ledb200_conv_layer_forward.argtypes = [vp, vp, vp, vp] + [i32] * 9 + [vp]
     lib.ledb200_conv_layer_destroy.argtypes = [vp]

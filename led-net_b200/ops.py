@@ -101,6 +101,9 @@ def conv2d(x_nhwc, weight_oihw, bias=None, stride=1, relu=False, residual=None, 
     return out_full[..., :Cout]
 
 
+_FLIP = {None: 0, False: 0, 'horizontal': 1, 'vertical': 2}
+
+
 def postprocess(seg_logit, padding=None, flip=None, ori_shape=None, align_corners=False, threshold=0.3,
                 pred_dtype=torch.int64, want_logits=True):
     """BaseSegmentor.postprocess_result for ONE image (base.py:153-198): seg_logit fp32 [K,H,W] -> crop `padding`
@@ -117,10 +120,54 @@ def postprocess(seg_logit, padding=None, flip=None, ori_shape=None, align_corner
     pred = torch.empty((1, oh, ow), dtype=pred_dtype, device=x.device)
     out = torch.empty((K, oh, ow), dtype=torch.float32, device=x.device) if want_logits else None
     pad_c = (C.c_int32 * 4)(*pad)
-    L.check(L.get().ledb200_postprocess(_p(x), K, H, W, pad_c, {None: 0, False: 0, 'horizontal': 1, 'vertical': 2}[flip],
+    L.check(L.get().ledb200_postprocess(_p(x), K, H, W, pad_c, _FLIP[flip],
                                         oh, ow, int(bool(align_corners)), float(threshold), _p(pred),
                                         L.torch_dtype_code(pred), _p(out), L.stream_ptr(x.device)), 'ledb200_postprocess')
     return pred, out
+
+
+def tta_merge(views, ori_shape, align_corners=False, mode=0, threshold=0.3, pred_dtype=torch.int64, want_pred=True,
+              want_probs=False, pred=None):
+    """SegTTAModel.merge_preds (seg_tta.py) over every view of N images in ONE launch.
+
+    views: list (1..32, augmentation order) of (logits, padding, flip): logits fp32 [N,K,H,W] on the device whose images
+    are each [K,H,W]-contiguous (a slice of a larger engine batch is used in place), padding (left, right, top, bottom)
+    or None, flip 'horizontal' | 'vertical' | None.  Each view is post-processed exactly as `postprocess` does (un-pad,
+    un-flip, bilinear resize to `ori_shape`), soft-maxed over K (mode 0: out_channels > 1) or sigmoid-ed (mode 1:
+    out_channels == 1), summed in order and divided by the number of views.
+    Returns (pred, probs): pred = argmax [N,oh,ow] of `pred_dtype` (mode 0) or the float mask merged > threshold
+    [N,K,oh,ow] (mode 1), None unless want_pred (written into `pred` when given); probs = the merged fp32 [N,K,oh,ow]
+    when want_probs, else None."""
+    V = len(views)
+    flat = []
+    for lg, _, _ in views:
+        _need_cuda(lg)
+        lg = lg.float()
+        assert lg.dim() == 4, 'view logits are [N,K,H,W]'
+        if not lg[0].is_contiguous():
+            lg = lg.contiguous()
+        flat.append(lg)
+    N, K = (flat[0].shape[0], flat[0].shape[1]) if flat else (1, 1)
+    assert all(t.shape[0] == N for t in flat), 'every view must hold the same images'
+    assert all(t.shape[1] == K for t in flat), 'every view must have the same number of classes'
+    oh, ow = (int(v) for v in ori_shape)
+    arr = (L.TtaView * max(V, 1))()
+    for d, t, (_, padding, flip) in zip(arr, flat, views):
+        d.logits, d.image_stride, d.H, d.W = t.data_ptr(), t.stride(0), t.shape[2], t.shape[3]
+        d.pad_lrtb[:] = [int(v) for v in (padding if padding is not None else (0, 0, 0, 0))]
+        d.flip = _FLIP[flip]
+    dev = flat[0].device if flat else torch.device('cuda', torch.cuda.current_device())
+    if pred is not None:
+        _need_cuda(pred)
+        assert pred.is_contiguous() and pred.numel() == N * oh * ow * (K if mode == 1 else 1), 'pred has the wrong shape'
+    elif want_pred:
+        pred = (torch.empty((N, K, oh, ow), dtype=torch.float32, device=dev) if mode == 1 else
+                torch.empty((N, oh, ow), dtype=pred_dtype, device=dev))
+    probs = torch.empty((N, K, oh, ow), dtype=torch.float32, device=dev) if want_probs else None
+    L.check(L.get().ledb200_tta_merge(arr, V, N, K, oh, ow, int(bool(align_corners)), int(mode), float(threshold),
+                                      _p(pred), L.torch_dtype_code(pred) if pred is not None else L.I64, _p(probs),
+                                      L.stream_ptr(dev)), 'ledb200_tta_merge')
+    return pred, probs
 
 
 def slide_accumulate(preds, count, crop_logits, y1, x1):

@@ -20,6 +20,16 @@ def _meta(sample):
     return sample.setdefault('metainfo', {}) if 'metainfo' in sample or 'gt_sem_seg' in sample else sample
 
 
+def _view_geometry(meta):
+    """(padding (left, right, top, bottom), flip direction or None) that postprocess_result undoes (base.py:163-176)."""
+    padding = meta.get('img_padding_size', meta.get('padding_size', [0] * 4))
+    flip = None
+    if meta.get('flip', None):
+        flip = meta.get('flip_direction', None)
+        assert flip in ['horizontal', 'vertical']
+    return padding, flip
+
+
 @MODELS.register_module()
 class SegDataPreProcessor(nn.Module):
     """mmseg/models/data_preprocessor.py:98-151 on the device: per sample ONE kernel (ops.stack_pad) does the BGR<->RGB
@@ -211,6 +221,16 @@ class EncoderDecoder(nn.Module):
         optimizer.step()
         return log
 
+    def test_step(self, data):
+        """mmengine BaseModel.test_step: data_preprocessor(data, False), then forward(mode='predict').  `data` is a dict
+        (inputs, data_samples) or an (inputs, data_samples) sequence."""
+        if isinstance(data, (list, tuple)):
+            data = dict(zip(('inputs', 'data_samples'), data))
+        data = (self.data_preprocessor or SegDataPreProcessor())(data, False)
+        return self.predict(data['inputs'], data.get('data_samples'))
+
+    val_step = test_step                            # mmengine's val_step is the same call
+
     def encode_decode(self, inputs, batch_img_metas=None):
         """encoder_decoder.py:124-132: full-resolution logits [N,K,H,W] (fused, one call)."""
         if self._composed:
@@ -278,11 +298,7 @@ class EncoderDecoder(nn.Module):
             meta = {}
             if data_samples is not None and isinstance(data_samples[i], dict):
                 meta = data_samples[i].get('metainfo', data_samples[i])
-            padding = meta.get('img_padding_size', meta.get('padding_size', [0] * 4))
-            flip = None
-            if meta.get('flip', None):
-                flip = meta.get('flip_direction', None)
-                assert flip in ['horizontal', 'vertical']
+            padding, flip = _view_geometry(meta)
             pred, lg = ops.postprocess(seg_logits[i], padding=padding, flip=flip, ori_shape=meta.get('ori_shape'),
                                        align_corners=self.align_corners,
                                        threshold=getattr(self.decode_head, 'threshold', None) or 0.3)
