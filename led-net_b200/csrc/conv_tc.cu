@@ -77,9 +77,8 @@ struct TcParams {
   const __nv_bfloat16* res; int res_ld;
   const float* bias;
   int relu;
-  // optional: out += bilinear x2 upsample (align_corners=False) of `up` [N, up_h, up_w, up_ld], added AFTER the ReLU
-  const __nv_bfloat16* up; int up_ld, up_h, up_w;
-  int up_f16, out_f16;               // ladder rungs are kept in fp16 (11-bit mantissa; logits are far inside its range)
+  int out_f16;                       // `out` holds IEEE fp16 (conv_seg's x_c, the bottom rung of the head ladder)
+  int fast_epi;                      // interior tiles take the epilogue fast path (decided once per launch, launch_conv_tc)
   // TF32 epilogue only: output pixel (oy, ox) of image n lands at ((n * o_H + oy * o_mul + o_a) * o_W + ox * o_mul + o_b):
   // o_mul = 2 writes one parity class of a twice-as-large tensor (data gradient of a stride-2 convolution)
   int o_mul, o_a, o_b, o_H, o_W;
@@ -147,7 +146,7 @@ __device__ __forceinline__ float4 lds128f(uint32_t addr) {
 // The second output relu(s*y + b) (pre-activation BN+ReLU of the consumer) goes through its own
 // staging tile.  Templated on which tensors exist so the hot loop has no per-element branches; ReLU is
 // a max against 0 or -inf.
-template <bool HAS_RES, bool HAS_OUT, bool HAS_OUT2, bool HAS_UP>
+template <bool HAS_RES, bool HAS_OUT, bool HAS_OUT2>
 __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int lane, uint32_t tmem_base,
                                               uint64_t* t_full, uint64_t* t_empty, uint32_t st_u, uint32_t bias_u,
                                               uint32_t o2s_u, uint32_t o2b_u) {
@@ -190,24 +189,15 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
   // thread owns one output pixel: 32 channels = 64 contiguous bytes = two 256-bit stores (full 32 B sectors),
   // the residual comes in as two 256-bit loads issued before the accumulator wait, and nothing touches shared
   // memory except the bias broadcast.
-  const bool cout_all = (cout8 == P.cp);
-  const bool al32 = ((P.out_ld | P.out2_ld | P.res_ld) % 16 == 0) &&
-                    (((uintptr_t)P.out | (uintptr_t)P.out2 | (uintptr_t)P.res) % 32 == 0);
-  const bool fast_launch = (ncols_g % 32 == 0) && P.relu != 2 &&
-                           (HAS_UP ? (P.up_ld == 24 && P.cp == 32 && cout8 == 24 && P.out_ld % 8 == 0)
-                                   : (cout_all && al32));
   const int lane_px = ph * Wo + pw;                                         // this thread's pixel inside the tile
   for (uint32_t tile = first; tile < total; tile += step) {
-    if (fast_launch && th * TH + TH <= Ho && tw * TW + TW <= Wo) {
+    if (P.fast_epi && th * TH + TH <= Ho && tw * TW + TW <= Wo) {
       const int64_t pix = ((int64_t)n * Ho + th * TH) * Wo + tw * TW + lane_px;
       const int cgt = nt * NT;
       const __nv_bfloat16* res_px = HAS_RES ? P.res + pix * P.res_ld + cgt : nullptr;
       __nv_bfloat16* out_px = HAS_OUT ? P.out + pix * P.out_ld + cgt : nullptr;
       __nv_bfloat16* out2_px = HAS_OUT2 ? P.out2 + pix * P.out2_ld + cgt : nullptr;
       uint4 rr[HAS_RES ? 4 : 1];
-      uint4 uu[HAS_UP ? 3 : 1][4];
-      __half2 hwx0, hwx1, hwy0, hwy1;
-      float uwx = 0.f, uwy = 0.f;
       if (HAS_RES) { ldg256(res_px + cbeg, rr[0], rr[1]); ldg256(res_px + cbeg + 16, rr[2], rr[3]); }
       if (HAS_RES && tile + step < total) {
         // L1 prefetch of the residual row the NEXT tile of this warp will read: the residual epilogue is bound by
@@ -224,24 +214,6 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
           if (ncols_g > 64) prefetch_l1(rn + 64);
         }
       }
-      if (HAS_UP) {
-        int y0, y1, x0, x1;
-        float l0;
-        bilinear_coord(th * TH + ph, 0.5f, P.up_h, y0, y1, l0, uwy);
-        bilinear_coord(tw * TW + pw, 0.5f, P.up_w, x0, x1, l0, uwx);
-        hwx1 = __float2half2_rn(uwx); hwx0 = __float2half2_rn(1.f - uwx);   // 0, 1/4, 3/4, 1: exact in fp16
-        hwy1 = __float2half2_rn(uwy); hwy0 = __float2half2_rn(1.f - uwy);
-        const __nv_bfloat16* ub = P.up + (int64_t)n * P.up_h * P.up_w * P.up_ld;
-        const __nv_bfloat16 *u00 = ub + (y0 * P.up_w + x0) * P.up_ld, *u01 = ub + (y0 * P.up_w + x1) * P.up_ld;
-        const __nv_bfloat16 *u10 = ub + (y1 * P.up_w + x0) * P.up_ld, *u11 = ub + (y1 * P.up_w + x1) * P.up_ld;
-#pragma unroll
-        for (int g = 0; g < 3; ++g) {
-          uu[g][0] = __ldg(reinterpret_cast<const uint4*>(u00 + 8 * g));
-          uu[g][1] = __ldg(reinterpret_cast<const uint4*>(u01 + 8 * g));
-          uu[g][2] = __ldg(reinterpret_cast<const uint4*>(u10 + 8 * g));
-          uu[g][3] = __ldg(reinterpret_cast<const uint4*>(u11 + 8 * g));
-        }
-      }
       mbar_wait(&t_full[ts], tp);
       tc_fence_after();
       TL(7, tile == blockIdx.x && warp == 2 && lane == 0);
@@ -254,7 +226,7 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
         const uint32_t bias_b = bias_u + (uint32_t)(cgt + c0) * 4;
         uint4 o[4], o2[HAS_OUT2 ? 4 : 1];
 #pragma unroll
-        for (int g = 0; g < (HAS_UP ? 3 : 4); ++g) {     // ladder rungs: 24 stored channels, the 4th group is padding
+        for (int g = 0; g < 4; ++g) {
           float f[8];
           const float4 b0 = lds128f(bias_b + 32 * g);
           const float4 b1 = lds128f(bias_b + 32 * g + 16);
@@ -270,34 +242,6 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
           }
 #pragma unroll
           for (int j = 0; j < 8; ++j) f[j] = fmaxf(f[j], relu_lo);
-          if (HAS_UP && g < 3) {
-            const int gg = g < 3 ? g : 0;
-            if (P.up_f16) {
-              // rung stored in fp16: interpolate in packed half2 (the weights are exact; two roundings of 2^-11
-              // on a term that is itself an fp16-rounded value), widen once
-              const __half2* a = reinterpret_cast<const __half2*>(&uu[gg][0]);
-              const __half2* b = reinterpret_cast<const __half2*>(&uu[gg][1]);
-              const __half2* c = reinterpret_cast<const __half2*>(&uu[gg][2]);
-              const __half2* d = reinterpret_cast<const __half2*>(&uu[gg][3]);
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const __half2 r0 = __hfma2(b[j], hwx1, __hmul2(a[j], hwx0));
-                const __half2 r1 = __hfma2(d[j], hwx1, __hmul2(c[j], hwx0));
-                const float2 u2 = __half22float2(__hfma2(r1, hwy1, __hmul2(r0, hwy0)));
-                f[2 * j] += u2.x; f[2 * j + 1] += u2.y;
-              }
-            } else {
-              float a[8], b[8], c[8], d[8];
-              unpack8(uu[gg][0], a); unpack8(uu[gg][1], b); unpack8(uu[gg][2], c); unpack8(uu[gg][3], d);
-              const float ux = 1.f - uwx, uy = 1.f - uwy;
-#pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                const float r0 = fmaf(b[j], uwx, a[j] * ux);
-                const float r1 = fmaf(d[j], uwx, c[j] * ux);
-                f[j] += fmaf(r1, uwy, r0 * uy);
-              }
-            }
-          }
           if (P.out_f16) {                             // cvt.rn.satfinite: saturates at +-65504, never inf
             o[g] = make_uint4(pack_f16x2_sat(f[0], f[1]), pack_f16x2_sat(f[2], f[3]), pack_f16x2_sat(f[4], f[5]),
                               pack_f16x2_sat(f[6], f[7]));
@@ -317,13 +261,8 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
         }
         if (HAS_RES && c0 + 32 < cend) { ldg256(res_px + c0 + 32, rr[0], rr[1]); ldg256(res_px + c0 + 48, rr[2], rr[3]); }
         if (!(P.dbg & 1)) {
-          if (HAS_UP) {                               // 24 stored channels, 48 B pixels: three 128-bit stores
-#pragma unroll
-            for (int g = 0; g < 3; ++g) *reinterpret_cast<uint4*>(out_px + 8 * g) = o[g];
-          } else {
-            if (HAS_OUT) { stg256(out_px + c0, o[0], o[1]); stg256(out_px + c0 + 16, o[2], o[3]); }
-            if (HAS_OUT2) { stg256(out2_px + c0, o2[0], o2[1]); stg256(out2_px + c0 + 16, o2[2], o2[3]); }
-          }
+          if (HAS_OUT) { stg256(out_px + c0, o[0], o[1]); stg256(out_px + c0 + 16, o[2], o[3]); }
+          if (HAS_OUT2) { stg256(out2_px + c0, o2[0], o2[1]); stg256(out2_px + c0 + 16, o2[2], o2[3]); }
         }
       }
     } else {
@@ -335,23 +274,10 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
     __nv_bfloat16* out_t = HAS_OUT ? P.out + pix0 * P.out_ld + cgt : nullptr;
     __nv_bfloat16* out2_t = HAS_OUT2 ? P.out2 + pix0 * P.out2_ld + cgt : nullptr;
     const int rows_ok = Ho - th * TH - q * 4, cols_ok = Wo - tw * TW;      // valid rows (of this warp's 4) / cols
-    // operand prefetch (residual / up-add corners) for one 32-column block; issued BEFORE the accumulator
-    // wait for the first block and one block ahead afterwards, so the L2 latency hides behind the MMAs
+    // residual prefetch for one 32-column block; issued BEFORE the accumulator wait for the first block and
+    // one block ahead afterwards, so the L2 latency hides behind the MMAs
     uint4 rr[4];
     bool rv[4];
-    uint4 uu[HAS_UP ? 3 : 1][4];
-    bool uv[3];
-    float uwx = 0.f, uwy = 0.f;
-    const __nv_bfloat16 *u00 = nullptr, *u01 = nullptr, *u10 = nullptr, *u11 = nullptr;
-    if (HAS_UP) {
-      int y0, y1, x0, x1;
-      float l0;
-      bilinear_coord(min(th * TH + ph, Ho - 1), 0.5f, P.up_h, y0, y1, l0, uwy);
-      bilinear_coord(min(tw * TW + pw, Wo - 1), 0.5f, P.up_w, x0, x1, l0, uwx);
-      const __nv_bfloat16* ub = P.up + (int64_t)n * P.up_h * P.up_w * P.up_ld + cgt;
-      u00 = ub + (y0 * P.up_w + x0) * P.up_ld; u01 = ub + (y0 * P.up_w + x1) * P.up_ld;
-      u10 = ub + (y1 * P.up_w + x0) * P.up_ld; u11 = ub + (y1 * P.up_w + x1) * P.up_ld;
-    }
     auto prefetch = [&](int c0) {
       const int ncol = min(32, cend - c0);
       if (HAS_RES) {
@@ -359,18 +285,6 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
         for (int g = 0; g < 4; ++g) {
           rv[g] = pvalid && (8 * g < ncol) && (cgt + c0 + 8 * g < cout8) && !(P.dbg & 8);
           if (rv[g]) rr[g] = __ldg(reinterpret_cast<const uint4*>(res_px + c0 + 8 * g));
-        }
-      }
-      if (HAS_UP) {
-#pragma unroll
-        for (int g = 0; g < 3; ++g) {
-          uv[g] = pvalid && (8 * g < ncol) && (cgt + c0 + 8 * g < P.up_ld);
-          if (uv[g]) {
-            uu[g][0] = __ldg(reinterpret_cast<const uint4*>(u00 + c0 + 8 * g));
-            uu[g][1] = __ldg(reinterpret_cast<const uint4*>(u01 + c0 + 8 * g));
-            uu[g][2] = __ldg(reinterpret_cast<const uint4*>(u10 + c0 + 8 * g));
-            uu[g][3] = __ldg(reinterpret_cast<const uint4*>(u11 + c0 + 8 * g));
-          }
         }
       }
     };
@@ -410,24 +324,6 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
 #pragma unroll
             for (int j = 0; j < 8; ++j) f[j] = fminf(f[j], 6.f);
           }
-          if (HAS_UP) {
-            if (g < 3 && uv[g < 3 ? g : 0]) {
-              float a[8], b[8], c[8], d[8];
-              const int gg = g < 3 ? g : 0;
-              if (P.up_f16) {
-                unpack8h(uu[gg][0], a); unpack8h(uu[gg][1], b); unpack8h(uu[gg][2], c); unpack8h(uu[gg][3], d);
-              } else {
-                unpack8(uu[gg][0], a); unpack8(uu[gg][1], b); unpack8(uu[gg][2], c); unpack8(uu[gg][3], d);
-              }
-              const float ux = 1.f - uwx, uy = 1.f - uwy;
-#pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                const float r0 = fmaf(b[j], uwx, a[j] * ux);
-                const float r1 = fmaf(d[j], uwx, c[j] * ux);
-                f[j] += fmaf(r1, uwy, r0 * uy);
-              }
-            }
-          }
           const uint32_t so = swz(row_off + (uint32_t)(slice_c + 8 * g) * 2);
           if (P.out_f16) {
 #pragma unroll
@@ -448,7 +344,7 @@ __device__ __forceinline__ void epilogue_loop(const TcParams& P, int warp, int l
           }
         }
       }
-      if ((HAS_RES || HAS_UP) && c0 + 32 < cend) prefetch(c0 + 32);
+      if (HAS_RES && c0 + 32 < cend) prefetch(c0 + 32);
       // ---- flush a completed staging slice with coalesced stores
       if (slice_c + ncol == slice_cols) {
         __syncwarp();
@@ -942,18 +838,17 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   } else if (warp < 10) {
     // =========================== epilogue: two groups of 4 warps (see epilogue_loop) ==============
     const uint32_t st_u = smem_u32(sStage), bias_u = smem_u32(s_bias), o2s_u = smem_u32(s_o2s), o2b_u = smem_u32(s_o2b);
-    const int variant = P.up ? 8 : ((P.res ? 1 : 0) | (P.out ? 2 : 0) | (P.out2 ? 4 : 0));
+    const int variant = (P.res ? 1 : 0) | (P.out ? 2 : 0) | (P.out2 ? 4 : 0);
     if constexpr (TF32 != 0) {
       epilogue_f32(P, warp, lane, tmem_base, t_full, t_empty, bias_u);
     } else
     switch (variant) {
-      case 2: epilogue_loop<false, true, false, false>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
-      case 3: epilogue_loop<true, true, false, false>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
-      case 4: epilogue_loop<false, false, true, false>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
-      case 5: epilogue_loop<true, false, true, false>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
-      case 6: epilogue_loop<false, true, true, false>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
-      case 8: epilogue_loop<false, true, false, true>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
-      default: epilogue_loop<true, true, true, false>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
+      case 2: epilogue_loop<false, true, false>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
+      case 3: epilogue_loop<true, true, false>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
+      case 4: epilogue_loop<false, false, true>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
+      case 5: epilogue_loop<true, false, true>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
+      case 6: epilogue_loop<false, true, true>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
+      default: epilogue_loop<true, true, true>(P, warp, lane, tmem_base, t_full, t_empty, st_u, bias_u, o2s_u, o2b_u); break;
     }
   }
 
@@ -1029,7 +924,7 @@ bool conv_tc_eligible(const ConvArgs& a) {
   if (a.tf32) {
     // training convolutions: fp32 NHWC in, raw fp32 (+ bias) out, TF32 tensor-core arithmetic (see epilogue_f32)
     if (a.in_dtype != LEDB200_F32 || a.out_dtype != LEDB200_F32 || !a.out) return false;
-    if (a.pre_scale || a.res || a.out2 || a.up || a.relu == 2) return false;
+    if (a.pre_scale || a.res || a.out2 || a.relu == 2) return false;
     if (a.ksize != 1 && a.ksize != 3) return false;
     if (a.stride != 1 && a.stride != 2) return false;
     if (a.dil != 1 && a.ksize == 3) return false;
@@ -1058,10 +953,6 @@ bool conv_tc_eligible(const ConvArgs& a) {
   if (a.out2 && (a.out2_ld % 8 || a.out2_ld < c8)) return false;
   if (a.res && (a.res_ld % 8 || a.res_ld < c8)) return false;
   const int cp = a.cout_pad_tc > 0 ? a.cout_pad_tc : conv_tc_pad(a.Cout);
-  if (a.up) {   // fused x2 upsample-add: one 32-column block, <= 24 source channels, exact x2, no residual / 2nd output
-    if (cp > 32 || a.up_ld > 24 || a.up_ld % 8 || a.up_ld < c8 || a.res || a.out2 || !a.out) return false;
-    if (a.Ho != 2 * a.up_h || a.Wo != 2 * a.up_w) return false;
-  }
   if (cp > 256 && cp % 256) return false;
   if (cp != 16 && cp != 32 && cp % 64) return false;                 // epilogue staging slices are 16/32/64 channels
   if ((int64_t)a.N * ceil_div(a.Ho, TH) * ceil_div(a.Wo, TW) * (cp > 256 ? cp / 256 : 1) >= (1ll << 31)) return false;
@@ -1158,19 +1049,18 @@ int launch_conv_tc(const ConvArgs& a, cudaStream_t st) {
   P.ntaps_total = taps;
   // ---- shared-memory plan
   P.cp = cp;
-  P.stage_bytes = a.out2 ? 65536u : 32768u;
   {
-    // When every tile is interior and the launch takes the epilogue fast path (same conditions as in
-    // epilogue_loop), the staging tiles are never touched: give their 32-64 KB to the A ring / resident weights.
+    // Epilogue fast path for interior tiles (epilogue_loop): whole 32-column blocks per epilogue group, no ReLU6, no
+    // channel padding beyond the 8-channel groups, 32 B aligned pixels for the 256-bit accesses.
     const int cout8 = (a.Cout + 7) & ~7;
     const int ncols_g = P.NT >= 64 ? P.NT / 2 : P.NT;
     const bool al32 = ((a.out_ld | a.out2_ld | a.res_ld) % 16 == 0) &&
                       (((uintptr_t)a.out | (uintptr_t)a.out2 | (uintptr_t)a.res) % 32 == 0);
-    const bool fast = (ncols_g % 32 == 0) && a.relu != 2 &&
-                      (a.up ? (a.up_ld == 24 && cp == 32 && cout8 == 24 && a.out_ld % 8 == 0) : (cout8 == cp && al32));
-    if (fast && a.Ho % TH == 0 && a.Wo % TW == 0) P.stage_bytes = 0;
-    if (tf32) P.stage_bytes = 0;
+    P.fast_epi = (ncols_g % 32 == 0) && a.relu != 2 && cout8 == cp && al32;
   }
+  // When every tile is interior and takes the fast path (or the TF32 epilogue), the staging tiles are never touched:
+  // their 32-64 KB go to the A ring / resident weights.
+  P.stage_bytes = (tf32 || (P.fast_epi && a.Ho % TH == 0 && a.Wo % TW == 0)) ? 0u : (a.out2 ? 65536u : 32768u);
   const uint32_t bar_bytes = (uint32_t)((3 * cp * 4 + 48 * 8 + 16 + 1023) / 1024 * 1024) + P.stage_bytes;
   const uint32_t b_res_bytes = (uint32_t)(P.nchunks * 9) * P.b_tile_bytes;
   P.b_resident = (P.ntiles_n == 1 && b_res_bytes <= (P.stage_bytes ? 100u : 150u) * 1024) ? 1 : 0;
@@ -1225,8 +1115,7 @@ int launch_conv_tc(const ConvArgs& a, cudaStream_t st) {
   P.res = (const __nv_bfloat16*)a.res; P.res_ld = a.res_ld; P.bias = a.bias; P.relu = a.relu;
   { const char* e = getenv("LEDB200_TC_DBG"); P.dbg = e ? atoi(e) : 0; }
   { static int tl_counter = 0; P.tl_launch = tl_counter++; }
-  P.up = (const __nv_bfloat16*)a.up; P.up_ld = a.up_ld; P.up_h = a.up_h; P.up_w = a.up_w;
-  P.up_f16 = a.up_f16; P.out_f16 = a.out_f16;
+  P.out_f16 = a.out_f16;
   P.o_mul = a.sub ? 2 : 1; P.o_a = a.sub ? a.sub_a : 0; P.o_b = a.sub ? a.sub_b : 0;
   P.o_H = a.Ho * P.o_mul; P.o_W = a.Wo * P.o_mul;
 

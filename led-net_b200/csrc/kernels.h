@@ -19,11 +19,7 @@ struct ConvArgs {
   const void* res = nullptr;    // optional residual, same dtype as out
   int res_ld = 0;
   const float* bias = nullptr;  // [Cout] (device)
-  // tensor-core path only: out = act(conv) + bilinear x2 upsample (align_corners=False) of `up`
-  // [N, up_h, up_w, up_ld] bf16 with Ho == 2*up_h, Wo == 2*up_w (the head ladder, decode_head.py:366-372)
-  const void* up = nullptr;
-  int up_ld = 0, up_h = 0, up_w = 0;
-  int up_f16 = 0, out_f16 = 0;   // `up` / `out` hold IEEE fp16 instead of bf16 (ladder rungs r2, r1)
+  int out_f16 = 0;              // tensor-core path only: `out` holds IEEE fp16 instead of bf16 (x_c, the ladder's bottom rung)
   const float* pre_scale = nullptr;  // [Cin] prologue affine (device), CUDA-core path only
   const float* pre_shift = nullptr;
   int pre_relu = 1;
@@ -159,16 +155,15 @@ struct TailArgs {
 };
 int launch_tail(const TailArgs& a, cudaStream_t st);
 
-// last ladder stage only: r1 [N,h2,w2,ld] bf16 (the two lower rungs were added in the head convs' epilogues)
-// -> argmax of its exact x2 upsample (tail.cu, tail2_kernel)
+// last ladder stage only: r1 [N,h2,w2,ld] fp16 (the top rung written by ladder_kernel)
+// -> logits and argmax of its exact x2 upsample (tail.cu, tail2_kernel)
 struct Tail2Args {
-  const void* r1 = nullptr;   // fp16 (f16 = 1) or bf16
-  int f16 = 0;
+  const __half* r1 = nullptr;
   int ld = 0;
   int N = 0, K = 0, h2 = 0, w2 = 0;
   void* pred = nullptr;       // [N,2*h2,2*w2]
   int pred_dtype = LEDB200_U8;
-  float* logits = nullptr;    // optional fp32 NCHW
+  float* logits = nullptr;    // fp32 NCHW, required
 };
 int launch_tail2(const Tail2Args& a, cudaStream_t st);
 

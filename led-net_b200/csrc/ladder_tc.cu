@@ -9,17 +9,15 @@
 //   ladder_kernel<false>  (rung):  out[N,H,W,24] fp16 = relu(conv3x3(in) + b) + up2(up)          head_x2 always;
 //                                  head_x1 only when the caller wants the full-resolution logits (tail2 follows)
 //   ladder_kernel<true>   (final): label[N,2H,2W] = argmax_k up2(relu(conv3x3(in) + b) + up2(up))   head_x1 hot path:
-//                                  r1 (402 MB per 16-image batch as fp16) never reaches HBM - round 1 wrote it from
-//                                  the conv epilogue and read it back in tail3 (0.43 + 0.31 ms, VERDICT r1 item 5).
+//                                  r1 (402 MB per 16-image batch as fp16) never reaches HBM.
 //
 // GEMM side (same machinery as conv_tc.cu, MODE 0 / KC = 32 / resident weights): M = 128 pixels (16 x 8 tile),
 // N = 32 (K <= 24 classes, zero padded), K = 9 taps x Cin; ONE TMA halo slab (18 x 10 pixels x 32 ch, 64 B swizzle)
 // per Cin block, nine shifted UMMA descriptors into it; fp32 accumulators in TMEM, EIGHT 32-column stages.
 //
-// What is new against conv_tc's ladder epilogue (ncu r1g: issue 35 %, dram 27 %, 168 registers, 2 epilogue warps per
-// scheduler, 12 x 16 B global corner gathers per thread):
+// Epilogue:
 //   * 16 epilogue warps = four groups of four; group g owns every fourth tile of the CTA.  With a per-tile epilogue
-//     of ~700 instructions per thread the warp schedulers are the limiter, so they get 4 warps each instead of 2;
+//     of ~700 instructions per thread the warp schedulers are the limiter, so each gets 4 epilogue warps;
 //   * the `up` corner patch (10 x 6 pixels x 24 ch fp16 = 2.9 KB) arrives by TMA per tile (its own full / empty
 //     barrier ring, loaded with the A slab), so the gather is 12 conflict-free LDS.128 (48 B pixel stride) at 29 clk
 //     instead of L2 round trips, and nothing has to be prefetched into registers across the accumulator wait;
@@ -30,11 +28,12 @@
 //     leaves the tensor by at most one pixel).  The group writes its r1 tile (fp16, 48 B per pixel) to a
 //     double-buffered shared exchange tile, one named barrier, then thread (i, j) owns the 2 x 2 outputs BETWEEN r1
 //     pixels (i, j) .. (i+1, j+1) - rows 2y+1, 2y+2 - from its own pixel (registers) and three neighbours (LDS), with
-//     packed f32x2 lerps in tail3_kernel's operation order (bit-identical logits) and a strict `>` running argmax in
-//     ascending class order = torch.argmax's first-max rule.  Output row 0 / column 0 (source index clamped: a pure
-//     copy of the first r1 row / column) are written by the threads of r1 row 0 / column 0 in a second, rare pass.
-//     22 % of the MMA work is recomputed (pixels covered by two tiles get bit-identical values, so the duplicate
-//     label stores are benign); 0.8 GB per step of HBM traffic and one launch disappear.
+//     packed f32x2 lerps in tail2_kernel's operation order (horizontal with (1/4, 3/4), then vertical: bit-identical
+//     logits) and a strict `>` running argmax in ascending class order = torch.argmax's first-max rule.  Output row 0 /
+//     column 0 (source index clamped: a pure copy of the first r1 row / column) are written by the threads of r1 row 0
+//     / column 0 in a second, rare pass.  22 % of the MMA work is recomputed (pixels covered by two tiles get
+//     bit-identical values, so the duplicate label stores are benign); in exchange r1 never makes the 0.8 GB per step
+//     round trip through HBM and no separate tail launch is needed.
 //   * one producer thread per operand (warp 0: A slabs, warp 3: `up` patches), tile coordinates advanced as
 //     mixed-radix digits: a single thread doing both plus three integer divisions per tile bounded the kernel at
 //     ~800 clk per tile (probe: 239 us with every other role switched off).
@@ -408,7 +407,7 @@ ladder_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
               const bool two = k + 1 < K;
               const float2 TL = __half22float2(htl[j]), TR = __half22float2(htr[j]);
               const float2 BL = __half22float2(hbl[j]), BR = __half22float2(hbr[j]);
-              // horizontal first, then vertical (tail3_kernel's order)
+              // horizontal first, then vertical (tail2_kernel's order)
               const float2 t1 = lerp2(TL, TR, q34, q14), t2 = lerp2(TL, TR, q14, q34);
               const float2 b1 = lerp2(BL, BR, q34, q14), b2 = lerp2(BL, BR, q14, q34);
               const float2 o11 = lerp2(t1, b1, q34, q14), o12 = lerp2(t2, b2, q34, q14);

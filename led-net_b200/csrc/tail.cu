@@ -21,8 +21,6 @@
 // torch.argmax's first-max rule.  Every input element is read once per CTA (plus the 1-pixel clamped
 // halo); output is 1 byte per pixel (or int64 when asked).  The kernel is instruction-issue bound
 // (about 7.5 instructions per output logit in the last stage), not HBM bound: DESIGN.md section 3.
-#include <cstdlib>
-
 #include "kernels.h"
 
 namespace ledb {
@@ -273,10 +271,9 @@ tail_kernel(TailArgs a, float s2h, float s2w, float sch, float scw, int vec, int
 
 
 // ---------------------------------------------------------------------------------------------
-// tail2: the LAST stage only.  Used when the two lower rungs of the ladder were already folded into the
-// head convolutions' epilogues (conv_tc.cu, `up` operand): the input is r1 = head_x1 + up(head_x2 + up(x_c))
-// at half resolution (fp16 or bf16, NHWC, pixel stride `ld`), the output is argmax_k of its exact x2 bilinear
-// upsample (decode_head.py:373-378 + base.py:187-188).
+// tail2: the LAST stage only, for callers that want the full-resolution logits.  The ladder kernel (ladder_tc.cu) has
+// already formed r1 = head_x1 + up(head_x2 + up(x_c)) at half resolution (fp16, NHWC, pixel stride `ld`); the outputs
+// are its exact x2 bilinear upsample as fp32 NCHW logits and their argmax_k (decode_head.py:373-378 + base.py:187-188).
 //
 // CTA = 128 threads = 8 x 16 thread grid, 32 x 64 output tile, 18 x 34 r1 patch (clamped halo) staged in
 // shared memory as fp32 CLASS PAIRS: plane[kp][row][col] = float2(class 2kp, class 2kp+1), so one LDS.128
@@ -291,9 +288,9 @@ __device__ __forceinline__ float2 lerp2(float2 a, float2 b, float2 w0, float2 w1
   return __ffma2_rn(b, w1, __fmul2_rn(a, w0));   // b*w1 + a*w0 per lane: fmaf(b, w1, a*w0)
 }
 
-template <typename T, typename TP>
+template <typename TP>
 __global__ void __launch_bounds__(TAIL_THREADS, 4)
-tail2_kernel(const T* __restrict__ r1, int ld, int K, int h2, int w2, TP* __restrict__ pred_base,
+tail2_kernel(const __half* __restrict__ r1, int ld, int K, int h2, int w2, TP* __restrict__ pred_base,
              float* __restrict__ logits, int planes) {
   extern __shared__ __align__(16) float2 sp[];          // [pairs][R1_H][R1_W]
   const int Ho = 2 * h2, Wo = 2 * w2;
@@ -302,7 +299,7 @@ tail2_kernel(const T* __restrict__ r1, int ld, int K, int h2, int w2, TP* __rest
   const int a0 = (blockIdx.x / tiles_x) * TROWS, b0 = (blockIdx.x % tiles_x) * TCOLS;
   const int t = threadIdx.x;
   const int tr = t / TCOLS, tc = t % TCOLS;
-  const T* src = r1 + (int64_t)n * h2 * w2 * ld;
+  const __half* src = r1 + (int64_t)n * h2 * w2 * ld;
 
   const int oy0 = 4 * (a0 + tr), ox0 = 4 * (b0 + tc);
   // exact x2, align_corners=False: even outputs take (1/4, 3/4) of window (i-1, i), odd ones (3/4, 1/4) of
@@ -361,27 +358,25 @@ tail2_kernel(const T* __restrict__ r1, int ld, int K, int h2, int w2, TP* __rest
         for (int r = 0; r < 4; ++r) {
           if (o[r].x > best[r][c]) { best[r][c] = o[r].x; bidx[r][c] = k; }        // strict > : first max wins
           if (two && o[r].y > best[r][c]) { best[r][c] = o[r].y; bidx[r][c] = k + 1; }
-          hrow[r][c] = o[r];          // staging for the optional logits store
+          hrow[r][c] = o[r];          // staging for the logits store
         }
       }
-      if (logits) {
 #pragma unroll
-        for (int half = 0; half < 2; ++half) {
-          if (half && !two) break;
+      for (int half = 0; half < 2; ++half) {
+        if (half && !two) break;
 #pragma unroll
-          for (int r = 0; r < 4; ++r) {
-            const int oy = oy0 + r;
-            if (oy < Ho) {
-              float* lp = logits + (((int64_t)n * K + k + half) * Ho + oy) * Wo + ox0;
-              float vv[4];
+        for (int r = 0; r < 4; ++r) {
+          const int oy = oy0 + r;
+          if (oy < Ho) {
+            float* lp = logits + (((int64_t)n * K + k + half) * Ho + oy) * Wo + ox0;
+            float vv[4];
 #pragma unroll
-              for (int c = 0; c < 4; ++c) vv[c] = half ? hrow[r][c].y : hrow[r][c].x;
-              if (ox0 + 3 < Wo && (Wo & 3) == 0) {
-                *reinterpret_cast<float4*>(lp) = make_float4(vv[0], vv[1], vv[2], vv[3]);
-              } else {
+            for (int c = 0; c < 4; ++c) vv[c] = half ? hrow[r][c].y : hrow[r][c].x;
+            if (ox0 + 3 < Wo && (Wo & 3) == 0) {
+              *reinterpret_cast<float4*>(lp) = make_float4(vv[0], vv[1], vv[2], vv[3]);
+            } else {
 #pragma unroll
-                for (int c = 0; c < 4; ++c) if (ox0 + c < Wo) lp[c] = vv[c];
-              }
+              for (int c = 0; c < 4; ++c) if (ox0 + c < Wo) lp[c] = vv[c];
             }
           }
         }
@@ -392,93 +387,6 @@ tail2_kernel(const T* __restrict__ r1, int ld, int K, int h2, int w2, TP* __rest
   TP* pred = pred_base + (int64_t)n * Ho * Wo;
 #pragma unroll
   for (int r = 0; r < 4; ++r) {
-    const int oy = oy0 + r;
-    if (oy >= Ho) continue;
-    if (sizeof(TP) == 1 && ox0 + 3 < Wo && (Wo & 3) == 0) {
-      uchar4 u = make_uchar4((unsigned char)bidx[r][0], (unsigned char)bidx[r][1], (unsigned char)bidx[r][2],
-                             (unsigned char)bidx[r][3]);
-      *reinterpret_cast<uchar4*>(reinterpret_cast<uint8_t*>(pred) + (int64_t)oy * Wo + ox0) = u;
-    } else {
-#pragma unroll
-      for (int c = 0; c < 4; ++c)
-        if (ox0 + c < Wo) pred[(int64_t)oy * Wo + ox0 + c] = (TP)bidx[r][c];
-    }
-  }
-}
-
-
-// tail3: same stage as tail2 for the label-only hot path, at twice the occupancy.  tail2's 4 x 4 block per thread needs
-// 127 registers (16 running maxima + indices, 16 float2 of horizontal results), so only 16 warps fit per SM and the
-// issue slots are 45 % used (ncu r1b).  Here a thread owns 2 rows x 4 columns of outputs: 3 window rows instead of 4,
-// 8 running (max, index) pairs, 256 threads per 32 x 64 tile - ~20 % more instructions per output, half the registers.
-constexpr int T3_THREADS = 256;             // 16 x 16 threads, each 2 rows x 4 cols
-template <typename T, typename TP>
-__global__ void __launch_bounds__(T3_THREADS, 4)
-tail3_kernel(const T* __restrict__ r1, int ld, int K, int h2, int w2, TP* __restrict__ pred_base, int planes) {
-  extern __shared__ __align__(16) float2 sp[];          // [pairs][R1_H][R1_W]
-  const int Ho = 2 * h2, Wo = 2 * w2;
-  const int tiles_x = (Wo + OT_W - 1) / OT_W;
-  const int n = blockIdx.y;
-  const int a0 = (blockIdx.x / tiles_x) * TROWS, b0 = (blockIdx.x % tiles_x) * TCOLS;   // tile origin in 4-output units
-  const int t = threadIdx.x;
-  const int ty = t / TCOLS, tx = t % TCOLS;             // ty 0..15: r1 row of the tile, tx 0..15: pair of r1 columns
-  const T* src = r1 + (int64_t)n * h2 * w2 * ld;
-  const int oy0 = 4 * a0 + 2 * ty, ox0 = 4 * (b0 + tx);
-  const float2 q14 = make_float2(0.25f, 0.25f), q34 = make_float2(0.75f, 0.75f);
-  float best[2][4];
-  int bidx[2][4];
-#pragma unroll
-  for (int r = 0; r < 2; ++r)
-#pragma unroll
-    for (int c = 0; c < 4; ++c) { best[r][c] = -INFINITY; bidx[r][c] = 0; }
-
-  for (int k0 = 0; k0 < K; k0 += 2 * T2_PAIRS) {
-    const int kc = min(2 * T2_PAIRS, K - k0);
-    const int ng = (kc + 7) >> 3;
-    if (k0) __syncthreads();
-    for (int i = t; i < T2_PLANE * ng; i += T3_THREADS) {
-      const int p = i / ng, g = i - p * ng;
-      const int pi = p / R1_W, pj = p - pi * R1_W;
-      const int gy = clampi(2 * a0 - 1 + pi, 0, h2 - 1), gx = clampi(2 * b0 - 1 + pj, 0, w2 - 1);
-      float v[8];
-      load8(src + ((int64_t)gy * w2 + gx) * ld + k0 + 8 * g, v);
-#pragma unroll
-      for (int j = 0; j < 4; ++j)
-        if (4 * g + j < planes) sp[(4 * g + j) * T2_PLANE + p] = make_float2(v[2 * j], v[2 * j + 1]);
-    }
-    __syncthreads();
-    const int npair = (kc + 1) >> 1;
-    for (int kp = 0; kp < npair; ++kp) {
-      // patch row 0 is r1 row -1 of the tile: output rows 2 ty, 2 ty + 1 use patch rows ty, ty + 1, ty + 2
-      const float2* base = sp + kp * T2_PLANE + ty * R1_W + 2 * tx;
-      float2 hrow[3][4];
-#pragma unroll
-      for (int wi = 0; wi < 3; ++wi) {
-        const float4 pq = *reinterpret_cast<const float4*>(base + wi * R1_W);
-        const float4 rs = *reinterpret_cast<const float4*>(base + wi * R1_W + 2);
-        const float2 c0 = make_float2(pq.x, pq.y), c1 = make_float2(pq.z, pq.w);
-        const float2 c2 = make_float2(rs.x, rs.y), c3 = make_float2(rs.z, rs.w);
-        hrow[wi][0] = lerp2(c0, c1, q14, q34);
-        hrow[wi][1] = lerp2(c1, c2, q34, q14);
-        hrow[wi][2] = lerp2(c1, c2, q14, q34);
-        hrow[wi][3] = lerp2(c2, c3, q34, q14);
-      }
-      const int k = k0 + 2 * kp;
-      const bool two = (2 * kp + 1) < kc;
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        const float2 o0 = lerp2(hrow[0][c], hrow[1][c], q14, q34);     // even output row
-        const float2 o1 = lerp2(hrow[1][c], hrow[2][c], q34, q14);     // odd output row
-        if (o0.x > best[0][c]) { best[0][c] = o0.x; bidx[0][c] = k; }  // strict > in ascending class order: first max
-        if (two && o0.y > best[0][c]) { best[0][c] = o0.y; bidx[0][c] = k + 1; }
-        if (o1.x > best[1][c]) { best[1][c] = o1.x; bidx[1][c] = k; }
-        if (two && o1.y > best[1][c]) { best[1][c] = o1.y; bidx[1][c] = k + 1; }
-      }
-    }
-  }
-  TP* pred = pred_base + (int64_t)n * Ho * Wo;
-#pragma unroll
-  for (int r = 0; r < 2; ++r) {
     const int oy = oy0 + r;
     if (oy >= Ho) continue;
     if (sizeof(TP) == 1 && ox0 + 3 < Wo && (Wo & 3) == 0) {
@@ -542,44 +450,22 @@ int launch_tail(const TailArgs& a, cudaStream_t st) {
 int launch_tail2(const Tail2Args& a, cudaStream_t st) {
   if (a.K < 1 || a.K > 255) return fail(LEDB200_EINVAL, "tail2: K must be in [1,255]");
   if (a.N < 1 || a.h2 < 1 || a.w2 < 1) return fail(LEDB200_EINVAL, "tail2: empty input");
+  if (!a.logits) return fail(LEDB200_EINVAL, "tail2: logits output required (labels alone come from the ladder kernel)");
   if (a.ld % 8 || a.ld < (a.K + 7) / 8 * 8 || ((uintptr_t)a.r1 & 15))
-    return fail(LEDB200_EINVAL, "tail2: r1 must be bf16 NHWC with a 16-byte aligned pixel stride covering K rounded up to 8");
+    return fail(LEDB200_EINVAL, "tail2: r1 must be fp16 NHWC with a 16-byte aligned pixel stride covering K rounded up to 8");
+  if (a.pred_dtype != LEDB200_U8 && a.pred_dtype != LEDB200_I64)
+    return fail(LEDB200_EINVAL, "tail2: pred dtype must be U8 or I64");
   const int Ho = 2 * a.h2, Wo = 2 * a.w2;
   dim3 grid(ceil_div(Wo, OT_W) * ceil_div(Ho, OT_H), a.N);
   const int pairs = std::min(T2_PAIRS, (a.K + 1) / 2);
   const size_t smem = (size_t)pairs * T2_PLANE * sizeof(float2);
-#define LEDB_TAIL2(T, TP)                                                                                \
+#define LEDB_TAIL2(TP)                                                                                   \
   do {                                                                                                   \
-    LEDB_CUDA_OK(cudaFuncSetAttribute(tail2_kernel<T, TP>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
+    LEDB_CUDA_OK(cudaFuncSetAttribute(tail2_kernel<TP>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
                                       (int)smem));                                                       \
-    tail2_kernel<T, TP><<<grid, TAIL_THREADS, smem, st>>>(reinterpret_cast<const T*>(a.r1), a.ld, a.K, a.h2, \
-                                                          a.w2, (TP*)a.pred, a.logits, pairs);           \
+    tail2_kernel<TP><<<grid, TAIL_THREADS, smem, st>>>(a.r1, a.ld, a.K, a.h2, a.w2, (TP*)a.pred, a.logits, pairs); \
   } while (0)
-  if (a.pred_dtype != LEDB200_U8 && a.pred_dtype != LEDB200_I64)
-    return fail(LEDB200_EINVAL, "tail2: pred dtype must be U8 or I64");
-  static const bool no_tail3 = getenv("LEDB200_NO_TAIL3") != nullptr;
-  if (!a.logits && !no_tail3) {            // label-only hot path: the 2 x 4 outputs-per-thread kernel
-#define LEDB_TAIL3(T, TP)                                                                                \
-  do {                                                                                                   \
-    LEDB_CUDA_OK(cudaFuncSetAttribute(tail3_kernel<T, TP>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                                      (int)smem));                                                       \
-    tail3_kernel<T, TP><<<grid, T3_THREADS, smem, st>>>(reinterpret_cast<const T*>(a.r1), a.ld, a.K, a.h2, \
-                                                        a.w2, (TP*)a.pred, pairs);                       \
-  } while (0)
-    if (a.f16) {
-      if (a.pred_dtype == LEDB200_U8) LEDB_TAIL3(__half, uint8_t); else LEDB_TAIL3(__half, int64_t);
-    } else {
-      if (a.pred_dtype == LEDB200_U8) LEDB_TAIL3(__nv_bfloat16, uint8_t); else LEDB_TAIL3(__nv_bfloat16, int64_t);
-    }
-#undef LEDB_TAIL3
-    LEDB_LAUNCH_OK("tail3_kernel");
-    return LEDB200_OK;
-  }
-  if (a.f16) {
-    if (a.pred_dtype == LEDB200_U8) LEDB_TAIL2(__half, uint8_t); else LEDB_TAIL2(__half, int64_t);
-  } else {
-    if (a.pred_dtype == LEDB200_U8) LEDB_TAIL2(__nv_bfloat16, uint8_t); else LEDB_TAIL2(__nv_bfloat16, int64_t);
-  }
+  if (a.pred_dtype == LEDB200_U8) LEDB_TAIL2(uint8_t); else LEDB_TAIL2(int64_t);
 #undef LEDB_TAIL2
   LEDB_LAUNCH_OK("tail2_kernel");
   return LEDB200_OK;

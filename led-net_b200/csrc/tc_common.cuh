@@ -225,11 +225,6 @@ __device__ __forceinline__ uint32_t pack_f16x2_sat(float a, float b) {   // a ->
   asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
   return r;
 }
-__device__ __forceinline__ void unpack8h(const uint4& u, float* f) {
-  const __half2* h = reinterpret_cast<const __half2*>(&u);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { float2 t = __half22float2(h[i]); f[2 * i] = t.x; f[2 * i + 1] = t.y; }
-}
 __device__ __forceinline__ void unpack8(const uint4& u, float* f) {
   const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&u);
 #pragma unroll
