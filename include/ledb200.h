@@ -461,6 +461,44 @@ int ledb200_tta_merge(const ledb200_tta_view* views, int32_t V, int32_t N, int32
                       int32_t align_corners, int32_t mode, float threshold, void* pred, int32_t pred_dtype,
                       float* probs_opt, void* stream);
 
+/* ---- training augmentation (csrc/augment.cu) ---------------------------------------------------------------------------
+ * The config's train_pipeline RandomResize (keep_ratio) -> RandomCrop (cat_max_ratio) -> RandomFlip (horizontal) ->
+ * PhotoMetricDistortion, then SegDataPreProcessor's swap / normalisation / padding, for up to 64 samples per call; the
+ * random draws are the caller's (one descriptor per sample, HOST array).  img: [3,h,w] uint8 CHW as decoded (BGR);
+ * label: [h,w] of `label_dtype` (U8 or I64).  (rh, rw): the RandomResize size of the sample (cv2 INTER_LINEAR for the
+ * image, INTER_NEAREST for the label).  offsets[k] = (offset_h, offset_w) of candidate box k in the resized frame, each
+ * in [0, max(rh - crop_h, 0)] x [0, max(rw - crop_w, 0)]; the box is clipped to the frame.  flip: 1 mirrors the cropped
+ * extent horizontally.  Photometric steps fire when their flag is 1, in the order brightness (+beta), contrast if
+ * contrast_mode == 1 (*contrast_alpha), saturation (*saturation_alpha on S of HSV), hue (H + hue_delta mod 180), contrast
+ * if contrast_mode == 0, each step in uint8 arithmetic as mmseg's PhotoMetricDistortion computes it. */
+typedef struct {
+  const uint8_t* img;
+  const void* label;
+  int32_t h, w;
+  int32_t rh, rw;
+  int32_t num_candidates;        /* 1 .. 11 */
+  int32_t offsets[11][2];
+  int32_t flip;
+  int32_t contrast_mode;
+  int32_t brightness, contrast, saturation, hue;
+  float beta, contrast_alpha, saturation_alpha;
+  int32_t hue_delta;
+} ledb200_aug_sample;
+/* ledb200_crop_select: RandomCrop's cat_max_ratio loop for every sample at once.  Candidate k < num_candidates - 1 is
+ *   accepted when the nearest-resized label inside its box, ignore_index (in [0, 255]) dropped, holds more than one class
+ *   and max(count) / sum(count) < cat_max_ratio (float64); label values outside [0, 255] count as one class.
+ *   crop_index [N] int32 (device) receives the first accepted candidate, else num_candidates - 1. */
+int ledb200_crop_select(const ledb200_aug_sample* samples, int32_t N, int32_t crop_h, int32_t crop_w, int32_t label_dtype,
+                        double cat_max_ratio, int32_t ignore_index, int32_t* crop_index, void* stream);
+/* ledb200_train_augment: out [N,3,Hp,Wp] fp32 and label_out [N,Hp,Wp] int64 of the augmented batch, the box of sample n
+ *   being candidate crop_index[n] (device; nullable when every sample has one candidate).  Channel c of out reads
+ *   augmented channel 2 - c when swap_rb, then (v - mean3[c]) / std3[c] when mean3 / std3 (HOST, both or neither) are
+ *   given; pixels right of / below the cropped extent get pad_val and seg_pad_val. */
+int ledb200_train_augment(const ledb200_aug_sample* samples, int32_t N, int32_t crop_h, int32_t crop_w,
+                          int32_t label_dtype, const int32_t* crop_index, int32_t swap_rb, const float* mean3,
+                          const float* std3, float pad_val, float* out, int32_t Hp, int32_t Wp, int64_t* label_out,
+                          int32_t seg_pad_val, void* stream);
+
 /* ---- layer-level operators for module compositions outside the R0 plan (the LED wiring, led_variant.py) ---------------
  * A conv layer handle is ONE mmcv ConvModule (mmcv/cnn/bricks/conv_module.py; conv k = 1 | 3, stride 1 | 2, padding k/2)
  * whose BatchNorm the caller folded into `weight` (OIHW, HOST fp32) / `bias` (nullable); `pre_scale` / `pre_shift`

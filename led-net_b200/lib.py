@@ -36,7 +36,7 @@ SYMBOLS = [
     'ledb200_mfaf_param_floats', 'ledb200_mfaf_workspace_bytes', 'ledb200_mfaf_forward',
     'ledb200_getb_param_floats', 'ledb200_getb_create', 'ledb200_getb_destroy', 'ledb200_getb_forward',
     'ledb200_postprocess', 'ledb200_slide_accumulate', 'ledb200_slide_finalize', 'ledb200_slide_merge', 'ledb200_stack_pad',
-    'ledb200_tta_merge',
+    'ledb200_tta_merge', 'ledb200_crop_select', 'ledb200_train_augment',
     'ledb200_seam_param_floats', 'ledb200_seam_workspace_bytes', 'ledb200_seam_forward',
     'ledb200_conv_layer_create', 'ledb200_conv_layer_forward', 'ledb200_conv_layer_destroy',
     'ledb200_avgpool2d', 'ledb200_resize_bilinear', 'ledb200_add_relu', 'ledb200_conv_layer_forward_image',
@@ -60,6 +60,16 @@ class TtaView(C.Structure):
     """ledb200_tta_view: image n of the view at logits + n * image_stride (fp32 elements); padding / flip to undo."""
     _fields_ = [('logits', C.c_void_p), ('image_stride', C.c_int64), ('H', C.c_int32), ('W', C.c_int32),
                 ('pad_lrtb', C.c_int32 * 4), ('flip', C.c_int32)]
+
+
+class AugSample(C.Structure):
+    """ledb200_aug_sample: one sample's source buffers, resized size, candidate boxes, flip and photometric draws."""
+    _fields_ = [('img', C.c_void_p), ('label', C.c_void_p), ('h', C.c_int32), ('w', C.c_int32),
+                ('rh', C.c_int32), ('rw', C.c_int32), ('num_candidates', C.c_int32),
+                ('offsets', (C.c_int32 * 2) * 11), ('flip', C.c_int32), ('contrast_mode', C.c_int32),
+                ('brightness', C.c_int32), ('contrast', C.c_int32), ('saturation', C.c_int32), ('hue', C.c_int32),
+                ('beta', C.c_float), ('contrast_alpha', C.c_float), ('saturation_alpha', C.c_float),
+                ('hue_delta', C.c_int32)]
 
 
 _lib = None
@@ -164,6 +174,9 @@ def get():
     lib.ledb200_slide_merge.argtypes = [vp, i32, vp, vp] + [i32] * 6 + [vp, vp, i32, vp]
     lib.ledb200_stack_pad.argtypes = [vp, i32, i32, i32, i32, vp, vp, f32, vp, i32, i32, vp, i32, vp, i32, vp]
     lib.ledb200_tta_merge.argtypes = [C.POINTER(TtaView)] + [i32] * 7 + [f32, vp, i32, vp, vp]
+    lib.ledb200_crop_select.argtypes = [C.POINTER(AugSample)] + [i32] * 4 + [C.c_double, i32, vp, vp]
+    lib.ledb200_train_augment.argtypes = [C.POINTER(AugSample)] + [i32] * 4 + [vp, i32, vp, vp, f32, vp, i32, i32, vp,
+                                                                               i32, vp]
     lib.ledb200_conv_layer_create.argtypes = [vp, vp, vp, vp] + [i32] * 5 + [C.POINTER(vp)]
     lib.ledb200_conv_layer_forward.argtypes = [vp, vp, vp, vp] + [i32] * 9 + [vp]
     lib.ledb200_conv_layer_destroy.argtypes = [vp]

@@ -231,3 +231,72 @@ def stack_pad(img, out, swap_rb=False, mean=None, std=None, pad_val=0.0, label=N
                                       L.torch_dtype_code(label) if label is not None else L.U8, _p(label_out),
                                       int(seg_pad_val), L.stream_ptr(img.device)), 'ledb200_stack_pad')
     return out
+
+
+MAX_AUG_SAMPLES = 64          # ledb200_train_augment's descriptors per call
+
+
+def _aug_desc(p, img, lab):
+    d = L.AugSample()
+    d.img, d.label = img.data_ptr(), lab.data_ptr()
+    d.h, d.w = img.shape[1], img.shape[2]
+    d.rh, d.rw = (int(v) for v in p['resized_hw'])
+    cands = p['candidates']
+    if not 1 <= len(cands) <= 11:
+        raise L.LedB200Error(f'train_augment: {len(cands)} candidate boxes (1 .. 11 per sample)')
+    d.num_candidates = len(cands)
+    for k, (oy, ox) in enumerate(cands):
+        d.offsets[k][0], d.offsets[k][1] = int(oy), int(ox)
+    d.flip = int(bool(p['flip']))
+    d.contrast_mode = int(p['contrast_mode'])
+    d.brightness, d.beta = p['brightness'] is not None, p['brightness'] or 0.0
+    d.contrast, d.contrast_alpha = p['contrast'] is not None, p['contrast'] or 1.0
+    d.saturation, d.saturation_alpha = p['saturation'] is not None, p['saturation'] or 1.0
+    d.hue, d.hue_delta = p['hue'] is not None, int(p['hue'] or 0)
+    return d
+
+
+def train_augment(imgs, labels, params, crop_size, out, label_out, cat_max_ratio=1.0, ignore_index=255,
+                  swap_rb=False, mean=None, std=None, pad_val=0.0, seg_pad_val=255, crop_index=None):
+    """RandomResize -> RandomCrop -> RandomFlip -> PhotoMetricDistortion -> SegDataPreProcessor on the device, with the
+    random draws given: imgs [3,h,w] uint8 (BGR as decoded), labels [h,w] or [1,h,w] uint8 / int64, params one dict per
+    sample (lednet_b200.augment.draw_sample's format: resized_hw, candidates [(offset_h, offset_w)] (1 .. 11),
+    flip, brightness / contrast / saturation / hue (None when the step does not fire), contrast_mode).
+    crop_size (h, w); out [N,3,Hp,Wp] fp32 and label_out [N,Hp,Wp] int64, contiguous.  When a sample has several
+    candidates, crop_select picks the first that passes cat_max_ratio (the last one otherwise) into crop_index
+    (int32 [N], allocated when None) and that box is used.  Returns crop_index (None when every sample has one)."""
+    N = len(imgs)
+    assert len(labels) == N == len(params) and N >= 1
+    _need_cuda(out, label_out, *imgs, *labels)
+    assert out.is_contiguous() and out.dtype == torch.float32 and out.shape[:2] == (N, 3)
+    assert label_out.is_contiguous() and label_out.dtype == torch.int64 and label_out.numel() == N * out[0, 0].numel()
+    for t in imgs:
+        if t.dtype != torch.uint8 or t.dim() != 3 or t.shape[0] != 3:
+            raise L.LedB200Error('train_augment: images are [3, h, w] uint8')
+    imgs = [t.contiguous() for t in imgs]
+    ldt = torch.uint8 if all(t.dtype == torch.uint8 for t in labels) else torch.int64
+    labels = [t.reshape(t.shape[-2:]).to(ldt).contiguous() for t in labels]
+    for t, lab in zip(imgs, labels):
+        if tuple(lab.shape) != tuple(t.shape[1:]):
+            raise L.LedB200Error('train_augment: a label differs in size from its image')
+    ch, cw = (int(v) for v in crop_size)
+    Hp, Wp = out.shape[-2:]
+    select = any(len(p['candidates']) > 1 for p in params)
+    if select and crop_index is None:
+        crop_index = torch.empty(N, dtype=torch.int32, device=out.device)
+    lab_code = L.torch_dtype_code(labels[0])
+    m3 = (C.c_float * 3)(*[float(v) for v in mean]) if mean is not None else None
+    s3 = (C.c_float * 3)(*[float(v) for v in std]) if std is not None else None
+    lib, st = L.get(), L.stream_ptr(out.device)
+    lout = label_out.view(N, Hp, Wp)
+    for i0 in range(0, N, MAX_AUG_SAMPLES):
+        i1 = min(N, i0 + MAX_AUG_SAMPLES)
+        arr = (L.AugSample * (i1 - i0))(*[_aug_desc(params[i], imgs[i], labels[i]) for i in range(i0, i1)])
+        ci = crop_index[i0:i1] if crop_index is not None else None
+        if select:
+            L.check(lib.ledb200_crop_select(arr, i1 - i0, ch, cw, lab_code, float(cat_max_ratio), int(ignore_index),
+                                            _p(ci), st), 'ledb200_crop_select')
+        L.check(lib.ledb200_train_augment(arr, i1 - i0, ch, cw, lab_code, _p(ci), int(bool(swap_rb)), m3, s3,
+                                          float(pad_val), _p(out[i0:i1]), Hp, Wp, _p(lout[i0:i1]), int(seg_pad_val),
+                                          st), 'ledb200_train_augment')
+    return crop_index
