@@ -499,6 +499,26 @@ int ledb200_train_augment(const ledb200_aug_sample* samples, int32_t N, int32_t 
                           const float* std3, float pad_val, float* out, int32_t Hp, int32_t Wp, int64_t* label_out,
                           int32_t seg_pad_val, void* stream);
 
+/* ---- test-time views (csrc/augment.cu) ---------------------------------------------------------------------------------
+ * mmcv Resize (keep_ratio; cv2 INTER_LINEAR, the same taps as ledb200_train_augment) of a decoded image, optionally
+ * followed by RandomFlip (horizontal), then SegDataPreProcessor's swap / normalisation / padding: the views of
+ * TestTimeAug and the test pipeline's own Resize.  One descriptor per (image, resized size), HOST array.
+ * src: [3,h,w] uint8 CHW as decoded (BGR).  (rh, rw): the resized size, computed by the caller with mmcv's arithmetic.
+ * out / out_flip: [3,Hp,Wp] fp32 of the unflipped / horizontally flipped view, either may be NULL but not both; a flip
+ * pair costs one sampling pass. */
+typedef struct {
+  const uint8_t* src;
+  float* out;
+  float* out_flip;
+  int32_t h, w;
+  int32_t rh, rw;
+} ledb200_view_desc;
+/* ledb200_view_resize: 1 <= n <= 64 views of one padded size Hp x Wp (rh <= Hp, rw <= Wp).  Channel c of an output reads
+ *   resized channel 2 - c when swap_rb, then (v - mean3[c]) / std3[c] when mean3 / std3 (HOST, both or neither) are
+ *   given; pixels right of / below the resized frame get pad_val. */
+int ledb200_view_resize(const ledb200_view_desc* views, int32_t n, int32_t Hp, int32_t Wp, int32_t swap_rb,
+                        const float* mean3, const float* std3, float pad_val, void* stream);
+
 /* ---- layer-level operators for module compositions outside the R0 plan (the LED wiring, led_variant.py) ---------------
  * A conv layer handle is ONE mmcv ConvModule (mmcv/cnn/bricks/conv_module.py; conv k = 1 | 3, stride 1 | 2, padding k/2)
  * whose BatchNorm the caller folded into `weight` (OIHW, HOST fp32) / `bias` (nullable); `pre_scale` / `pre_shift`

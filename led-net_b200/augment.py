@@ -77,6 +77,69 @@ def parse_pipeline(pipeline):
                 hue_delta=int(pmd.get('hue_delta', 18)))
 
 
+def parse_resize(t):
+    """One test-time mmcv Resize dict -> ('scale', (a, b)) or ('scale_factor', r).  keep_ratio=True with cv2's bilinear
+    only; exactly one of a `scale` pair or a float `scale_factor`; anything else raises NotImplementedError."""
+    if not isinstance(t, dict) or t.get('type') != 'Resize':
+        raise NotImplementedError(f'a Resize dict is supported here, got {t!r}')
+    _check_keys(t, ('scale', 'scale_factor', 'keep_ratio', 'clip_object_border', 'backend', 'interpolation'))
+    if t.get('keep_ratio') is not True:
+        raise NotImplementedError('Resize: only keep_ratio=True')
+    if t.get('interpolation', 'bilinear') != 'bilinear' or t.get('backend', 'cv2') != 'cv2':
+        raise NotImplementedError("Resize: only interpolation='bilinear' with backend='cv2'")
+    scale, factor = t.get('scale'), t.get('scale_factor')
+    if (scale is None) == (factor is None):
+        raise NotImplementedError('Resize: exactly one of scale and scale_factor')
+    if scale is not None:
+        scale = _pair(scale, 'Resize scale')
+        if not all(isinstance(v, int) and v > 0 for v in scale):
+            raise NotImplementedError(f'Resize: scale must be two positive ints, got {scale!r}')
+        return 'scale', scale
+    if not isinstance(factor, float) or not factor > 0:
+        raise NotImplementedError(f'Resize: scale_factor must be one positive float, got {factor!r}')
+    return 'scale_factor', factor
+
+
+def view_size(h, w, resize):
+    """mmcv Resize.transform (keep_ratio) of an (h, w) image: `_scale_size((w, h), scale_factor)` when the dict gives a
+    factor, then mmcv.imrescale's rescale_size.  Returns (rh, rw)."""
+    kind, v = resize
+    scale = (int(w * v + 0.5), int(h * v + 0.5)) if kind == 'scale_factor' else v
+    return rescale_size(h, w, scale)
+
+
+def parse_flip(t):
+    """One test-time RandomFlip dict -> flip (bool): prob exactly 0. or 1., direction='horizontal'."""
+    if not isinstance(t, dict) or t.get('type') != 'RandomFlip':
+        raise NotImplementedError(f'a RandomFlip dict is supported here, got {t!r}')
+    _check_keys(t, ('prob', 'direction'))
+    prob = t.get('prob')
+    if not isinstance(prob, float) or prob not in (0., 1.):
+        raise NotImplementedError(f'RandomFlip: prob must be exactly 0. or 1. at test time, got {prob!r}')
+    if t.get('direction', 'horizontal') != 'horizontal':
+        raise NotImplementedError("RandomFlip: direction='horizontal' only")
+    return prob == 1.
+
+
+def parse_tta_transforms(transforms):
+    """The first two lists of TestTimeAug.transforms, verbatim: [[Resize ...], [RandomFlip ...]] (the flip list is
+    optional) -> (resizes, flips).  Each flip state may appear once."""
+    if not isinstance(transforms, (list, tuple)) or len(transforms) not in (1, 2):
+        raise NotImplementedError('tta_transforms: [[Resize, ...]] or [[Resize, ...], [RandomFlip, ...]]')
+    if not all(isinstance(ts, (list, tuple)) and len(ts) > 0 for ts in transforms):
+        raise NotImplementedError('tta_transforms: each entry is a non-empty list of transform dicts')
+    resizes = [parse_resize(t) for t in transforms[0]]
+    flips = [parse_flip(t) for t in transforms[1]] if len(transforms) == 2 else [False]
+    if len(set(flips)) != len(flips):
+        raise NotImplementedError('tta_transforms: each flip state at most once')
+    return resizes, flips
+
+
+def view_meta(h, w, rh, rw):
+    """The metainfo mmcv Resize (keep_ratio) leaves on an (h, w) image resized to (rh, rw)."""
+    return dict(img_shape=(rh, rw), scale_factor=(rw / w, rh / h), keep_ratio=True)
+
+
 def draw_sample(rng, cfg, h, w):
     """One sample's random parameters, drawn from `rng` (numpy Generator) in the reference's order: the resize ratio,
     the crop boxes (offset_h then offset_w each), the flip, then PhotoMetricDistortion's draws.  All 11 crop boxes are
@@ -116,6 +179,17 @@ def draw_sample(rng, cfg, h, w):
     return p
 
 
+def device_images(inputs):
+    """The decoded uint8 [3, h, w] images of a batch (list or [N, 3, h, w] tensor) on the device; anything else raises
+    NotImplementedError."""
+    inputs = list(inputs) if isinstance(inputs, (list, tuple)) else list(inputs.unbind(0))
+    if not inputs or any(not isinstance(t, torch.Tensor) or t.dtype != torch.uint8 or t.dim() != 3 or t.shape[0] != 3
+                         for t in inputs):
+        raise NotImplementedError('the device augmentation takes decoded uint8 [3, h, w] images')
+    dev = next((t.device for t in inputs if t.is_cuda), None) or torch.device('cuda', torch.cuda.current_device())
+    return [t.to(dev, non_blocking=True) for t in inputs]
+
+
 @MODELS.register_module()
 class DeviceAugSegDataPreProcessor(SegDataPreProcessor):
     """SegDataPreProcessor that also runs the config's training augmentations.
@@ -127,11 +201,22 @@ class DeviceAugSegDataPreProcessor(SegDataPreProcessor):
     CPU pipeline, plus the metainfo those transforms leave (img_shape, scale_factor, flip, flip_direction, pad_shape,
     padding_size) and the drawn parameters under `aug_params` (with `crop_index`, the chosen box as a device tensor).
     The crop boxes are all drawn up front (see `draw_sample`): the random stream differs from the reference's lazy
-    redraws, the distribution does not.  forward(data, training=False) is SegDataPreProcessor.forward."""
+    redraws, the distribution does not.
 
-    def __init__(self, train_pipeline=None, seed=0, **kwargs):
+    `test_pipeline` (optional) holds the test pipeline's one Resize dict (keep_ratio=True, `scale` pair or float
+    `scale_factor`), moved verbatim from the dataset: forward(data, training=False) then resizes the decoded uint8 images
+    with cv2's INTER_LINEAR on the device, fused with the swap / normalisation / test_cfg padding (ops.view_resize), and
+    sets img_shape, scale_factor and keep_ratio (ori_shape stays the decoded size, so predict resizes back to it).
+    Without it, forward(data, training=False) is SegDataPreProcessor.forward."""
+
+    def __init__(self, train_pipeline=None, seed=0, test_pipeline=None, **kwargs):
         super().__init__(**kwargs)
         self.aug = parse_pipeline(train_pipeline)
+        self.test_resize = None
+        if test_pipeline is not None:
+            if not isinstance(test_pipeline, (list, tuple)) or len(test_pipeline) != 1:
+                raise NotImplementedError('test_pipeline must be exactly [Resize(...)]')
+            self.test_resize = parse_resize(test_pipeline[0])
         rank = 0
         if torch.distributed.is_available() and torch.distributed.is_initialized():
             rank = torch.distributed.get_rank()
@@ -143,15 +228,13 @@ class DeviceAugSegDataPreProcessor(SegDataPreProcessor):
 
     def forward(self, data, training=False):
         if not training:
-            return super().forward(data, False)
-        inputs = data['inputs']
+            if self.test_resize is None:
+                return super().forward(data, False)
+            return self._forward_test(data)
         samples = data.get('data_samples', None)
         assert samples is not None, 'During training, `data_samples` must be define.'
-        inputs = list(inputs) if isinstance(inputs, (list, tuple)) else list(inputs.unbind(0))
-        dev = next((t.device for t in inputs if t.is_cuda), None) or torch.device('cuda', torch.cuda.current_device())
-        inputs = [t.to(dev, non_blocking=True) for t in inputs]
-        if any(t.dtype != torch.uint8 or t.dim() != 3 or t.shape[0] != 3 for t in inputs):
-            raise NotImplementedError('the device augmentation takes decoded uint8 [3, h, w] images')
+        inputs = device_images(data['inputs'])
+        dev = inputs[0].device
         labels = [s['gt_sem_seg']['data'].to(dev, non_blocking=True) for s in samples]
         params = self.draw([tuple(t.shape[-2:]) for t in inputs])
         ch, cw = self.aug['crop_size']
@@ -172,4 +255,30 @@ class DeviceAugSegDataPreProcessor(SegDataPreProcessor):
                             flip_direction='horizontal' if p['flip'] else None, pad_shape=(Hp, Wp),
                             padding_size=(0, Wp - ew, 0, Hp - eh),
                             aug_params=dict(p, crop_index=crop_index[i] if crop_index is not None else 0))
+        return dict(inputs=out, data_samples=samples)
+
+    def _forward_test(self, data):
+        """The test pipeline's Resize + SegDataPreProcessor.forward(training=False) in one launch per 64 images."""
+        samples = data.get('data_samples', None)
+        inputs = device_images(data['inputs'])
+        src = [tuple(t.shape[-2:]) for t in inputs]
+        sizes = [view_size(h, w, self.test_resize) for h, w in src]
+        if self.test_cfg:
+            Hp, Wp = self._padded_hw(sizes, self.test_cfg.get('size', None), self.test_cfg.get('size_divisor', None))
+        else:
+            assert all(sh == sizes[0] for sh in sizes), 'The image size in a batch should be the same.'
+            Hp, Wp = sizes[0]
+        out = torch.empty((len(inputs), 3, Hp, Wp), dtype=torch.float32, device=inputs[0].device)
+        mean, std = self.mean_std() if self._enable_normalize else (None, None)
+        ops.view_resize(inputs, sizes, out=out, swap_rb=self.channel_conversion, mean=mean, std=std,
+                        pad_val=self.pad_val)
+        if samples is not None:
+            for s, (h, w), (rh, rw) in zip(samples, src, sizes):
+                if not isinstance(s, dict):
+                    continue
+                m = _meta(s)
+                m.update(view_meta(h, w, rh, rw))
+                m.setdefault('ori_shape', (h, w))
+                if self.test_cfg:
+                    m.update(img_padding_size=(0, Wp - rw, 0, Hp - rh), pad_shape=(Hp, Wp))
         return dict(inputs=out, data_samples=samples)

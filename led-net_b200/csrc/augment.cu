@@ -11,6 +11,9 @@
 //      the cropped extent, the resized-frame coordinate, cv2's fixed-point INTER_LINEAR taps on the uint8 CHW source,
 //      the photometric chain in cv2 / numpy's own integer and float32 arithmetic, the channel swap and normalisation.
 //      The label is cv2's INTER_NEAREST of the source label.  Only the outputs reach memory.
+//  * view_resize_kernel   : the test-time views (TestTimeAug's Resize x RandomFlip, or the test pipeline's Resize): one
+//      thread per pixel of the padded frame, the same INTER_LINEAR taps (sample_linear), written to the unflipped view
+//      and to the mirrored pixel of the flipped one, then stack_pad_kernel's swap and normalisation, bit for bit.
 //
 // The restatement these kernels are checked against is tests/augment_oracle.py; the cv2 formulations it follows:
 //   INTER_LINEAR (imgproc/resize.cpp): scale = 1 / (dst / src) in double, fx = (float)((dx + 0.5) * scale - 0.5),
@@ -135,6 +138,25 @@ __device__ __forceinline__ void linear_taps(int d, double scale, int src, int& i
   c1 = (int)rintf(__fmul_rn(f, 2048.f));
 }
 
+// cv2 INTER_LINEAR of the uint8 CHW source [3, h, w] at resized-frame pixel (ry, rx): the taps of both axes, the horizontal
+// sums into int and the vertical pass in the SIMD rounding.  c[ch] is the resized uint8 value of source channel ch.
+__device__ __forceinline__ void sample_linear(const uint8_t* img, int h, int w, double sy, double sx, int ry, int rx,
+                                              int* c) {
+  int y0, y1, b0, b1, x0, x1, a0, a1;
+  linear_taps(ry, sy, h, y0, y1, b0, b1);
+  linear_taps(rx, sx, w, x0, x1, a0, a1);
+  const int64_t plane = (int64_t)h * w;
+  const uint8_t* r0p = img + (int64_t)y0 * w;
+  const uint8_t* r1p = img + (int64_t)y1 * w;
+#pragma unroll
+  for (int ch = 0; ch < 3; ++ch) {
+    const int S0 = __ldg(r0p + ch * plane + x0) * a0 + __ldg(r0p + ch * plane + x1) * a1;
+    const int S1 = __ldg(r1p + ch * plane + x0) * a0 + __ldg(r1p + ch * plane + x1) * a1;
+    const int v = ((((S0 >> 4) * b0) >> 16) + (((S1 >> 4) * b1) >> 16) + 2) >> 2;
+    c[ch] = min(max(v, 0), 255);
+  }
+}
+
 // numpy: clip(x.astype(float32) * alpha + beta, 0, 255).astype(uint8), two roundings, truncation
 __device__ __forceinline__ int convert_u8(int x, float alpha, float beta) {
   const float v = __fadd_rn(__fmul_rn((float)x, alpha), beta);
@@ -215,20 +237,8 @@ __global__ void __launch_bounds__(256) train_augment_kernel(const __grid_constan
   *lout = (int64_t)reinterpret_cast<const TL*>(s.label)[(int64_t)nearest_src(ry, s.sy, s.h) * s.w +
                                                         nearest_src(rx, s.sx, s.w)];
 
-  int y0, y1, b0, b1, x0, x1, a0, a1;
-  linear_taps(ry, s.sy, s.h, y0, y1, b0, b1);
-  linear_taps(rx, s.sx, s.w, x0, x1, a0, a1);
-  const int64_t plane = (int64_t)s.h * s.w;
-  const uint8_t* r0p = s.img + (int64_t)y0 * s.w;
-  const uint8_t* r1p = s.img + (int64_t)y1 * s.w;
   int c[3];
-#pragma unroll
-  for (int ch = 0; ch < 3; ++ch) {
-    const int S0 = __ldg(r0p + ch * plane + x0) * a0 + __ldg(r0p + ch * plane + x1) * a1;
-    const int S1 = __ldg(r1p + ch * plane + x0) * a0 + __ldg(r1p + ch * plane + x1) * a1;
-    const int v = ((((S0 >> 4) * b0) >> 16) + (((S1 >> 4) * b1) >> 16) + 2) >> 2;
-    c[ch] = min(max(v, 0), 255);
-  }
+  sample_linear(s.img, s.h, s.w, s.sy, s.sx, ry, rx, c);
   // PhotoMetricDistortion: brightness; contrast if mode 1; saturation; hue; contrast if mode 0
   if (s.brightness) {
 #pragma unroll
@@ -257,6 +267,53 @@ __global__ void __launch_bounds__(256) train_augment_kernel(const __grid_constan
   for (int ch = 0; ch < 3; ++ch) {
     const float v = (float)c[a.swap_rb ? 2 - ch : ch];
     out[ch * HWp] = a.normalize ? __fdiv_rn(v - a.mean[ch], a.stdv[ch]) : v;
+  }
+}
+
+// ---- test-time views: mmcv Resize (keep_ratio, cv2 INTER_LINEAR) + RandomFlip (horizontal) + SegDataPreProcessor ----
+constexpr int kViewMax = 64;
+
+struct View {
+  const uint8_t* src;            // [3, h, w] CHW
+  float* out;                    // [3, Hp, Wp] or null
+  float* out_flip;               // [3, Hp, Wp] or null
+  int h, w, rh, rw;
+  double sy, sx;                 // cv2's source-per-destination scales, as in fill_samples
+};
+
+struct ViewArgs {
+  View v[kViewMax];
+  int n, Hp, Wp, swap_rb, normalize;
+  float mean[3], stdv[3], pad_val;
+};
+
+// One thread per pixel of the padded frame of one view.  Inside the resized frame the pixel is sampled once and written
+// to out[y][x] and to out_flip[y][rw - 1 - x]; outside it both outputs get pad_val at [y][x].
+__global__ void __launch_bounds__(256) view_resize_kernel(const __grid_constant__ ViewArgs a) {
+  const int64_t HWp = (int64_t)a.Hp * a.Wp;
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (int64_t)a.n * HWp) return;
+  const int n = (int)(idx / HWp);
+  const int64_t pix = idx % HWp;
+  const int y = (int)(pix / a.Wp), x = (int)(pix % a.Wp);
+  const View& v = a.v[n];
+  if (y >= v.rh || x >= v.rw) {
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) {
+      if (v.out) v.out[ch * HWp + pix] = a.pad_val;
+      if (v.out_flip) v.out_flip[ch * HWp + pix] = a.pad_val;
+    }
+    return;
+  }
+  int c[3];
+  sample_linear(v.src, v.h, v.w, v.sy, v.sx, y, x, c);
+  const int64_t fpix = pix + (v.rw - 1 - 2 * x);
+#pragma unroll
+  for (int ch = 0; ch < 3; ++ch) {
+    const float f = (float)c[a.swap_rb ? 2 - ch : ch];
+    const float o = a.normalize ? __fdiv_rn(f - a.mean[ch], a.stdv[ch]) : f;   // stack_pad_kernel's expression
+    if (v.out) v.out[ch * HWp + pix] = o;
+    if (v.out_flip) v.out_flip[ch * HWp + fpix] = o;
   }
 }
 
@@ -347,6 +404,32 @@ int ledb200_train_augment(const ledb200_aug_sample* samples, int32_t N, int32_t 
   if (label_dtype == LEDB200_I64) train_augment_kernel<int64_t><<<grid, 256, 0, st>>>(a);
   else train_augment_kernel<uint8_t><<<grid, 256, 0, st>>>(a);
   LEDB_LAUNCH_OK("train_augment_kernel");
+  return LEDB200_OK;
+}
+
+int ledb200_view_resize(const ledb200_view_desc* views, int32_t n, int32_t Hp, int32_t Wp, int32_t swap_rb,
+                        const float* mean3, const float* std3, float pad_val, void* stream) {
+  if (!views) return fail(LEDB200_EINVAL, "view_resize: null view descriptors");
+  if (n < 1 || n > kViewMax) return fail(LEDB200_EINVAL, "view_resize: between 1 and 64 views per call");
+  if ((mean3 == nullptr) != (std3 == nullptr)) return fail(LEDB200_EINVAL, "view_resize: mean and std come together");
+  ViewArgs a;
+  for (int i = 0; i < n; ++i) {
+    const ledb200_view_desc& d = views[i];
+    if (!d.src) return fail(LEDB200_EINVAL, "view_resize: null source image");
+    if (!d.out && !d.out_flip) return fail(LEDB200_EINVAL, "view_resize: a view needs out or out_flip");
+    if (d.h < 1 || d.w < 1 || d.rh < 1 || d.rw < 1) return fail(LEDB200_EINVAL, "view_resize: empty image or resized frame");
+    if (d.rh > Hp || d.rw > Wp) return fail(LEDB200_EINVAL, "view_resize: the padded size is smaller than a resized view");
+    View& v = a.v[i];
+    v.src = d.src; v.out = d.out; v.out_flip = d.out_flip;
+    v.h = d.h; v.w = d.w; v.rh = d.rh; v.rw = d.rw;
+    v.sy = 1.0 / ((double)d.rh / d.h);
+    v.sx = 1.0 / ((double)d.rw / d.w);
+  }
+  a.n = n; a.Hp = Hp; a.Wp = Wp; a.swap_rb = swap_rb ? 1 : 0; a.normalize = mean3 ? 1 : 0; a.pad_val = pad_val;
+  for (int c = 0; c < 3; ++c) { a.mean[c] = mean3 ? mean3[c] : 0.f; a.stdv[c] = std3 ? std3[c] : 1.f; }
+  const unsigned grid = (unsigned)ceil_div64((int64_t)n * Hp * Wp, 256);
+  view_resize_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(a);
+  LEDB_LAUNCH_OK("view_resize_kernel");
   return LEDB200_OK;
 }
 

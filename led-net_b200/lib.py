@@ -36,7 +36,7 @@ SYMBOLS = [
     'ledb200_mfaf_param_floats', 'ledb200_mfaf_workspace_bytes', 'ledb200_mfaf_forward',
     'ledb200_getb_param_floats', 'ledb200_getb_create', 'ledb200_getb_destroy', 'ledb200_getb_forward',
     'ledb200_postprocess', 'ledb200_slide_accumulate', 'ledb200_slide_finalize', 'ledb200_slide_merge', 'ledb200_stack_pad',
-    'ledb200_tta_merge', 'ledb200_crop_select', 'ledb200_train_augment',
+    'ledb200_tta_merge', 'ledb200_crop_select', 'ledb200_train_augment', 'ledb200_view_resize',
     'ledb200_seam_param_floats', 'ledb200_seam_workspace_bytes', 'ledb200_seam_forward',
     'ledb200_conv_layer_create', 'ledb200_conv_layer_forward', 'ledb200_conv_layer_destroy',
     'ledb200_avgpool2d', 'ledb200_resize_bilinear', 'ledb200_add_relu', 'ledb200_conv_layer_forward_image',
@@ -70,6 +70,12 @@ class AugSample(C.Structure):
                 ('brightness', C.c_int32), ('contrast', C.c_int32), ('saturation', C.c_int32), ('hue', C.c_int32),
                 ('beta', C.c_float), ('contrast_alpha', C.c_float), ('saturation_alpha', C.c_float),
                 ('hue_delta', C.c_int32)]
+
+
+class ViewDesc(C.Structure):
+    """ledb200_view_desc: one decoded uint8 [3,h,w] source, its resized size and the unflipped / flipped outputs."""
+    _fields_ = [('src', C.c_void_p), ('out', C.c_void_p), ('out_flip', C.c_void_p), ('h', C.c_int32), ('w', C.c_int32),
+                ('rh', C.c_int32), ('rw', C.c_int32)]
 
 
 _lib = None
@@ -177,6 +183,7 @@ def get():
     lib.ledb200_crop_select.argtypes = [C.POINTER(AugSample)] + [i32] * 4 + [C.c_double, i32, vp, vp]
     lib.ledb200_train_augment.argtypes = [C.POINTER(AugSample)] + [i32] * 4 + [vp, i32, vp, vp, f32, vp, i32, i32, vp,
                                                                                i32, vp]
+    lib.ledb200_view_resize.argtypes = [C.POINTER(ViewDesc)] + [i32] * 4 + [vp, vp, f32, vp]
     lib.ledb200_conv_layer_create.argtypes = [vp, vp, vp, vp] + [i32] * 5 + [C.POINTER(vp)]
     lib.ledb200_conv_layer_forward.argtypes = [vp, vp, vp, vp] + [i32] * 9 + [vp]
     lib.ledb200_conv_layer_destroy.argtypes = [vp]

@@ -300,3 +300,44 @@ def train_augment(imgs, labels, params, crop_size, out, label_out, cat_max_ratio
                                           float(pad_val), _p(out[i0:i1]), Hp, Wp, _p(lout[i0:i1]), int(seg_pad_val),
                                           st), 'ledb200_train_augment')
     return crop_index
+
+
+MAX_VIEWS = 64                # ledb200_view_resize's descriptors per call
+
+
+def view_resize(imgs, resized_hw, out=None, out_flip=None, swap_rb=False, mean=None, std=None, pad_val=0.0):
+    """mmcv Resize (keep_ratio, cv2 INTER_LINEAR) + optional horizontal RandomFlip + SegDataPreProcessor on the device:
+    imgs N [3,h,w] uint8 (BGR as decoded), resized_hw one (rh, rw) for all or one per image (mmcv's arithmetic,
+    lednet_b200.augment.view_size).  out / out_flip: [N,3,Hp,Wp] fp32 contiguous (one may be None) receive the unflipped
+    / flipped view of image n at index n, swapped, normalised and padded with pad_val to Hp x Wp, as SegDataPreProcessor
+    writes a view the CPU pipeline resized.  Returns (out, out_flip)."""
+    N = len(imgs)
+    assert N >= 1 and (out is not None or out_flip is not None)
+    _need_cuda(out, out_flip, *imgs)
+    for t in imgs:
+        if t.dtype != torch.uint8 or t.dim() != 3 or t.shape[0] != 3:
+            raise L.LedB200Error('view_resize: images are [3, h, w] uint8')
+    imgs = [t.contiguous() for t in imgs]
+    if len(resized_hw) == 2 and not isinstance(resized_hw[0], (tuple, list)):
+        resized_hw = [resized_hw] * N
+    assert len(resized_hw) == N
+    ref = out if out is not None else out_flip
+    Hp, Wp = ref.shape[-2:]
+    for t in (out, out_flip):
+        if t is not None:
+            assert t.is_contiguous() and t.dtype == torch.float32 and tuple(t.shape) == (N, 3, Hp, Wp)
+    m3 = (C.c_float * 3)(*[float(v) for v in mean]) if mean is not None else None
+    s3 = (C.c_float * 3)(*[float(v) for v in std]) if std is not None else None
+    lib, st = L.get(), L.stream_ptr(ref.device)
+    for i0 in range(0, N, MAX_VIEWS):
+        i1 = min(N, i0 + MAX_VIEWS)
+        arr = (L.ViewDesc * (i1 - i0))()
+        for d, i in zip(arr, range(i0, i1)):
+            d.src = imgs[i].data_ptr()
+            d.out = out[i].data_ptr() if out is not None else None
+            d.out_flip = out_flip[i].data_ptr() if out_flip is not None else None
+            d.h, d.w = imgs[i].shape[1], imgs[i].shape[2]
+            d.rh, d.rw = (int(v) for v in resized_hw[i])
+        L.check(lib.ledb200_view_resize(arr, i1 - i0, Hp, Wp, int(bool(swap_rb)), m3, s3, float(pad_val), st),
+                'ledb200_view_resize')
+    return out, out_flip
