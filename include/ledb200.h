@@ -519,6 +519,21 @@ typedef struct {
 int ledb200_view_resize(const ledb200_view_desc* views, int32_t n, int32_t Hp, int32_t Wp, int32_t swap_rb,
                         const float* mean3, const float* std3, float pad_val, void* stream);
 
+/* ---- label maps -> PNG files (csrc/png.cu) ------------------------------------------------------------------------------
+ * What IoUMetric(output_dir=...) writes for each prediction (mmseg: Image.fromarray((pred + reduce_zero_label)
+ * .astype(np.uint8)).save(path)): an 8-bit grayscale PNG (colour type 0, no interlace) of (label + add) mod 256, one
+ * IDAT holding one zlib stream.  Files decode to exactly those pixels; they are not byte-identical to PIL's.
+ * ledb200_png_bound: the largest file an H x W map can give (headers plus the whole image in stored blocks), or
+ *   LEDB200_EINVAL when H or W < 1 or the map does not fit one IDAT chunk.
+ * ledb200_png_workspace_bytes: device workspace of ledb200_png_encode for N maps of H x W.
+ * ledb200_png_encode: labels [N,H,W] contiguous, dtype LEDB200_U8 | LEDB200_I64, add 0 | 1.  out (capacity N * bound)
+ *   receives the files back to back, file i at out[offsets[i] : offsets[i + 1]]; offsets: device int64 [N + 1].  The
+ *   host reads offsets, then offsets[N] bytes of out. */
+int64_t ledb200_png_bound(int32_t H, int32_t W);
+int64_t ledb200_png_workspace_bytes(int32_t N, int32_t H, int32_t W);
+int ledb200_png_encode(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, int32_t add, uint8_t* out,
+                       int64_t* offsets, void* workspace, void* stream);
+
 /* ---- layer-level operators for module compositions outside the R0 plan (the LED wiring, led_variant.py) ---------------
  * A conv layer handle is ONE mmcv ConvModule (mmcv/cnn/bricks/conv_module.py; conv k = 1 | 3, stride 1 | 2, padding k/2)
  * whose BatchNorm the caller folded into `weight` (OIHW, HOST fp32) / `bias` (nullable); `pre_scale` / `pre_shift`

@@ -37,6 +37,7 @@ SYMBOLS = [
     'ledb200_getb_param_floats', 'ledb200_getb_create', 'ledb200_getb_destroy', 'ledb200_getb_forward',
     'ledb200_postprocess', 'ledb200_slide_accumulate', 'ledb200_slide_finalize', 'ledb200_slide_merge', 'ledb200_stack_pad',
     'ledb200_tta_merge', 'ledb200_crop_select', 'ledb200_train_augment', 'ledb200_view_resize',
+    'ledb200_png_bound', 'ledb200_png_workspace_bytes', 'ledb200_png_encode',
     'ledb200_seam_param_floats', 'ledb200_seam_workspace_bytes', 'ledb200_seam_forward',
     'ledb200_conv_layer_create', 'ledb200_conv_layer_forward', 'ledb200_conv_layer_destroy',
     'ledb200_avgpool2d', 'ledb200_resize_bilinear', 'ledb200_add_relu', 'ledb200_conv_layer_forward_image',
@@ -184,6 +185,11 @@ def get():
     lib.ledb200_train_augment.argtypes = [C.POINTER(AugSample)] + [i32] * 4 + [vp, i32, vp, vp, f32, vp, i32, i32, vp,
                                                                                i32, vp]
     lib.ledb200_view_resize.argtypes = [C.POINTER(ViewDesc)] + [i32] * 4 + [vp, vp, f32, vp]
+    lib.ledb200_png_bound.argtypes = [i32, i32]
+    lib.ledb200_png_bound.restype = i64
+    lib.ledb200_png_workspace_bytes.argtypes = [i32, i32, i32]
+    lib.ledb200_png_workspace_bytes.restype = i64
+    lib.ledb200_png_encode.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp]
     lib.ledb200_conv_layer_create.argtypes = [vp, vp, vp, vp] + [i32] * 5 + [C.POINTER(vp)]
     lib.ledb200_conv_layer_forward.argtypes = [vp, vp, vp, vp] + [i32] * 9 + [vp]
     lib.ledb200_conv_layer_destroy.argtypes = [vp]

@@ -2,9 +2,12 @@
 
 Device work is one confusion-matrix kernel launch per image (csrc/metrics.cu) instead of two
 boolean gathers, three float32 `histc` calls and three device->host syncs; nothing leaves the GPU
-until `compute_metrics`.  Across ranks the (K+1) x K int64 matrix is summed with ONE NCCL
+until `compute_metrics`.  With `output_dir`, the predictions are written as PNG files encoded on the device
+(csrc/png.cu, one launch sequence per shape of a `process` call); only the files come back to the host.  Across ranks the (K+1) x K int64 matrix is summed with ONE NCCL
 all-reduce (2.9 KB at K=19) instead of mmengine's pickled `collect_results` object gather.
 """
+import logging
+import os
 from collections import OrderedDict
 
 import numpy as np
@@ -12,6 +15,20 @@ import torch
 
 from . import ops
 from .registry import METRICS
+
+
+def _is_main_process():
+    d = torch.distributed
+    return not (d.is_available() and d.is_initialized()) or d.get_rank() == 0
+
+
+def _sample_meta(sample, key, default=None):
+    """`key` of a data sample or of its `metainfo` (a SegDataSample or its dict form)."""
+    v = sample.get(key, None)
+    if v is None:
+        meta = sample.get('metainfo', None)
+        v = meta.get(key, None) if meta is not None else None
+    return default if v is None else v
 
 
 def _areas_from_cm(cm):
@@ -33,8 +50,8 @@ class IoUMetric:
         self.nan_to_num, self.beta = nan_to_num, beta
         self.collect_device, self.output_dir, self.format_only, self.prefix = \
             collect_device, output_dir, format_only, prefix
-        if output_dir is not None or format_only:
-            raise NotImplementedError('PNG dumping (format_only / output_dir) is outside the hot path')
+        if output_dir and _is_main_process():
+            os.makedirs(output_dir, exist_ok=True)
         self.results = []
         self.dataset_meta = None
         self._cm = None
@@ -43,22 +60,50 @@ class IoUMetric:
 
     # -- reference API --------------------------------------------------------------------
     def process(self, data_batch, data_samples):
-        """iou_metric.py:67-100: one entry per image in self.results (here: its int64 matrix)."""
-        num_classes = len(self.dataset_meta['classes'])
+        """iou_metric.py:67-100: one entry per image in self.results (here: its int64 matrix).  With `format_only`
+        no matrix is computed and `gt_sem_seg` may be missing.  With `output_dir`, each prediction is written to
+        `{splitext(basename(img_path))[0]}.png`, plus one when the sample's `reduce_zero_label` is set."""
+        preds = []
         for s in data_samples:
             pred = s['pred_sem_seg']['data'].squeeze()
-            label = s['gt_sem_seg']['data'].squeeze().to(pred.device)
-            self.results.append(ops.confusion_accumulate(pred, label, num_classes, self.ignore_index))
+            preds.append(pred)
+            if not self.format_only:
+                num_classes = len(self.dataset_meta['classes'])
+                label = s['gt_sem_seg']['data'].squeeze().to(pred.device)
+                self.results.append(ops.confusion_accumulate(pred, label, num_classes, self.ignore_index))
+                self._last = (pred, label, num_classes)
             self._n_samples += 1
-            self._last = (pred, label, num_classes)
+        if self.output_dir is not None:
+            self._write_pngs(preds, [_sample_meta(s, 'img_path') for s in data_samples],
+                             [bool(_sample_meta(s, 'reduce_zero_label', False)) for s in data_samples])
 
-    def process_batch(self, pred, label, num_classes=None):
-        """Batched fast path: accumulate a whole [N,H,W] prediction/label pair into the running matrix."""
-        k = num_classes or len(self.dataset_meta['classes'])
-        self._cm = ops.confusion_accumulate(pred, label, k, self.ignore_index, self._cm)
-        self._n_samples += int(pred.shape[0]) if pred.dim() == 3 else 1
-        self._last = (pred[-1] if pred.dim() == 3 else pred, label[-1] if label.dim() == 3 else label, k)
+    def process_batch(self, pred, label=None, num_classes=None, img_paths=None, reduce_zero_label=False):
+        """Batched fast path: accumulate a whole [N,H,W] prediction/label pair into the running matrix (not with
+        `format_only` or without a label), and with `output_dir` write image n to the PNG named from img_paths[n]."""
+        preds = list(pred) if pred.dim() == 3 else [pred]
+        if label is not None and not self.format_only:
+            k = num_classes or len(self.dataset_meta['classes'])
+            self._cm = ops.confusion_accumulate(pred, label, k, self.ignore_index, self._cm)
+            self._last = (preds[-1], label[-1] if label.dim() == 3 else label, k)
+        self._n_samples += len(preds)
+        if self.output_dir is not None and img_paths is not None:
+            if isinstance(img_paths, str):
+                img_paths = [img_paths]
+            assert len(img_paths) == len(preds), 'one img_path per image'
+            self._write_pngs(preds, img_paths, [bool(reduce_zero_label)] * len(preds))
         return self._cm
+
+    def _write_pngs(self, preds, img_paths, reduce_zero_label):
+        """One ops.png_encode call per (shape, dtype, reduce_zero_label) group, then the files."""
+        groups = OrderedDict()
+        for i, (p, z) in enumerate(zip(preds, reduce_zero_label)):
+            groups.setdefault((tuple(p.shape), p.dtype, z), []).append(i)
+        for (_, _, z), idx in groups.items():
+            batch = preds[idx[0]][None] if len(idx) == 1 else torch.stack([preds[i] for i in idx])
+            for i, data in zip(idx, ops.png_encode(batch, add=int(z))):
+                base = os.path.splitext(os.path.basename(img_paths[i]))[0]
+                with open(os.path.abspath(os.path.join(self.output_dir, f'{base}.png')), 'wb') as f:
+                    f.write(data)
 
     @staticmethod
     def intersect_and_union(pred_label, label, num_classes, ignore_index):
@@ -81,7 +126,11 @@ class IoUMetric:
         return total
 
     def compute_metrics(self, results=None):
-        """iou_metric.py:102-161.  Accepts this class's matrices or reference-style 4-tuples."""
+        """iou_metric.py:102-161.  Accepts this class's matrices or reference-style 4-tuples.  With `format_only`
+        nothing is computed: an empty OrderedDict, and a log line saying where the files went."""
+        if self.format_only:
+            logging.getLogger(__name__).info(f'results are saved to {self.output_dir}')
+            return OrderedDict()
         results = self.results if results is None else results
         if len(results) and not torch.is_tensor(results[0]):
             cols = tuple(zip(*results))

@@ -341,3 +341,30 @@ def view_resize(imgs, resized_hw, out=None, out_flip=None, swap_rb=False, mean=N
         L.check(lib.ledb200_view_resize(arr, i1 - i0, Hp, Wp, int(bool(swap_rb)), m3, s3, float(pad_val), st),
                 'ledb200_view_resize')
     return out, out_flip
+
+
+def png_encode(labels, add=0):
+    """Label maps -> PNG files on the device: labels [H,W], [1,H,W] or [N,H,W], CUDA uint8 or int64.  Returns N `bytes`,
+    each an 8-bit grayscale PNG of (label + add) mod 256 (add 0 or 1: mmseg's reduce_zero_label), which decodes to the
+    pixels of `Image.fromarray((label + add).astype(np.uint8))`.  One launch sequence, then two copies back: the offsets
+    and the files."""
+    _need_cuda(labels)
+    if labels.dtype not in (torch.uint8, torch.int64):
+        raise L.LedB200Error('png_encode: labels must be uint8 or int64')
+    if labels.dim() == 2:
+        labels = labels[None]
+    if labels.dim() != 3:
+        raise L.LedB200Error('png_encode: labels must be [H, W] or [N, H, W]')
+    labels = labels.contiguous()
+    N, H, W = labels.shape
+    lib, dev = L.get(), labels.device
+    bound = L.check(lib.ledb200_png_bound(H, W), 'ledb200_png_bound')
+    ws = torch.empty(L.check(lib.ledb200_png_workspace_bytes(N, H, W), 'ledb200_png_workspace_bytes'),
+                     dtype=torch.uint8, device=dev)
+    out = torch.empty(N * bound, dtype=torch.uint8, device=dev)
+    offsets = torch.empty(N + 1, dtype=torch.int64, device=dev)
+    L.check(lib.ledb200_png_encode(_p(labels), L.torch_dtype_code(labels), N, H, W, int(add), _p(out), _p(offsets),
+                                   _p(ws), L.stream_ptr(dev)), 'ledb200_png_encode')
+    offs = offsets.cpu().tolist()
+    data = out[:offs[-1]].cpu().numpy().tobytes()
+    return [data[offs[i]:offs[i + 1]] for i in range(N)]
