@@ -1,7 +1,5 @@
 // Stand-alone C-ABI operators (no handle): the fused head tail, the confusion matrix, OHEM CE and a
 // single convolution through the same launchers the engine uses.  See include/ledb200.h.
-#include <vector>
-
 #include "kernels.h"
 
 using namespace ledb;
@@ -67,52 +65,20 @@ int ledb200_conv2d(const void* in, void* out, const void* residual, int32_t dtyp
   if (res_ld == 0) res_ld = Cout;
   if (in_ld < Cin || out_ld < Cout || res_ld < Cout) return fail(LEDB200_EINVAL, "conv2d: pixel stride smaller than the channel count");
   cudaStream_t st = (cudaStream_t)stream;
-  const int taps = ksize * ksize, cp16 = (Cout + 15) / 16 * 16, cptc = conv_tc_pad(Cout);
-  std::vector<float> wd((size_t)taps * Cin * cp16, 0.f), bz(cptc > cp16 ? cptc : cp16, 0.f);
-  std::vector<__nv_bfloat16> wt((size_t)cptc * taps * Cin, __float2bfloat16(0.f));
-  for (int o = 0; o < Cout; ++o)
-    for (int c = 0; c < Cin; ++c)
-      for (int t = 0; t < taps; ++t) {
-        const float v = weight_oihw[((size_t)o * Cin + c) * taps + t];
-        wd[((size_t)t * Cin + c) * cp16 + o] = v;
-        wt[((size_t)o * taps + t) * Cin + c] = __float2bfloat16(v);
-      }
-  if (bias) for (int o = 0; o < Cout; ++o) bz[o] = bias[o];
-  float *d_wd = nullptr, *d_b = nullptr, *d_ps = nullptr, *d_pb = nullptr;
-  __nv_bfloat16* d_wt = nullptr;
-  int rc = LEDB200_OK;
-  auto up = [&](void** dst, const void* src, size_t bytes) -> int {
-    LEDB_CUDA_OK(cudaMalloc(dst, bytes));
-    LEDB_CUDA_OK(cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, st));
-    return LEDB200_OK;
-  };
-  rc = up((void**)&d_wd, wd.data(), wd.size() * 4);
-  if (!rc) rc = up((void**)&d_wt, wt.data(), wt.size() * 2);
-  if (!rc) rc = up((void**)&d_b, bz.data(), bz.size() * 4);
-  if (!rc && pre_scale) rc = up((void**)&d_ps, pre_scale, Cin * 4);
-  if (!rc && pre_shift) rc = up((void**)&d_pb, pre_shift, Cin * 4);
+  PackedConv c;
+  c.cin = Cin; c.cout = Cout; c.k = ksize; c.stride = stride;
+  int rc = pack_conv(weight_oihw, bias, nullptr, nullptr, c);
+  if (!rc && pre_scale) rc = upload(pre_scale, Cin * 4, (void**)&c.pre_scale);
+  if (!rc && pre_shift) rc = upload(pre_shift, Cin * 4, (void**)&c.pre_shift);
   if (!rc) {
-    ConvArgs a;
-    const int pad = ksize / 2;
+    ConvArgs a = conv_args(c, N, H, W);
     a.in = in; a.in_dtype = dtype; a.in_sc = 1; a.in_sw = in_ld; a.in_sh = (int64_t)W * in_ld; a.in_sn = (int64_t)H * W * in_ld;
-    a.out = out; a.out_dtype = dtype; a.out_ld = out_ld; a.res = residual; a.res_ld = res_ld;
-    a.bias = d_b; a.pre_scale = d_ps; a.pre_shift = d_pb; a.pre_relu = 1;
-    a.w_direct = d_wd; a.w_tc = d_wt; a.cout_pad16 = cp16; a.cout_pad_tc = cptc;
-    a.N = N; a.H = H; a.W = W; a.Cin = Cin; a.Cout = Cout; a.ksize = ksize; a.stride = stride; a.pad = pad; a.dil = 1;
-    a.Ho = (H + 2 * pad - ksize) / stride + 1; a.Wo = (W + 2 * pad - ksize) / stride + 1; a.relu = relu;
-    if (backend == 2) {
-      if (dtype != LEDB200_BF16 || pre_scale || !conv_tc_eligible(a))
-        rc = fail(LEDB200_EINVAL, "conv2d: shape not eligible for the tcgen05 path");
-      else rc = launch_conv_tc(a, st);
-    } else if (backend == 0 && dtype == LEDB200_BF16 && !pre_scale && conv_tc_eligible(a)) {
-      rc = launch_conv_tc(a, st);
-    } else {
-      rc = launch_conv_direct(a, st);
-    }
+    a.out = out; a.out_dtype = dtype; a.out_ld = out_ld; a.res = residual; a.res_ld = res_ld; a.relu = relu;
+    rc = launch_conv(a, backend, "conv2d", st);
   }
   cudaError_t ce = cudaStreamSynchronize(st);
   if (!rc && ce != cudaSuccess) rc = fail(LEDB200_ECUDA, std::string("conv2d: ") + cudaGetErrorString(ce));
-  cudaFree(d_wd); cudaFree(d_wt); cudaFree(d_b); cudaFree(d_ps); cudaFree(d_pb);
+  free_conv(c);
   return rc;
 }
 

@@ -38,15 +38,11 @@ namespace {
 
 struct HostTensor { std::vector<float> v; std::vector<int64_t> shape; };
 
-struct ConvDef {
+struct ConvDef : PackedConv {  // cin .. stride from the model definition, the device side from finalize
   std::string name;          // op / debug name
   std::string wkey;          // state-dict key of conv weight
   std::string bias_key;      // conv bias key or ""
   std::string bn_after;      // BN prefix folded into the conv ("" = none)
-  int cin = 0, cout = 0, k = 1, stride = 1;
-  // device side
-  float* w_direct = nullptr; __nv_bfloat16* w_tc = nullptr; float* bias = nullptr;
-  int cout_pad16 = 0, cout_pad_tc = 0;
 };
 struct AffineDef { std::string bn; int c = 0; float* scale = nullptr; float* shift = nullptr; };
 
@@ -93,7 +89,7 @@ struct ledb200_handle {
   std::map<std::string, int> conv_by_name, aff_by_name;
   float* pre_scale = nullptr;   // uint8 preprocessing affine [3]
   float* pre_shift = nullptr;
-  std::vector<void*> dev_allocs;
+  std::vector<void*> dev_allocs;   // everything on the device except the convs
   char* arena = nullptr;
   size_t arena_cap = 0;
   std::map<std::string, std::unique_ptr<Plan>> plans;
@@ -198,14 +194,10 @@ void define_model(ledb200_handle& e) {
 }
 
 // ------------------------------------------------------------------ finalize (fold + upload)
-template <typename T>
-int upload(ledb200_handle& e, const std::vector<T>& host, T** dev) {
-  void* p = nullptr;
-  LEDB_CUDA_OK(cudaMalloc(&p, std::max<size_t>(host.size() * sizeof(T), 16)));
-  LEDB_CUDA_OK(cudaMemcpy(p, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice));
-  e.dev_allocs.push_back(p);
-  *dev = reinterpret_cast<T*>(p);
-  return LEDB200_OK;
+int upload(ledb200_handle& e, const std::vector<float>& host, float** dev) {
+  const int rc = ledb::upload(host, dev);
+  if (!rc) e.dev_allocs.push_back(*dev);
+  return rc;
 }
 
 const HostTensor* get(const ledb200_handle& e, const std::string& k) {
@@ -229,39 +221,6 @@ int bn_affine(const ledb200_handle& e, const std::string& bn, int c, std::vector
   return LEDB200_OK;
 }
 
-int tc_pad(int cout) { return conv_tc_pad(cout); }   // UMMA N tile: 16, 32 or a multiple of 64 (<= 256 per tile)
-
-// Fold BN into OIHW weights and repack for both conv back ends.
-int pack_conv(ledb200_handle& e, ConvDef& d, const float* w_oihw, const float* bias_in, const float* scale,
-              const float* shift) {
-  const int taps = d.k * d.k;
-  d.cout_pad16 = (d.cout + 15) / 16 * 16;
-  d.cout_pad_tc = tc_pad(d.cout);
-  std::vector<float> wd((size_t)taps * d.cin * d.cout_pad16, 0.f);
-  std::vector<__nv_bfloat16> wt((size_t)d.cout_pad_tc * taps * d.cin, __float2bfloat16(0.f));
-  std::vector<float> bias(d.cout_pad_tc > d.cout_pad16 ? d.cout_pad_tc : d.cout_pad16, 0.f);
-  bool has_bias = false;
-  for (int o = 0; o < d.cout; ++o) {
-    const float s = scale ? scale[o] : 1.f;
-    float bv = 0.f;
-    if (bias_in) { bv = bias_in[o] * s; has_bias = true; }
-    if (shift) { bv += shift[o]; has_bias = true; }
-    bias[o] = bv;
-    for (int c = 0; c < d.cin; ++c)
-      for (int t = 0; t < taps; ++t) {
-        const float v = w_oihw[((size_t)o * d.cin + c) * taps + t] * s;
-        wd[((size_t)t * d.cin + c) * d.cout_pad16 + o] = v;
-        wt[((size_t)o * taps + t) * d.cin + c] = __float2bfloat16(v);
-      }
-  }
-  int rc = upload(e, wd, &d.w_direct);
-  if (rc) return rc;
-  rc = upload(e, wt, &d.w_tc);
-  if (rc) return rc;
-  if (has_bias) rc = upload(e, bias, &d.bias);
-  return rc;
-}
-
 int finalize(ledb200_handle& e) {
   std::string missing;
   int nmiss = 0;
@@ -280,8 +239,9 @@ int finalize(ledb200_handle& e) {
     }
     const HostTensor* b = d.bias_key.empty() ? nullptr : get(e, d.bias_key);
     if (b && (int)b->v.size() != d.cout) return fail(LEDB200_EINVAL, d.bias_key + ": wrong size");
-    int rc = pack_conv(e, d, w->v.data(), b ? b->v.data() : nullptr, scale.empty() ? nullptr : scale.data(),
-                       shift.empty() ? nullptr : shift.data());
+    free_conv(d);   // a finalize retried after a failure packs again
+    int rc = pack_conv(w->v.data(), b ? b->v.data() : nullptr, scale.empty() ? nullptr : scale.data(),
+                       shift.empty() ? nullptr : shift.data(), d);
     if (rc) return rc;
   }
   for (auto& a : e.affs) {
@@ -322,62 +282,52 @@ struct Builder {
   }
   static void* ptr(ledb200_handle& e, Plan& p, int id) { return id < 0 ? nullptr : e.arena + p.bufs[id].off; }
 
-  // would this conv run on the tensor-core kernel?
-  bool conv_uses_tc(const std::string& cname, int in, int out, int res = -1, int out2 = -1) {
-    const ConvDef& d = e.convs[e.conv_by_name.at(cname)];
-    const Buf bi = p.bufs[in];
-    const int pad = d.k / 2;
-    const int Ho = (bi.h + 2 * pad - d.k) / d.stride + 1, Wo = (bi.w + 2 * pad - d.k) / d.stride + 1;
-    ConvArgs s;
-    s.in_dtype = s.out_dtype = dt; s.N = bi.n; s.H = bi.h; s.W = bi.w; s.Cin = d.cin; s.Ho = Ho; s.Wo = Wo;
-    s.Cout = d.cout; s.ksize = d.k; s.stride = d.stride; s.pad = pad; s.in_sw = bi.ld; s.in_sc = 1;
-    s.out_ld = out >= 0 ? p.bufs[out].ld : 0; s.out2_ld = out2 >= 0 ? p.bufs[out2].ld : 0;
-    s.res_ld = res >= 0 ? p.bufs[res].ld : 0; s.cout_pad_tc = d.cout_pad_tc ? d.cout_pad_tc : tc_pad(d.cout);
-    // eligibility only looks at which optional tensors exist, not at their addresses
-    static const char dummy = 0;
-    if (out >= 0) s.out = const_cast<char*>(&dummy);
-    if (out2 >= 0) s.out2 = const_cast<char*>(&dummy);
-    if (res >= 0) s.res = &dummy;
-    return e.cfg.conv_backend != 1 && dt == LEDB200_BF16 && conv_tc_eligible(s);
+  // One conv op on arena buffers.  aff2: affine id for the second output (-1 = plain ReLU copy)
+  struct ConvOp {
+    int ci, in, out, res = -1;
+    bool relu = false;
+    int out2 = -1, aff2 = -1, out_coff = 0, out2_coff = 0;
+    bool out_f16 = false;
+  };
+  // Its launch arguments.  Before the arena exists (plan time) any non-null base will do: eligibility looks only at which
+  // optional tensors exist, not at their addresses.
+  static ConvArgs op_args(ledb200_handle& e, Plan& p, int dtype, const ConvOp& c) {
+    const Buf& bi = p.bufs[c.in];
+    char* base = e.arena ? e.arena : reinterpret_cast<char*>(256);
+    const size_t es = dtype == LEDB200_BF16 ? 2 : 4;
+    ConvArgs a = conv_args(e.convs[c.ci], bi.n, bi.h, bi.w);
+    a.in = base + bi.off; a.in_dtype = dtype;
+    a.in_sc = 1; a.in_sw = bi.ld; a.in_sh = (int64_t)bi.w * bi.ld; a.in_sn = (int64_t)bi.h * bi.w * bi.ld;
+    if (c.out >= 0) { a.out = base + p.bufs[c.out].off + c.out_coff * es; a.out_ld = p.bufs[c.out].ld; }
+    a.out_dtype = dtype;
+    if (c.out2 >= 0) {
+      a.out2 = base + p.bufs[c.out2].off + c.out2_coff * es; a.out2_ld = p.bufs[c.out2].ld;
+      if (c.aff2 >= 0) { a.o2_scale = e.affs[c.aff2].scale + c.out2_coff; a.o2_shift = e.affs[c.aff2].shift + c.out2_coff; }
+    }
+    if (c.res >= 0) { a.res = base + p.bufs[c.res].off; a.res_ld = p.bufs[c.res].ld; }
+    a.out_f16 = c.out_f16 ? 1 : 0;
+    a.relu = c.relu ? 1 : 0;
+    return a;
   }
+  // would this conv run on the tensor-core kernel?
+  bool conv_uses_tc(const ConvOp& c) { return conv_use_tc(op_args(e, p, dt, c), e.cfg.conv_backend); }
 
-  // generic conv op on arena buffers.  aff2: affine id for the second output (-1 = plain ReLU copy)
   int conv(const std::string& cname, int in, int out, int res = -1, bool relu = false, int out2 = -1,
            int aff2 = -1, int out_coff = 0, int out2_coff = 0, bool out_f16 = false) {
-    const int ci = e.conv_by_name.at(cname);
+    const ConvOp c{e.conv_by_name.at(cname), in, out, res, relu, out2, aff2, out_coff, out2_coff, out_f16};
     const Buf bi = p.bufs[in];
-    const ConvDef& d = e.convs[ci];
-    const int pad = d.k / 2;
-    const int Ho = (bi.h + 2 * pad - d.k) / d.stride + 1, Wo = (bi.w + 2 * pad - d.k) / d.stride + 1;
+    const ConvDef& d = e.convs[c.ci];
+    const ConvArgs a = op_args(e, p, dt, c);
     const int dtype = dt;
-    const bool use_tc = conv_uses_tc(cname, in, out, res, out2);
-    const double es_ = (double)esize(e), npo = (double)bi.n * Ho * Wo;
+    const bool use_tc = conv_use_tc(a, e.cfg.conv_backend);
+    const double es_ = (double)esize(e), npo = (double)bi.n * a.Ho * a.Wo;
     const double flops = 2.0 * npo * d.cout * d.cin * d.k * d.k;
     // SURVEY 8(d): every tensor read once and written once.  A second, pre-activated copy of the output (x2h, DAPPM
     // inputs ...) is an implementation choice, not an algorithmic byte: the output is counted ONCE.
     const double bytes = es_ * ((double)bi.n * bi.h * bi.w * d.cin + npo * d.cout * ((out >= 0 || out2 >= 0) + (res >= 0))) +
                          es_ * (double)d.cout * d.cin * d.k * d.k;
     p.ops.push_back({cname, [=](ledb200_handle& e, Plan& p, cudaStream_t st) -> int {
-      const ConvDef& d = e.convs[ci];
-      const Buf& bi = p.bufs[in];
-      ConvArgs a;
-      a.in = ptr(e, p, in); a.in_dtype = dtype;
-      a.in_sc = 1; a.in_sw = bi.ld; a.in_sh = (int64_t)bi.w * bi.ld; a.in_sn = (int64_t)bi.h * bi.w * bi.ld;
-      const size_t es = dtype == LEDB200_BF16 ? 2 : 4;
-      if (out >= 0) { a.out = (char*)ptr(e, p, out) + out_coff * es; a.out_ld = p.bufs[out].ld; }
-      a.out_dtype = dtype;
-      if (out2 >= 0) {
-        a.out2 = (char*)ptr(e, p, out2) + out2_coff * es; a.out2_ld = p.bufs[out2].ld;
-        if (aff2 >= 0) { a.o2_scale = e.affs[aff2].scale + out2_coff; a.o2_shift = e.affs[aff2].shift + out2_coff; }
-      }
-      if (res >= 0) { a.res = ptr(e, p, res); a.res_ld = p.bufs[res].ld; }
-      a.out_f16 = out_f16 ? 1 : 0;
-      a.bias = d.bias; a.w_direct = d.w_direct; a.w_tc = d.w_tc;
-      a.cout_pad16 = d.cout_pad16; a.cout_pad_tc = d.cout_pad_tc;
-      a.N = bi.n; a.H = bi.h; a.W = bi.w; a.Cin = d.cin; a.Ho = Ho; a.Wo = Wo; a.Cout = d.cout;
-      a.ksize = d.k; a.stride = d.stride; a.pad = d.k / 2; a.dil = 1; a.relu = relu ? 1 : 0;
-      if (use_tc) return launch_conv_tc(a, st);
-      return launch_conv_direct(a, st);
+      return launch_conv(op_args(e, p, dtype, c), use_tc ? 2 : 1, "engine", st);
     }, use_tc ? K_CONV_TC : K_CONV_DIRECT, flops, bytes});
     tag();
     return out;
@@ -490,8 +440,7 @@ void add_stem0(Builder& B, int out_x1, int out_x1h) {
   const int c0 = e0.convs[ci].cout;
   const bool use_tc = e0.cfg.conv_backend != 1 && dtype == LEDB200_BF16 && (c0 == 16 || c0 == 32);
   B.p.ops.push_back({"backbone.stem.0", [=](ledb200_handle& e, Plan& p, cudaStream_t st) -> int {
-    const ConvDef& d = e.convs[ci];
-    ConvArgs a;
+    ConvArgs a = conv_args(e.convs[ci], n, H, W);
     const int lay = e.ext_layout;
     const int64_t HW = (int64_t)H * W;
     a.in = e.ext_img;
@@ -509,9 +458,7 @@ void add_stem0(Builder& B, int out_x1, int out_x1h) {
       a.out2 = Builder::ptr(e, p, out_x1h); a.out2_ld = p.bufs[out_x1h].ld;
       a.o2_scale = e.affs[a2].scale; a.o2_shift = e.affs[a2].shift;
     }
-    a.bias = d.bias; a.w_direct = d.w_direct; a.w_tc = d.w_tc; a.cout_pad16 = d.cout_pad16; a.cout_pad_tc = d.cout_pad_tc;
-    a.N = n; a.H = H; a.W = W; a.Cin = d.cin; a.Ho = p.bufs[out_x1].h; a.Wo = p.bufs[out_x1].w; a.Cout = d.cout;
-    a.ksize = 3; a.stride = 2; a.pad = 1; a.dil = 1; a.relu = 1;
+    a.relu = 1;
     if (use_tc && stem_tc_eligible(a)) return launch_stem_tc(a, st);
     return launch_conv_direct(a, st);
   }, use_tc ? K_CONV_TC : K_CONV_DIRECT, 0.0, 0.0});
@@ -720,7 +667,7 @@ void build_head_fused(Builder& B) {
   const bool ladder = exact2 && dtype == LEDB200_BF16 && e.cfg.conv_backend != 1 &&
                       ladder_eligible(rung_args(p, h + "head_x2", x2h, xc, hx2)) &&
                       ladder_eligible(rung_args(p, h + "head_x1", x1h, hx2, hx1)) &&
-                      B.conv_uses_tc(h + "conv_seg", hf, xc);
+                      B.conv_uses_tc({e.conv_by_name.at(h + "conv_seg"), hf, xc});
   if (ladder) {
     p.bufs[xc].f16 = p.bufs[hx1].f16 = p.bufs[hx2].f16 = 1;
     // the rungs are stored as IEEE fp16 (same 2 bytes, 11-bit mantissa): tighter than bf16, and class logits are far
@@ -798,16 +745,12 @@ void build_head_standalone(Builder& B, int h8, int w8, int h2, int w2, int h4, i
                       int H, int W, int out) {
     const int ci = e.conv_by_name.at(cname), ai = aff(e, bn);
     p.ops.push_back({cname, [=](ledb200_handle& e, Plan& p, cudaStream_t st) -> int {
-      const ConvDef& d = e.convs[ci];
-      ConvArgs a;
+      ConvArgs a = conv_args(e.convs[ci], n, H, W);
       const int64_t HW = (int64_t)H * W;
       a.in = e.*src; a.in_dtype = LEDB200_F32; a.in_sn = cin * HW; a.in_sc = HW; a.in_sh = W; a.in_sw = 1;
       a.pre_scale = e.affs[ai].scale; a.pre_shift = e.affs[ai].shift; a.pre_relu = 1;
-      a.out = Builder::ptr(e, p, out); a.out_ld = p.bufs[out].ld; a.out_dtype = dtype;
-      a.bias = d.bias; a.w_direct = d.w_direct; a.cout_pad16 = d.cout_pad16;
-      a.N = n; a.H = H; a.W = W; a.Cin = cin; a.Ho = H; a.Wo = W; a.Cout = d.cout;
-      a.ksize = 3; a.stride = 1; a.pad = 1; a.dil = 1; a.relu = 1;
-      return launch_conv_direct(a, st);
+      a.out = Builder::ptr(e, p, out); a.out_ld = p.bufs[out].ld; a.out_dtype = dtype; a.relu = 1;
+      return launch_conv(a, 1, "engine", st);
     }, K_CONV_DIRECT, 0.0, 0.0});
   };
   const int hf = B.buf("head.feat", n, h8, w8, HC);
@@ -1019,6 +962,7 @@ int ledb200_destroy(ledb200_handle* h) {
   for (int i = 0; i < 2; ++i) { if (h->cap[i]) cudaStreamDestroy(h->cap[i]); if (h->ev_x[i]) cudaEventDestroy(h->ev_x[i]); }
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
   if (h->ev_join) cudaEventDestroy(h->ev_join);
+  for (auto& d : h->convs) free_conv(d);
   for (void* p : h->dev_allocs) cudaFree(p);
   if (h->arena) cudaFree(h->arena);
   delete h;

@@ -28,11 +28,7 @@ namespace {
 constexpr int WS = 8, NTOK = WS * WS;
 
 struct GetbDev {
-  // conv weights in both layouts (see ConvArgs)
-  float* wd[4] = {nullptr, nullptr, nullptr, nullptr};
-  __nv_bfloat16* wt[4] = {nullptr, nullptr, nullptr, nullptr};
-  float* bias[4] = {nullptr, nullptr, nullptr, nullptr};
-  int cin[4], cout[4], cp16[4], cptc[4];
+  PackedConv conv[4];   // qkv, proj, fc1, fc2
   float *n1s = nullptr, *n1b = nullptr, *relb = nullptr, *wdw = nullptr, *dws = nullptr, *dwb = nullptr;
 };
 
@@ -220,42 +216,19 @@ __global__ void __launch_bounds__(256) getb_dw_kernel(DwArgs a) {
   store8(reinterpret_cast<T*>(a.out) + (((int64_t)n * a.H + y) * a.W + x) * a.C + cg * 8, acc);
 }
 
-int upload(void** dst, const void* src, size_t bytes) {
-  LEDB_CUDA_OK(cudaMalloc(dst, bytes));
-  LEDB_CUDA_OK(cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice));
-  return LEDB200_OK;
-}
-
 // 1x1 conv weights [Cout][Cin] fp32 (host) -> both device layouts + padded bias
-int pack_conv(GetbDev& d, int i, const float* w, const float* bias, int cin, int cout) {
-  const int cp16 = (cout + 15) / 16 * 16, cptc = conv_tc_pad(cout);
-  d.cin[i] = cin; d.cout[i] = cout; d.cp16[i] = cp16; d.cptc[i] = cptc;
-  std::vector<float> wd((size_t)cin * cp16, 0.f), bz(cptc > cp16 ? cptc : cp16, 0.f);
-  std::vector<__nv_bfloat16> wt((size_t)cptc * cin, __float2bfloat16(0.f));
-  for (int o = 0; o < cout; ++o)
-    for (int c = 0; c < cin; ++c) {
-      const float v = w[(size_t)o * cin + c];
-      wd[(size_t)c * cp16 + o] = v;
-      wt[(size_t)o * cin + c] = __float2bfloat16(v);
-    }
-  if (bias) for (int o = 0; o < cout; ++o) bz[o] = bias[o];
-  int rc = upload((void**)&d.wd[i], wd.data(), wd.size() * 4);
-  if (!rc) rc = upload((void**)&d.wt[i], wt.data(), wt.size() * 2);
-  if (!rc) rc = upload((void**)&d.bias[i], bz.data(), bz.size() * 4);
-  return rc;
+int pack_conv1x1(PackedConv& c, const float* w, const float* bias, int cin, int cout) {
+  c.cin = cin; c.cout = cout;
+  return pack_conv(w, bias, nullptr, nullptr, c);
 }
 
 int conv1x1(const ledb200_getb& g, int i, const void* in, void* out, const void* res, int relu, int N, int H, int W,
             cudaStream_t st) {
-  ConvArgs a;
-  const int cin = g.d.cin[i], cout = g.d.cout[i];
-  a.in = in; a.in_dtype = g.dtype; a.in_sc = 1; a.in_sw = cin; a.in_sh = (int64_t)W * cin; a.in_sn = (int64_t)H * W * cin;
-  a.out = out; a.out_dtype = g.dtype; a.out_ld = cout; a.res = res; a.res_ld = cout;
-  a.bias = g.d.bias[i]; a.w_direct = g.d.wd[i]; a.w_tc = g.d.wt[i]; a.cout_pad16 = g.d.cp16[i]; a.cout_pad_tc = g.d.cptc[i];
-  a.N = N; a.H = H; a.W = W; a.Cin = cin; a.Cout = cout; a.ksize = 1; a.stride = 1; a.pad = 0; a.dil = 1;
-  a.Ho = H; a.Wo = W; a.relu = relu;
-  if (g.dtype == LEDB200_BF16 && conv_tc_eligible(a)) return launch_conv_tc(a, st);
-  return launch_conv_direct(a, st);
+  const PackedConv& c = g.d.conv[i];
+  ConvArgs a = conv_args(c, N, H, W);
+  a.in = in; a.in_dtype = g.dtype; a.in_sc = 1; a.in_sw = c.cin; a.in_sh = (int64_t)W * c.cin; a.in_sn = (int64_t)H * W * c.cin;
+  a.out = out; a.out_dtype = g.dtype; a.out_ld = c.cout; a.res = res; a.res_ld = c.cout; a.relu = relu;
+  return launch_conv(a, 0, "getb_forward", st);
 }
 
 template <typename T, int D>
@@ -333,16 +306,16 @@ int ledb200_getb_create(int32_t dim, int32_t heads, int32_t hidden, int32_t wind
   std::vector<float> dwt((size_t)NTOK * C);                 // tap-major depthwise weights
   for (int c = 0; c < C; ++c)
     for (int t = 0; t < NTOK; ++t) dwt[(size_t)t * C + c] = w_dw[(size_t)c * NTOK + t];
-  int rc = pack_conv(g->d, 0, w_qkv, b_qkv, C, 3 * C);
-  if (!rc) rc = pack_conv(g->d, 1, w_proj, nullptr, C, C);
-  if (!rc) rc = pack_conv(g->d, 2, w_fc1, b_fc1, C, hidden);
-  if (!rc) rc = pack_conv(g->d, 3, w_fc2, b_fc2, hidden, C);
-  if (!rc) rc = upload((void**)&g->d.n1s, n1s, C * 4);
-  if (!rc) rc = upload((void**)&g->d.n1b, n1b, C * 4);
-  if (!rc) rc = upload((void**)&g->d.relb, relb, (size_t)heads * NTOK * NTOK * 4);
-  if (!rc) rc = upload((void**)&g->d.wdw, dwt.data(), dwt.size() * 4);
-  if (!rc) rc = upload((void**)&g->d.dws, dws, C * 4);
-  if (!rc) rc = upload((void**)&g->d.dwb, dwb, C * 4);
+  int rc = pack_conv1x1(g->d.conv[0], w_qkv, b_qkv, C, 3 * C);
+  if (!rc) rc = pack_conv1x1(g->d.conv[1], w_proj, nullptr, C, C);
+  if (!rc) rc = pack_conv1x1(g->d.conv[2], w_fc1, b_fc1, C, hidden);
+  if (!rc) rc = pack_conv1x1(g->d.conv[3], w_fc2, b_fc2, hidden, C);
+  if (!rc) rc = upload(n1s, C * 4, (void**)&g->d.n1s);
+  if (!rc) rc = upload(n1b, C * 4, (void**)&g->d.n1b);
+  if (!rc) rc = upload(relb, (size_t)heads * NTOK * NTOK * 4, (void**)&g->d.relb);
+  if (!rc) rc = upload(dwt, &g->d.wdw);
+  if (!rc) rc = upload(dws, C * 4, (void**)&g->d.dws);
+  if (!rc) rc = upload(dwb, C * 4, (void**)&g->d.dwb);
   if (rc) { ledb200_getb_destroy(g); return rc; }
   *out = g;
   return LEDB200_OK;
@@ -350,7 +323,7 @@ int ledb200_getb_create(int32_t dim, int32_t heads, int32_t hidden, int32_t wind
 
 int ledb200_getb_destroy(ledb200_getb* g) {
   if (!g) return LEDB200_OK;
-  for (int i = 0; i < 4; ++i) { cudaFree(g->d.wd[i]); cudaFree(g->d.wt[i]); cudaFree(g->d.bias[i]); }
+  for (PackedConv& c : g->d.conv) free_conv(c);
   cudaFree(g->d.n1s); cudaFree(g->d.n1b); cudaFree(g->d.relb); cudaFree(g->d.wdw); cudaFree(g->d.dws); cudaFree(g->d.dwb);
   cudaFree(g->ws);
   delete g;

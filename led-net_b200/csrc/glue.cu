@@ -12,11 +12,9 @@
 using namespace ledb;
 
 struct ledb200_conv_layer {
-  int cin = 0, cout = 0, k = 1, stride = 1, depthwise = 0;
-  float* w_direct = nullptr; __nv_bfloat16* w_tc = nullptr; float* bias = nullptr;
-  float* pre_scale = nullptr; float* pre_shift = nullptr;
+  PackedConv c;                               // depthwise: only cin .. stride, bias
+  int depthwise = 0;
   float* w_dw = nullptr;                      // depthwise: [9][C]
-  int cout_pad16 = 0, cout_pad_tc = 0;
 };
 
 namespace ledb {
@@ -151,16 +149,6 @@ add_relu_kernel(const T* __restrict__ a, const T* __restrict__ b, T* __restrict_
   }
 }
 
-template <typename T>
-int upload_vec(const std::vector<T>& host, T** dev) {
-  void* p = nullptr;
-  LEDB_CUDA_OK(cudaMalloc(&p, std::max<size_t>(host.size() * sizeof(T), 16)));
-  cudaError_t e = cudaMemcpy(p, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) { cudaFree(p); return fail(LEDB200_ECUDA, std::string("conv_layer upload: ") + cudaGetErrorString(e)); }
-  *dev = reinterpret_cast<T*>(p);
-  return LEDB200_OK;
-}
-
 bool dt_ok(int dt) { return dt == LEDB200_F32 || dt == LEDB200_BF16; }
 
 }  // namespace
@@ -180,37 +168,20 @@ int ledb200_conv_layer_create(const float* weight, const float* bias, const floa
   if (dw && (groups != Cin || Cin != Cout || ksize != 3 || Cin % 8 || pre_scale))
     return fail(LEDB200_EINVAL, "conv_layer_create: grouped convolutions are depthwise 3x3 (groups == Cin == Cout, Cin % 8 == 0)");
   ledb200_conv_layer* L = new ledb200_conv_layer();
-  L->cin = Cin; L->cout = Cout; L->k = ksize; L->stride = stride; L->depthwise = dw ? 1 : 0;
+  L->c.cin = Cin; L->c.cout = Cout; L->c.k = ksize; L->c.stride = stride; L->depthwise = dw ? 1 : 0;
   int rc = LEDB200_OK;
-  const int taps = ksize * ksize;
   if (dw) {
     std::vector<float> w((size_t)9 * Cin);                      // weight [C][1][3][3] -> [tap][C]
     for (int c = 0; c < Cin; ++c)
       for (int t = 0; t < 9; ++t) w[(size_t)t * Cin + c] = weight[(size_t)c * 9 + t];
-    rc = upload_vec(w, &L->w_dw);
+    rc = upload(w, &L->w_dw);
+    if (!rc && bias) rc = upload(bias, Cout * 4, (void**)&L->c.bias);
   } else {
-    L->cout_pad16 = (Cout + 15) / 16 * 16; L->cout_pad_tc = conv_tc_pad(Cout);
-    std::vector<float> wd((size_t)taps * Cin * L->cout_pad16, 0.f);
-    std::vector<__nv_bfloat16> wt((size_t)L->cout_pad_tc * taps * Cin, __float2bfloat16(0.f));
-    for (int o = 0; o < Cout; ++o)
-      for (int c = 0; c < Cin; ++c)
-        for (int t = 0; t < taps; ++t) {
-          const float v = weight[((size_t)o * Cin + c) * taps + t];
-          wd[((size_t)t * Cin + c) * L->cout_pad16 + o] = v;
-          wt[((size_t)o * taps + t) * Cin + c] = __float2bfloat16(v);
-        }
-    rc = upload_vec(wd, &L->w_direct);
-    if (!rc) rc = upload_vec(wt, &L->w_tc);
-  }
-  if (!rc) {
-    std::vector<float> bz(std::max(L->cout_pad_tc, std::max(L->cout_pad16, Cout)), 0.f);
-    if (bias) for (int o = 0; o < Cout; ++o) bz[o] = bias[o];
-    rc = upload_vec(bz, &L->bias);
+    rc = pack_conv(weight, bias, nullptr, nullptr, L->c);
   }
   if (!rc && pre_scale) {
-    std::vector<float> ps(pre_scale, pre_scale + Cin), pb(pre_shift, pre_shift + Cin);
-    rc = upload_vec(ps, &L->pre_scale);
-    if (!rc) rc = upload_vec(pb, &L->pre_shift);
+    rc = upload(pre_scale, Cin * 4, (void**)&L->c.pre_scale);
+    if (!rc) rc = upload(pre_shift, Cin * 4, (void**)&L->c.pre_shift);
   }
   if (rc) { ledb200_conv_layer_destroy(L); return rc; }
   *out = L;
@@ -219,7 +190,8 @@ int ledb200_conv_layer_create(const float* weight, const float* bias, const floa
 
 int ledb200_conv_layer_destroy(ledb200_conv_layer* L) {
   if (!L) return LEDB200_OK;
-  cudaFree(L->w_direct); cudaFree(L->w_tc); cudaFree(L->bias); cudaFree(L->pre_scale); cudaFree(L->pre_shift); cudaFree(L->w_dw);
+  free_conv(L->c);
+  cudaFree(L->w_dw);
   delete L;
   return LEDB200_OK;
 }
@@ -230,55 +202,43 @@ int ledb200_conv_layer_forward(ledb200_conv_layer* L, const void* in, void* out,
   if (!L || !in || !out) return fail(LEDB200_EINVAL, "conv_layer_forward: null pointer");
   if (!dt_ok(dtype)) return fail(LEDB200_EINVAL, "conv_layer_forward: dtype must be F32 or BF16");
   if (N < 1 || H < 1 || W < 1) return fail(LEDB200_EINVAL, "conv_layer_forward: empty input");
-  if (in_ld == 0) in_ld = L->cin;
-  if (out_ld == 0) out_ld = L->cout;
-  if (res_ld == 0) res_ld = L->cout;
-  if (in_ld < L->cin || out_ld < L->cout || (residual && res_ld < L->cout))
+  const PackedConv& c = L->c;
+  if (in_ld == 0) in_ld = c.cin;
+  if (out_ld == 0) out_ld = c.cout;
+  if (res_ld == 0) res_ld = c.cout;
+  if (in_ld < c.cin || out_ld < c.cout || (residual && res_ld < c.cout))
     return fail(LEDB200_EINVAL, "conv_layer_forward: pixel stride smaller than the channel count");
   cudaStream_t st = (cudaStream_t)stream;
-  const int pad = L->k / 2;
-  const int Ho = (H + 2 * pad - L->k) / L->stride + 1, Wo = (W + 2 * pad - L->k) / L->stride + 1;
+  ConvArgs a = conv_args(c, N, H, W);
   if (L->depthwise) {
     if (residual) return fail(LEDB200_EINVAL, "conv_layer_forward: the depthwise layer takes no residual");
     if (in_ld % 8 || out_ld % 8) return fail(LEDB200_EINVAL, "conv_layer_forward: depthwise pixel strides must be multiples of 8");
-    const int64_t total = (int64_t)N * Ho * Wo * (L->cin / 8);
+    const int64_t total = (int64_t)N * a.Ho * a.Wo * (c.cin / 8);
     if (dtype == LEDB200_BF16)
-      dwconv3x3_kernel<__nv_bfloat16><<<grid_for(total), kT, 0, st>>>((const __nv_bfloat16*)in, (__nv_bfloat16*)out, L->w_dw, L->bias, N,
-                                                                      H, W, L->cin, Ho, Wo, L->stride, relu, in_ld, out_ld);
+      dwconv3x3_kernel<__nv_bfloat16><<<grid_for(total), kT, 0, st>>>((const __nv_bfloat16*)in, (__nv_bfloat16*)out, L->w_dw, c.bias, N,
+                                                                      H, W, c.cin, a.Ho, a.Wo, c.stride, relu, in_ld, out_ld);
     else
-      dwconv3x3_kernel<float><<<grid_for(total), kT, 0, st>>>((const float*)in, (float*)out, L->w_dw, L->bias, N, H, W, L->cin, Ho,
-                                                              Wo, L->stride, relu, in_ld, out_ld);
+      dwconv3x3_kernel<float><<<grid_for(total), kT, 0, st>>>((const float*)in, (float*)out, L->w_dw, c.bias, N, H, W, c.cin, a.Ho,
+                                                              a.Wo, c.stride, relu, in_ld, out_ld);
     LEDB_LAUNCH_OK("dwconv3x3_kernel");
     return LEDB200_OK;
   }
-  ConvArgs a;
   a.in = in; a.in_dtype = dtype; a.in_sc = 1; a.in_sw = in_ld; a.in_sh = (int64_t)W * in_ld; a.in_sn = (int64_t)H * W * in_ld;
-  a.out = out; a.out_dtype = dtype; a.out_ld = out_ld; a.res = residual; a.res_ld = res_ld;
-  a.bias = L->bias; a.pre_scale = L->pre_scale; a.pre_shift = L->pre_shift; a.pre_relu = 1;
-  a.w_direct = L->w_direct; a.w_tc = L->w_tc; a.cout_pad16 = L->cout_pad16; a.cout_pad_tc = L->cout_pad_tc;
-  a.N = N; a.H = H; a.W = W; a.Cin = L->cin; a.Cout = L->cout; a.ksize = L->k; a.stride = L->stride; a.pad = pad; a.dil = 1;
-  a.Ho = Ho; a.Wo = Wo; a.relu = relu;
-  const bool tc_ok = dtype == LEDB200_BF16 && !L->pre_scale && conv_tc_eligible(a);
-  if (backend == 2 && !tc_ok) return fail(LEDB200_EINVAL, "conv_layer_forward: shape not eligible for the tcgen05 path");
-  if (backend != 1 && tc_ok) return launch_conv_tc(a, st);
-  return launch_conv_direct(a, st);
+  a.out = out; a.out_dtype = dtype; a.out_ld = out_ld; a.res = residual; a.res_ld = res_ld; a.relu = relu;
+  return launch_conv(a, backend, "conv_layer_forward", st);
 }
 
 int ledb200_conv_layer_forward_image(ledb200_conv_layer* L, const void* img, int32_t img_layout, void* out, int32_t dtype, int32_t N,
                                      int32_t H, int32_t W, int32_t out_ld, int32_t relu, void* stream) {
   if (!L || !img || !out) return fail(LEDB200_EINVAL, "conv_layer_forward_image: null pointer");
-  if (L->depthwise || L->cin != 3 || L->k != 3) return fail(LEDB200_EINVAL, "conv_layer_forward_image: a dense 3x3 layer on 3 input channels");
+  if (L->depthwise || L->c.cin != 3 || L->c.k != 3) return fail(LEDB200_EINVAL, "conv_layer_forward_image: a dense 3x3 layer on 3 input channels");
   if (!dt_ok(dtype)) return fail(LEDB200_EINVAL, "conv_layer_forward_image: output dtype must be F32 or BF16");
   if (img_layout != LEDB200_IMG_NCHW_F32) return fail(LEDB200_EINVAL, "conv_layer_forward_image: image layout must be NCHW fp32");
-  if (out_ld == 0) out_ld = L->cout;
-  const int Ho = (H + 2 - 3) / L->stride + 1, Wo = (W + 2 - 3) / L->stride + 1;
-  ConvArgs a;
+  if (out_ld == 0) out_ld = L->c.cout;
+  ConvArgs a = conv_args(L->c, N, H, W);
   const int64_t HW = (int64_t)H * W;
   a.in = img; a.in_dtype = LEDB200_F32; a.in_sn = 3 * HW; a.in_sc = HW; a.in_sh = W; a.in_sw = 1;
-  a.out = out; a.out_dtype = dtype; a.out_ld = out_ld;
-  a.bias = L->bias; a.w_direct = L->w_direct; a.w_tc = L->w_tc; a.cout_pad16 = L->cout_pad16; a.cout_pad_tc = L->cout_pad_tc;
-  a.N = N; a.H = H; a.W = W; a.Cin = 3; a.Ho = Ho; a.Wo = Wo; a.Cout = L->cout; a.ksize = 3; a.stride = L->stride; a.pad = 1;
-  a.dil = 1; a.relu = relu;
+  a.out = out; a.out_dtype = dtype; a.out_ld = out_ld; a.relu = relu;
   cudaStream_t st = (cudaStream_t)stream;
   if (stem_tc_eligible(a)) return launch_stem_tc(a, st);       // bf16 output, stride 2, Cout 16 / 32: tensor cores
   return launch_conv_direct(a, st);
@@ -360,21 +320,14 @@ namespace {
 int dappm_upload_conv(ledb200_dappm* D, const ledb200_preact_conv& pc, int cin, int cout, int k, const float** a, const float** b,
                       const __nv_bfloat16** w, const float** bias) {
   if (!pc.weight || !pc.bn_scale || !pc.bn_shift) return fail(LEDB200_EINVAL, "dappm_create: null parameter");
-  const int taps = k * k;
-  std::vector<float> av(pc.bn_scale, pc.bn_scale + cin), bv(pc.bn_shift, pc.bn_shift + cin);
-  std::vector<__nv_bfloat16> wt((size_t)cout * taps * cin);
-  for (int o = 0; o < cout; ++o)
-    for (int c = 0; c < cin; ++c)
-      for (int t = 0; t < taps; ++t) wt[((size_t)o * taps + t) * cin + c] = __float2bfloat16(pc.weight[((size_t)o * cin + c) * taps + t]);
   float *da = nullptr, *db = nullptr, *dbias = nullptr;
   __nv_bfloat16* dw = nullptr;
-  int rc = upload_vec(av, &da);
-  if (!rc) { D->allocs.push_back(da); rc = upload_vec(bv, &db); }
-  if (!rc) { D->allocs.push_back(db); rc = upload_vec(wt, &dw); }
+  int rc = upload(pc.bn_scale, cin * 4, (void**)&da);
+  if (!rc) { D->allocs.push_back(da); rc = upload(pc.bn_shift, cin * 4, (void**)&db); }
+  if (!rc) { D->allocs.push_back(db); rc = upload_kmajor_bf16(pc.weight, nullptr, cin, cout, k, &dw); }
   if (!rc) D->allocs.push_back(dw);
   if (!rc && pc.bias) {
-    std::vector<float> bz(pc.bias, pc.bias + cout);
-    rc = upload_vec(bz, &dbias);
+    rc = upload(pc.bias, cout * 4, (void**)&dbias);
     if (!rc) D->allocs.push_back(dbias);
   }
   *a = da; *b = db; *w = dw; *bias = dbias;

@@ -1,8 +1,17 @@
-// Launcher declarations shared by the engine (engine.cu) and the raw C-ABI ops (api.cu).
+// Launcher declarations shared by the engine (engine.cu), the layer handles (glue.cu, getb.cu, ...) and the raw C-ABI
+// ops (api.cu), and the one packed-weight format of their inference convolutions (PackedConv: fp32 Cout padded to 16 for
+// the CUDA cores, bf16 K-major with conv_tc_pad(Cout) = 32 or a multiple of 64 rows for the tensor cores).
 #pragma once
+#include <vector>
+
 #include "common.cuh"
 
 namespace ledb {
+
+// cudaMalloc + host-to-device copy of `bytes` (at least 16 are allocated).  On failure nothing stays allocated.
+int upload(const void* host, size_t bytes, void** dev);
+template <typename T>
+int upload(const std::vector<T>& host, T** dev) { return upload(host.data(), host.size() * sizeof(T), (void**)dev); }
 
 // One convolution layer (BN folded by the host side).  NHWC unless strides say otherwise.
 struct ConvArgs {
@@ -24,7 +33,7 @@ struct ConvArgs {
   const float* pre_shift = nullptr;
   int pre_relu = 1;
   const float* w_direct = nullptr;         // [k*k][Cin][cout_pad16] fp32 (device)
-  const __nv_bfloat16* w_tc = nullptr;     // [cout_padN][k*k*Cin] bf16 (device), K-major
+  const __nv_bfloat16* w_tc = nullptr;     // [cout_pad_tc][k*k*Cin] bf16 (device), K-major
   const float* w_tc32 = nullptr;           // tf32 launches: the same matrix as fp32 words (tf32-rounded)
   int tf32 = 0;                            // 1 / 3: fp32 tensors through the kind::tf32 instantiations, passes per product (training, train.cu)
   // tf32 only - one parity class (sub_a, sub_b) of the data gradient of a stride-2 convolution: a stride-1 convolution over
@@ -46,6 +55,32 @@ int launch_conv_direct(const ConvArgs& a, cudaStream_t st);
 bool conv_tc_eligible(const ConvArgs& a);
 int conv_tc_pad(int cout);   // rows of the K-major bf16 weight matrix: 32 or a multiple of 64
 int launch_conv_tc(const ConvArgs& a, cudaStream_t st);
+
+// One inference convolution resident on the device (packed_conv.cu), BatchNorm already folded, in the layouts both
+// kernels read.  k x k, padding k / 2, dilation 1.
+struct PackedConv {
+  int cin = 0, cout = 0, k = 1, stride = 1;
+  float* w_direct = nullptr;        // [k*k][cin][cout_pad16] fp32 (conv_direct)
+  __nv_bfloat16* w_tc = nullptr;    // [cout_pad_tc][k*k*cin] bf16, K-major (conv_tc)
+  float* bias = nullptr;            // [max(cout_pad16, cout_pad_tc)]; null when the conv has neither a bias nor a shift
+  float* pre_scale = nullptr;       // optional [cin] prologue BN + ReLU (CUDA-core path only)
+  float* pre_shift = nullptr;
+  int cout_pad16 = 0, cout_pad_tc = 0;
+};
+// Packs OIHW fp32 weights of c.cin -> c.cout, c.k for both kernels and uploads them.  Per output channel o the weights
+// are scaled by scale[o] and the bias is bias[o] * scale[o] + shift[o]; any of bias / scale / shift may be null.
+int pack_conv(const float* w_oihw, const float* bias, const float* scale, const float* shift, PackedConv& c);
+// The bf16 K-major matrix alone: conv_tc_pad(cout) rows (zero beyond cout), uploaded to *dev.
+int upload_kmajor_bf16(const float* w_oihw, const float* scale, int cin, int cout, int k, __nv_bfloat16** dev);
+void free_conv(PackedConv& c);
+// Weight / padding fields, Cin, Cout, ksize, stride, pad, dil, N, H, W, Ho and Wo of c on an N x H x W input.  The
+// caller sets the tensors, their strides and dtypes, relu, residual and out2.
+ConvArgs conv_args(const PackedConv& c, int N, int H, int W);
+// backend 0 = tensor cores when conv_tc_eligible, else CUDA cores; 1 = CUDA cores; 2 = tensor cores.
+bool conv_use_tc(const ConvArgs& a, int backend);
+// Launches on the kernel conv_use_tc picks; backend 2 on a shape the tensor cores do not take fails with
+// LEDB200_EINVAL ("<who>: shape not eligible for the tcgen05 path").
+int launch_conv(const ConvArgs& a, int backend, const char* who, cudaStream_t st);
 
 // One rung of the LEDHead logit ladder on the tensor cores (ladder_tc.cu):
 //   rung : out[N,H,W,24] fp16 = relu(conv3x3(in) + bias) + up2(up)

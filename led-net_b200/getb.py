@@ -13,6 +13,7 @@ import torch
 import torch.nn as nn
 
 from . import lib as L
+from .ops import fold_bn
 from .registry import MODELS
 
 
@@ -25,11 +26,6 @@ def _relative_position_index(ws):
     rel[:, :, 1] += ws - 1
     rel[:, :, 0] *= 2 * ws - 1
     return rel.sum(-1)
-
-
-def _bn_affine(bn):
-    s = bn.weight.detach().double() / torch.sqrt(bn.running_var.detach().double() + bn.eps)
-    return s, bn.bias.detach().double() - bn.running_mean.detach().double() * s
 
 
 class GlobalLocalAttention(nn.Module):
@@ -100,9 +96,9 @@ class GETBBlock(nn.Module):
     def packed_params(self):
         """host fp32 block in the order include/ledb200.h documents; BN1 folded into qkv, BN2 into fc1."""
         Cc, a = self.dim, self.attn
-        s1, t1 = _bn_affine(self.norm1)
-        s2, t2 = _bn_affine(self.norm2)
-        sp, tp = _bn_affine(a.proj[1])
+        s1, t1 = fold_bn(self.norm1)
+        s2, t2 = fold_bn(self.norm2)
+        sp, tp = fold_bn(a.proj[1])
         wq = a.qkv[0].weight.detach().double().reshape(3 * Cc, Cc)
         bq = wq @ t1 + (a.qkv[0].bias.detach().double() if a.qkv[0].bias is not None else 0.)
         relb = a.relative_position_bias_table.detach()[a.relative_position_index.view(-1)]

@@ -24,6 +24,7 @@ from . import lib as L
 from .getb import GETBBlock
 from .mfaf import Muti_AFF
 from .modules import ConvModule, BasicBlock, DAPPM, _layer, _bn
+from .ops import fold_bn
 from .seam import SEAM
 
 _DAPPM_POOLS = ((5, 2, 2), (9, 4, 4), (17, 8, 8), (0, 1, 0))     # ppm.py:66-90; k == 0: global average
@@ -60,8 +61,7 @@ class STDCModule(nn.Module):
 
 def _fold_post(conv, bn):
     """conv -> BN  =>  (w * a, (conv.bias) * a + b)   (float64 fold, fp32 result)."""
-    a = bn.weight.detach().double() / torch.sqrt(bn.running_var.detach().double() + bn.eps)
-    b = bn.bias.detach().double() - bn.running_mean.detach().double() * a
+    a, b = fold_bn(bn)
     w = conv.weight.detach().double() * a.view(-1, 1, 1, 1)
     if conv.bias is not None:
         b = b + conv.bias.detach().double() * a
@@ -69,8 +69,7 @@ def _fold_post(conv, bn):
 
 
 def _fold_pre(bn):
-    a = bn.weight.detach().double() / torch.sqrt(bn.running_var.detach().double() + bn.eps)
-    return a.float().cpu().contiguous(), (bn.bias.detach().double() - bn.running_mean.detach().double() * a).float().cpu().contiguous()
+    return tuple(t.float().cpu().contiguous() for t in fold_bn(bn))
 
 
 def _vp(t):

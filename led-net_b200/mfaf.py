@@ -11,6 +11,7 @@ import torch
 import torch.nn as nn
 
 from . import lib as L
+from .ops import fold_bn
 from .registry import MODELS
 
 
@@ -24,7 +25,7 @@ def _att(channels, inter, pool):
 
 def _fold_conv_bn(conv, bn):
     """y = BN(W x + bias)  ->  y = a * (W x) + b  (float64 fold, fp32 result)."""
-    a = bn.weight.detach().double() / torch.sqrt(bn.running_var.detach().double() + bn.eps)
+    a = fold_bn(bn)[0]
     b = bn.bias.detach().double() + (conv.bias.detach().double() - bn.running_mean.detach().double()) * a
     return conv.weight.detach().reshape(conv.out_channels, conv.in_channels).float(), a.float(), b.float()
 

@@ -14,6 +14,12 @@ def _p(t):
     return C.c_void_p(t.data_ptr()) if t is not None else None
 
 
+def fold_bn(bn):
+    """Eval BatchNorm as a per-channel affine in float64: (scale, shift) = (gamma / sqrt(var + eps), beta - mean * scale)."""
+    scale = bn.weight.detach().double() / torch.sqrt(bn.running_var.detach().double() + bn.eps)
+    return scale, bn.bias.detach().double() - bn.running_mean.detach().double() * scale
+
+
 def _need_cuda(*ts):
     for t in ts:
         if t is not None and not t.is_cuda:

@@ -12,6 +12,7 @@ import torch
 import torch.nn as nn
 
 from . import lib as L
+from .ops import fold_bn
 from .registry import MODELS
 
 
@@ -22,11 +23,6 @@ class _ConvBN(nn.Module):
         super().__init__()
         self.conv = nn.Conv2d(cin, cout, 3, padding=1, bias=False)
         self.bn = nn.BatchNorm2d(cout)
-
-
-def _fold(bn):
-    a = bn.weight.detach().double() / torch.sqrt(bn.running_var.detach().double() + bn.eps)
-    return a.float(), (bn.bias.detach().double() - bn.running_mean.detach().double() * a).float()
 
 
 @MODELS.register_module()
@@ -52,8 +48,8 @@ class SEAM(nn.Module):
         if self._packed is None or self._packed.device != device:
             if not torch.allclose(self.fusion_kernel.detach().reshape(-1).cpu(), torch.tensor([0.6, 0.3, 0.1])):
                 raise NotImplementedError('the B200 SEAM kernel hard-codes fusion_kernel = (0.6, 0.3, 0.1)')
-            a1, b1 = _fold(self.conv_1.bn)
-            a2, b2 = _fold(self.conv_2.bn)
+            a1, b1 = fold_bn(self.conv_1.bn)
+            a2, b2 = fold_bn(self.conv_2.bn)
             w1 = self.conv_1.conv.weight.detach().reshape(self.channels, 9).t().contiguous()      # [tap][C]
             w2 = self.conv_2.conv.weight.detach().reshape(self.channels, 9).t().contiguous()      # [tap][C]
             flat = torch.cat([t.float().cpu().reshape(-1) for t in (w1, a1, b1, torch.zeros(6), w2, a2, b2)])

@@ -11,6 +11,7 @@ import torch
 import torch.nn as nn
 
 from . import lib as L
+from .ops import fold_bn
 from .registry import MODELS
 
 
@@ -51,12 +52,6 @@ class _CDilated(nn.Module):
         self.conv = nn.Conv2d(n, n, 3, 1, d, d, groups=n, bias=False)
 
 
-def _fold(bn):
-    scale = bn.weight.detach().double() / torch.sqrt(bn.running_var.detach().double() + bn.eps)
-    shift = bn.bias.detach().double() - bn.running_mean.detach().double() * scale
-    return scale.float(), shift.float()
-
-
 @MODELS.register_module()
 class SESP(nn.Module):
 
@@ -91,9 +86,9 @@ class SESP(nn.Module):
         """BN folded to scale/shift, everything in the one fp32 block csrc/sesp.cu expects."""
         if self._packed is None or self._packed.device != device:
             n = self.nOut // 4
-            ps, pb = _fold(self.proj_1x1.bn)
-            bs, bb = _fold(self.br_after_cat.bn)
-            es, eb = _fold(self.conv_1x1_exp.bn)
+            ps, pb = fold_bn(self.proj_1x1.bn)
+            bs, bb = fold_bn(self.br_after_cat.bn)
+            es, eb = fold_bn(self.conv_1x1_exp.bn)
             dw2 = ([m.conv.weight.detach().reshape(-1) for m in self.spp_dw_v2] if self.SESPV2
                    else [torch.zeros(n * 9)] * 4)
             parts = [self.proj_1x1.conv.weight.detach().reshape(-1), ps, pb,
