@@ -534,6 +534,51 @@ int64_t ledb200_png_workspace_bytes(int32_t N, int32_t H, int32_t W);
 int ledb200_png_encode(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, int32_t add, uint8_t* out,
                        int64_t* offsets, void* workspace, void* stream);
 
+/* ---- PNG files -> decoded images and label maps (csrc/png_decode.cu) -----------------------------------------------------
+ * The dataset feed of LoadImageFromFile (mmcv imfrombytes, cv2 backend, flag 'color') and LoadAnnotations (pillow backend,
+ * 'unchanged') on the device.  Bit depth 8, colour types 0 / 2 / 3 / 4 / 6, no interlace; the caller reads the IHDR (at
+ * its fixed offset) and rejects everything else before the call.
+ *   LEDB200_PNG_COLOR: out [3,h,w] uint8 BGR, bit-identical to cv2.imdecode(buf, IMREAD_COLOR) transposed to CHW (grey
+ *     replicated, palette expanded through PLTE, alpha dropped, tRNS / gAMA / other ancillary chunks ignored).
+ *   LEDB200_PNG_LABEL: colour types 0 and 3 only; out [1,h,w] uint8 = lut[grey value or palette index] (lut: HOST 256
+ *     bytes, NULL = identity), i.e. np.array(Image.open(f)) through the table.
+ * One descriptor per file (HOST array): data / size = the whole file (device), out = its output (device), h / w /
+ * color_type as the IHDR states them (the device checks that they do).  status: device int32 [n], one LEDB200_PNG_*
+ * code per file; a file with a non-zero status leaves its output undefined.  Every file is decoded at once (one warp
+ * inflates each file; a block per file undoes the filters).  No file makes the kernels read outside it or write
+ * outside its output and its workspace slot, whatever its content.
+ * ledb200_png_decode_workspace_bytes: device workspace of one ledb200_png_decode call over these descriptors.
+ * ledb200_png_decode_host: the same decoder on the CPU (diagnostics, like ledb200_debug_fetch): every pointer of the
+ *   descriptors, status and lut are HOST memory; the statuses equal the device's. */
+enum { LEDB200_PNG_COLOR = 0, LEDB200_PNG_LABEL = 1 };
+enum {
+  LEDB200_PNG_OK = 0,
+  LEDB200_PNG_EHEADER = 1,      /* signature or IHDR differs from the descriptor                                 */
+  LEDB200_PNG_ECHUNK = 2,       /* chunk past the end of the file, bad chunk name, chunk order (PLTE after IDAT,
+                                   split IDAT run, second PLTE / IHDR), unknown critical chunk, no IDAT / IEND     */
+  LEDB200_PNG_ECRC = 3,         /* CRC-32 of a critical chunk (IDAT, PLTE, IEND)                                 */
+  LEDB200_PNG_EPLTE = 4,        /* palette image without a valid PLTE                                            */
+  LEDB200_PNG_EUNSUPPORTED = 5, /* an eXIf chunk (cv2 would apply its orientation)                               */
+  LEDB200_PNG_EZLIB = 6,        /* zlib header (method, window, preset dictionary, check bits), data after the
+                                   end of the zlib stream                                                        */
+  LEDB200_PNG_EDEFLATE = 7,     /* invalid deflate data: block type, stored length, Huffman code (over-subscribed,
+                                   incomplete, no end-of-block), symbol, distance before the start of the stream */
+  LEDB200_PNG_ETRUNC = 8,       /* the zlib stream ends early                                                    */
+  LEDB200_PNG_ESIZE = 9,        /* the inflated scanlines are not exactly h * (1 + w * bytes per pixel) bytes     */
+  LEDB200_PNG_EADLER = 10,      /* Adler-32 of the inflated scanlines                                            */
+  LEDB200_PNG_EFILTER = 11      /* a scanline filter type above 4                                                */
+};
+typedef struct {
+  const uint8_t* data;
+  int64_t size;
+  uint8_t* out;
+  int32_t h, w, color_type;
+} ledb200_png_file;
+int64_t ledb200_png_decode_workspace_bytes(const ledb200_png_file* files, int32_t n);
+int ledb200_png_decode(const ledb200_png_file* files, int32_t n, int32_t mode, const uint8_t* lut, void* workspace,
+                       int32_t* status, void* stream);
+int ledb200_png_decode_host(const ledb200_png_file* files, int32_t n, int32_t mode, const uint8_t* lut, int32_t* status);
+
 /* ---- layer-level operators for module compositions outside the R0 plan (the LED wiring, led_variant.py) ---------------
  * A conv layer handle is ONE mmcv ConvModule (mmcv/cnn/bricks/conv_module.py; conv k = 1 | 3, stride 1 | 2, padding k/2)
  * whose BatchNorm the caller folded into `weight` (OIHW, HOST fp32) / `bias` (nullable); `pre_scale` / `pre_shift`

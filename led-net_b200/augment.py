@@ -11,6 +11,7 @@ import numpy as np
 import torch
 
 from .registry import MODELS
+from .png_feed import decode_batch
 from .segmentor import SegDataPreProcessor, _meta
 from . import ops
 
@@ -227,6 +228,7 @@ class DeviceAugSegDataPreProcessor(SegDataPreProcessor):
         return [draw_sample(self.rng, self.aug, h, w) for h, w in shapes]
 
     def forward(self, data, training=False):
+        decode_batch(data)
         if not training:
             if self.test_resize is None:
                 return super().forward(data, False)

@@ -23,12 +23,12 @@
 #include <string>
 
 #include "kernels.h"
+#include "png_common.cuh"
 
 namespace ledb {
 namespace {
 
 constexpr int kLL = 286, kDist = 30, kCL = 19;
-constexpr uint32_t kAdlerMod = 65521;
 constexpr int64_t kStoredMax = 65535;
 // file bytes outside the zlib data: signature 8, IHDR 25, IDAT length + type 8, zlib header 2, Adler-32 4, IDAT CRC 4,
 // IEND 12
@@ -259,10 +259,9 @@ __global__ void __launch_bounds__(32) png_band_kernel(const uint8_t* __restrict_
   __syncwarp();
 
   // Adler-32 sums of this lane's nominal segment (any partition works for the sums)
-  uint64_t s1 = 0, s2 = 0;
-  for (int64_t i = a_nom; i < e_nom; ++i) { s1 += __ldg(raw + i); s2 += s1; }
-  s1 %= kAdlerMod; s2 %= kAdlerMod;
-  s2 = (s2 + s1 * ((uint64_t)(B1 - e_nom) % kAdlerMod)) % kAdlerMod;
+  uint64_t s1, s2;
+  adler_sums(raw + a_nom, e_nom - a_nom, s1, s2);
+  s2 = adler_shift(s1, s2, B1 - e_nom);
   for (int o = 16; o; o >>= 1) {
     s1 += __shfl_xor_sync(0xffffffffu, s1, o);
     s2 += __shfl_xor_sync(0xffffffffu, s2, o);
@@ -500,31 +499,6 @@ __global__ void __launch_bounds__(1024) png_scan_kernel(int64_t* __restrict__ of
   }
 }
 
-constexpr uint32_t kCrcPoly = 0xedb88320u;
-
-// a * b modulo the CRC-32 polynomial, bit-reflected (zlib's multmodp)
-__device__ uint32_t crc_multmodp(uint32_t a, uint32_t b) {
-  uint32_t m = 1u << 31, r = 0;
-  for (;;) {
-    if (a & m) {
-      r ^= b;
-      if ((a & (m - 1)) == 0) break;
-    }
-    m >>= 1;
-    b = (b & 1) ? (b >> 1) ^ kCrcPoly : b >> 1;
-  }
-  return r;
-}
-
-// crc32(A || B) from crc32(A), crc32(B) and |B|; x2n[k] = x^(2^k) mod P
-__device__ uint32_t crc_combine(uint32_t c1, uint32_t c2, int64_t len2, const uint32_t* x2n) {
-  uint32_t pw = 1u << 31;                       // x^0
-  int k = 3;                                    // x^(8 len2): start at 2^3
-  for (int64_t n = len2; n; n >>= 1, ++k)
-    if (n & 1) pw = crc_multmodp(x2n[k & 31], pw);
-  return crc_multmodp(pw, c1) ^ c2;
-}
-
 __device__ __forceinline__ void put_be32(uint8_t* p, uint32_t v) {
   p[0] = (uint8_t)(v >> 24); p[1] = (uint8_t)(v >> 16); p[2] = (uint8_t)(v >> 8); p[3] = (uint8_t)v;
 }
@@ -540,15 +514,10 @@ __global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W,
   uint8_t* f = out + offsets[img];
   const int64_t size = offsets[img + 1] - offsets[img];
   const int64_t idat_len = size - kFileOverhead + 2 + 4;   // zlib header + deflate data + Adler-32
-  {
-    uint32_t c = (uint32_t)t;
-    for (int k = 0; k < 8; ++k) c = (c & 1) ? (c >> 1) ^ kCrcPoly : c >> 1;
-    tab[t] = c;
-  }
+  tab[t] = crc_table_entry((uint32_t)t);
   __syncthreads();
   if (t == 0) {
-    x2n[0] = 1u << 30;                          // x^1
-    for (int k = 1; k < 32; ++k) x2n[k] = crc_multmodp(x2n[k - 1], x2n[k - 1]);
+    crc_x2n_table(x2n);
     const uint8_t sig[8] = {0x89, 'P', 'N', 'G', 0x0d, 0x0a, 0x1a, 0x0a};
     for (int k = 0; k < 8; ++k) f[k] = sig[k];
     uint8_t* h = f + 8;
@@ -556,9 +525,7 @@ __global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W,
     h[4] = 'I'; h[5] = 'H'; h[6] = 'D'; h[7] = 'R';
     put_be32(h + 8, (uint32_t)W); put_be32(h + 12, (uint32_t)H);
     h[16] = 8; h[17] = 0; h[18] = 0; h[19] = 0; h[20] = 0;   // bit depth 8, grayscale, deflate, filter 0, no interlace
-    uint32_t c = 0xffffffffu;
-    for (int k = 4; k < 21; ++k) c = tab[(c ^ h[k]) & 0xff] ^ (c >> 8);
-    put_be32(h + 21, ~c);
+    put_be32(h + 21, ~crc_update(tab, 0xffffffffu, h + 4, 17));
     uint8_t* d = f + 33;
     put_be32(d, (uint32_t)idat_len);
     d[4] = 'I'; d[5] = 'D'; d[6] = 'A'; d[7] = 'T';
@@ -581,9 +548,7 @@ __global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W,
   const int64_t clen = 4 + idat_len, per = (clen + 255) / 256;
   const int64_t c0 = min(clen, t * per), c1 = min(clen, c0 + per);
   const uint8_t* q = f + 37;
-  uint32_t c = 0xffffffffu;
-  for (int64_t i = c0; i < c1; ++i) c = tab[(c ^ q[i]) & 0xff] ^ (c >> 8);
-  crc_s[t] = ~c; len_s[t] = c1 - c0;
+  crc_s[t] = ~crc_update(tab, 0xffffffffu, q + c0, c1 - c0); len_s[t] = c1 - c0;
   __syncthreads();
   for (int s = 1; s < 256; s <<= 1) {
     if ((t & (2 * s - 1)) == 0) {

@@ -38,6 +38,7 @@ SYMBOLS = [
     'ledb200_postprocess', 'ledb200_slide_accumulate', 'ledb200_slide_finalize', 'ledb200_slide_merge', 'ledb200_stack_pad',
     'ledb200_tta_merge', 'ledb200_crop_select', 'ledb200_train_augment', 'ledb200_view_resize',
     'ledb200_png_bound', 'ledb200_png_workspace_bytes', 'ledb200_png_encode',
+    'ledb200_png_decode_workspace_bytes', 'ledb200_png_decode', 'ledb200_png_decode_host',
     'ledb200_seam_param_floats', 'ledb200_seam_workspace_bytes', 'ledb200_seam_forward',
     'ledb200_conv_layer_create', 'ledb200_conv_layer_forward', 'ledb200_conv_layer_destroy',
     'ledb200_avgpool2d', 'ledb200_resize_bilinear', 'ledb200_add_relu', 'ledb200_conv_layer_forward_image',
@@ -77,6 +78,30 @@ class ViewDesc(C.Structure):
     """ledb200_view_desc: one decoded uint8 [3,h,w] source, its resized size and the unflipped / flipped outputs."""
     _fields_ = [('src', C.c_void_p), ('out', C.c_void_p), ('out_flip', C.c_void_p), ('h', C.c_int32), ('w', C.c_int32),
                 ('rh', C.c_int32), ('rw', C.c_int32)]
+
+
+class PngFile(C.Structure):
+    """ledb200_png_file: one PNG file (its bytes and size), its output and the IHDR's h, w and colour type."""
+    _fields_ = [('data', C.c_void_p), ('size', C.c_int64), ('out', C.c_void_p), ('h', C.c_int32), ('w', C.c_int32),
+                ('color_type', C.c_int32)]
+
+
+PNG_COLOR, PNG_LABEL = 0, 1
+# ledb200_png_decode's per-file status codes (include/ledb200.h LEDB200_PNG_*)
+PNG_STATUS = {
+    1: 'signature or IHDR does not match the descriptor',
+    2: 'malformed chunk layout (a chunk past the end of the file, a bad chunk name or order, an unknown critical '
+       'chunk, or no IDAT / IEND)',
+    3: 'CRC-32 mismatch in a critical chunk',
+    4: 'palette image without a valid PLTE chunk',
+    5: 'unsupported: the file has an eXIf chunk (EXIF orientation is not applied)',
+    6: 'invalid zlib header, or data after the end of the zlib stream',
+    7: 'invalid deflate data',
+    8: 'the compressed data ends early',
+    9: 'wrong number of decompressed bytes for the image size',
+    10: 'Adler-32 mismatch of the decompressed data',
+    11: 'invalid scanline filter type',
+}
 
 
 _lib = None
@@ -190,6 +215,10 @@ def get():
     lib.ledb200_png_workspace_bytes.argtypes = [i32, i32, i32]
     lib.ledb200_png_workspace_bytes.restype = i64
     lib.ledb200_png_encode.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp]
+    lib.ledb200_png_decode_workspace_bytes.argtypes = [C.POINTER(PngFile), i32]
+    lib.ledb200_png_decode_workspace_bytes.restype = i64
+    lib.ledb200_png_decode.argtypes = [C.POINTER(PngFile), i32, i32, vp, vp, vp, vp]
+    lib.ledb200_png_decode_host.argtypes = [C.POINTER(PngFile), i32, i32, vp, vp]
     lib.ledb200_conv_layer_create.argtypes = [vp, vp, vp, vp] + [i32] * 5 + [C.POINTER(vp)]
     lib.ledb200_conv_layer_forward.argtypes = [vp, vp, vp, vp] + [i32] * 9 + [vp]
     lib.ledb200_conv_layer_destroy.argtypes = [vp]

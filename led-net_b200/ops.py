@@ -4,7 +4,10 @@ Layout changes between the reference's NCHW tensors and the library's NHWC are v
 with torch (plumbing); the arithmetic is in the CUDA kernels.
 """
 import ctypes as C
+import struct
+import zlib
 
+import numpy as np
 import torch
 
 from . import lib as L
@@ -374,3 +377,146 @@ def png_encode(labels, add=0):
     offs = offsets.cpu().tolist()
     data = out[:offs[-1]].cpu().numpy().tobytes()
     return [data[offs[i]:offs[i + 1]] for i in range(N)]
+
+
+PNG_SIGNATURE = b'\x89PNG\r\n\x1a\n'
+MAX_PNG_PIXELS = 1 << 30      # OpenCV's default CV_IO_MAX_IMAGE_PIXELS
+
+
+def _head(f, n):
+    """the first n bytes of a file given as bytes-like or a 1-D uint8 tensor (a device tensor costs one small copy)"""
+    if isinstance(f, torch.Tensor):
+        if f.dtype != torch.uint8 or f.dim() != 1:
+            raise L.LedB200Error('PNG files are bytes or 1-D uint8 tensors')
+        return f[:n].cpu().numpy().tobytes()
+    return bytes(memoryview(f)[:n])
+
+
+def png_info(f, kind='color'):
+    """(h, w, colour type) from the IHDR of a PNG file (bytes-like or 1-D uint8 tensor), which sits at a fixed offset
+    after the signature.  Checks the signature, the IHDR's length, name and CRC, and the sizes; a malformed header raises
+    LedB200Error, a valid PNG outside what png_decode supports raises NotImplementedError: bit depths other than 8,
+    interlaced (Adam7) files and, for kind='label', colour types 2 / 4 / 6."""
+    b = _head(f, 33)
+    if len(b) < 33 or b[:8] != PNG_SIGNATURE:
+        raise L.LedB200Error('not a PNG file (no PNG signature)')
+    if b[8:16] != b'\x00\x00\x00\x0dIHDR':
+        raise L.LedB200Error('the first chunk is not a 13-byte IHDR')
+    if zlib.crc32(b[12:29]) != struct.unpack('>I', b[29:33])[0]:
+        raise L.LedB200Error('IHDR CRC-32 mismatch')
+    w, h, depth, ct, comp, filt, interlace = struct.unpack('>IIBBBBB', b[16:29])
+    if not (1 <= w < 1 << 31 and 1 <= h < 1 << 31):
+        raise L.LedB200Error(f'IHDR: invalid size {w} x {h}')
+    if ct not in (0, 2, 3, 4, 6) or depth not in (1, 2, 4, 8, 16) or comp or filt or interlace > 1:
+        raise L.LedB200Error(f'IHDR: invalid header (bit depth {depth}, colour type {ct}, compression {comp}, '
+                             f'filter {filt}, interlace {interlace})')
+    if depth != 8:
+        raise NotImplementedError(f'{depth}-bit PNG files (png_decode reads bit depth 8)')
+    if interlace:
+        raise NotImplementedError('interlaced (Adam7) PNG files')
+    if kind == 'label' and ct not in (0, 3):
+        raise NotImplementedError(f'label maps of colour type {ct} (grey or palette only)')
+    if h * w > MAX_PNG_PIXELS:
+        raise L.LedB200Error(f'{w} x {h} is more than {MAX_PNG_PIXELS} pixels')
+    return h, w, ct
+
+
+def label_lut(reduce_zero_label=False, label_map=None):
+    """The 256-entry uint8 table that maps a stored label value to what LoadAnnotations._load_seg_map gives.
+
+    mmseg 1.2.2, mmseg/datasets/transforms/loading.py, LoadAnnotations._load_seg_map, restated here from the released
+    source (the reference checkout is not part of this repository), applies, to the uint8 map:
+      1. reduce_zero_label: 0 -> 255, then v - 1 (uint8), then 254 -> 255;
+      2. label_map: for each (old, new), map[copy == old] = new, where `copy` is the map after step 1 (every
+         replacement reads the values before any of them)."""
+    v = np.arange(256, dtype=np.uint8)
+    if reduce_zero_label:
+        v[v == 0] = 255
+        v = v - np.uint8(1)
+        v[v == 254] = 255
+    if label_map is not None:
+        src = v.copy()
+        for old, new in label_map.items():
+            if not 0 <= int(new) <= 255:
+                raise ValueError(f'label_map value {new} does not fit a uint8 label map')
+            v[src == old] = new
+    return v
+
+
+def png_decode(files, kind='color', reduce_zero_label=False, label_map=None, names=None, device=None):
+    """PNG files -> CUDA uint8 tensors, decoded on the device (csrc/png_decode.cu).
+
+    files: bytes-like objects or 1-D uint8 tensors (host or device), bit depth 8, not interlaced.
+    kind='color': each result is [3, h, w] BGR, bit-identical to cv2.imdecode(buf, cv2.IMREAD_COLOR).transpose(2, 0, 1)
+      (what LoadImageFromFile gives): grey replicated, palettes expanded, alpha dropped, ancillary chunks ignored.
+    kind='label': grey or palette files; each result is [1, h, w], the stored values (palette indices, not colours: what
+      np.array(Image.open(f)) gives) through label_lut(reduce_zero_label, label_map), as LoadAnnotations gives them.
+    The host reads each IHDR (png_info), packs the host files into one pinned buffer and uploads it with one copy; one
+    decode call covers every file and one small copy brings the statuses back.  A file that fails raises LedB200Error
+    naming it (names[i], default 'file i') and the reason."""
+    if kind not in ('color', 'label'):
+        raise ValueError(f"kind must be 'color' or 'label', not {kind!r}")
+    files = list(files)
+    n = len(files)
+    if n == 0:
+        return []
+    names = list(names) if names is not None else [f'file {i}' for i in range(n)]
+    infos = []
+    for f, name in zip(files, names):
+        try:
+            infos.append(png_info(f, kind))
+        except NotImplementedError as e:
+            raise NotImplementedError(f'{name}: {e}') from None
+        except L.LedB200Error as e:
+            raise L.LedB200Error(f'{name}: {e}') from None
+    if device is None:
+        device = next((f.device for f in files if isinstance(f, torch.Tensor) and f.is_cuda), None)
+    if device is None:
+        if not torch.cuda.is_available():
+            raise L.LedB200Error('png_decode decodes on a CUDA device (no CPU fallback)')
+        device = torch.device('cuda', torch.cuda.current_device())
+    dev = torch.device(device)
+    if dev.type != 'cuda':
+        raise L.LedB200Error('png_decode decodes on a CUDA device (no CPU fallback)')
+    # host files: one pinned staging buffer, one host-to-device copy
+    host = [i for i, f in enumerate(files) if not (isinstance(f, torch.Tensor) and f.is_cuda)]
+    sizes = [f.numel() if isinstance(f, torch.Tensor) else memoryview(f).nbytes for f in files]
+    data = [None] * n
+    if host:
+        offs = np.cumsum([0] + [sizes[i] for i in host])
+        pinned = torch.empty(int(offs[-1]), dtype=torch.uint8, pin_memory=True)
+        view = pinned.numpy()
+        for k, i in enumerate(host):
+            f = files[i]
+            src = f.contiguous().numpy() if isinstance(f, torch.Tensor) else np.frombuffer(f, np.uint8)
+            view[offs[k]:offs[k + 1]] = src
+        up = pinned.to(dev, non_blocking=True)
+        for k, i in enumerate(host):
+            data[i] = up[offs[k]:offs[k + 1]]
+    for i, f in enumerate(files):
+        if data[i] is None:
+            data[i] = f.to(dev).contiguous()
+    ch = 3 if kind == 'color' else 1
+    numel = [ch * h * w for h, w, _ in infos]
+    flat = torch.empty(sum(numel), dtype=torch.uint8, device=dev)
+    outs, at = [], 0
+    for (h, w, _), m in zip(infos, numel):
+        outs.append(flat[at:at + m].view(ch, h, w))
+        at += m
+    arr = (L.PngFile * n)()
+    for d, t, o, (h, w, ct), sz in zip(arr, data, outs, infos, sizes):
+        d.data, d.size, d.out, d.h, d.w, d.color_type = t.data_ptr(), sz, o.data_ptr(), h, w, ct
+    lib = L.get()
+    ws = torch.empty(max(1, L.check(lib.ledb200_png_decode_workspace_bytes(arr, n), 'ledb200_png_decode_workspace_bytes')),
+                     dtype=torch.uint8, device=dev)
+    status = torch.empty(n, dtype=torch.int32, device=dev)
+    lut = None
+    if kind == 'label':
+        lut = (C.c_uint8 * 256)(*label_lut(reduce_zero_label, label_map).tolist())
+    L.check(lib.ledb200_png_decode(arr, n, L.PNG_LABEL if kind == 'label' else L.PNG_COLOR, lut, _p(ws), _p(status),
+                                   L.stream_ptr(dev)), 'ledb200_png_decode')
+    st = status.cpu().tolist()
+    bad = [(names[i], L.PNG_STATUS.get(c, f'status {c}')) for i, c in enumerate(st) if c]
+    if bad:
+        raise L.LedB200Error('png_decode: ' + '; '.join(f'{nm}: {why}' for nm, why in bad))
+    return outs

@@ -1,0 +1,95 @@
+"""PNG files straight into the device preprocessors: `PackSegPNGFiles` (TRANSFORMS) and `decode_batch`.
+
+A dataset pipeline of LoadImageFromFile, LoadAnnotations and PackSegInputs decodes every file on a dataloader worker
+(cv2 / PIL) and moves the decoded uint8 arrays.  `PackSegPNGFiles` replaces the three: it reads the files' bytes and the
+IHDR, and packs the file bytes with the metainfo PackSegInputs would set.  `decode_batch`, called at the top of
+SegDataPreProcessor.forward, DeviceAugSegDataPreProcessor.forward and SegTTAModel's device-view test_step, decodes such a
+batch on the device (ops.png_decode: one call for the images, one for the label maps) into exactly the batch the
+decoded path delivers, so everything after it runs unchanged.
+"""
+import torch
+
+from .registry import TRANSFORMS
+from . import ops
+
+
+def _read(path):
+    with open(path, 'rb') as f:
+        return f.read()
+
+
+def _as_tensor(b):
+    return torch.frombuffer(bytearray(b), dtype=torch.uint8)
+
+
+@TRANSFORMS.register_module()
+class PackSegPNGFiles:
+    """LoadImageFromFile + LoadAnnotations + PackSegInputs for PNG datasets, without decoding.
+
+    Returns dict(inputs=<the image file as a 1-D uint8 tensor>, data_samples=<sample dict>), the sample holding
+    `metainfo` (img_path, ori_shape and img_shape from the IHDR, and with a label map seg_map_path, reduce_zero_label and
+    label_map) and, when `seg_map_path` is set, the label file as `gt_seg_map_file`.  reduce_zero_label: None takes the
+    dataset's results['reduce_zero_label'], as LoadAnnotations does.  A file png_decode cannot read (16-bit, interlaced,
+    a colour label map) raises NotImplementedError here, on the worker."""
+
+    def __init__(self, reduce_zero_label=None):
+        self.reduce_zero_label = reduce_zero_label
+
+    def __call__(self, results):
+        img_path = results['img_path']
+        img = _read(img_path)
+        h, w, _ = ops.png_info(img)
+        meta = dict(img_path=img_path, ori_shape=(h, w), img_shape=(h, w))
+        sample = dict(metainfo=meta)
+        seg_path = results.get('seg_map_path', None)
+        if seg_path is not None:
+            rzl = self.reduce_zero_label
+            if rzl is None:
+                rzl = results.get('reduce_zero_label', False)
+            assert rzl == results.get('reduce_zero_label', rzl), \
+                'Initialize dataset with `reduce_zero_label` consistently with PackSegPNGFiles'
+            seg = _read(seg_path)
+            ops.png_info(seg, 'label')
+            meta.update(seg_map_path=seg_path, reduce_zero_label=bool(rzl), label_map=results.get('label_map', None))
+            sample['gt_seg_map_file'] = _as_tensor(seg)
+        elif 'reduce_zero_label' in results:
+            meta['reduce_zero_label'] = results['reduce_zero_label']
+        return dict(inputs=_as_tensor(img), data_samples=sample)
+
+    def __repr__(self):
+        return f'{self.__class__.__name__}(reduce_zero_label={self.reduce_zero_label})'
+
+
+def _is_file(x):
+    if isinstance(x, torch.Tensor):
+        return x.dtype == torch.uint8 and x.dim() == 1
+    return isinstance(x, (bytes, bytearray, memoryview))
+
+
+def _meta(s):
+    return s.get('metainfo', s) if isinstance(s, dict) else {}
+
+
+def decode_batch(data):
+    """Decodes a batch of PackSegPNGFiles outputs in place: data['inputs'] becomes the [3, h, w] uint8 BGR images and
+    each sample's `gt_seg_map_file` becomes gt_sem_seg['data'], the [1, h, w] uint8 label map.  A batch of decoded
+    images is returned untouched.  Returns `data`."""
+    inputs = data.get('inputs', None) if isinstance(data, dict) else None
+    if not isinstance(inputs, (list, tuple)) or not inputs or not all(_is_file(x) for x in inputs):
+        return data
+    samples = data.get('data_samples', None)
+    metas = [_meta(s) for s in samples] if samples is not None else [{} for _ in inputs]
+    names = [m.get('img_path', f'image {i}') for i, m in enumerate(metas)]
+    data['inputs'] = ops.png_decode(inputs, 'color', names=names)
+    withlab = [i for i, s in enumerate(samples or []) if isinstance(s, dict) and 'gt_seg_map_file' in s]
+    if withlab:
+        rzl = {bool(metas[i].get('reduce_zero_label', False)) for i in withlab}
+        lmaps = {repr(metas[i].get('label_map', None)) for i in withlab}
+        if len(rzl) != 1 or len(lmaps) != 1:
+            raise NotImplementedError('the label maps of one batch must share reduce_zero_label and label_map')
+        labels = ops.png_decode([samples[i].pop('gt_seg_map_file') for i in withlab], 'label',
+                                reduce_zero_label=rzl.pop(), label_map=metas[withlab[0]].get('label_map', None),
+                                names=[metas[i].get('seg_map_path', f'label map {i}') for i in withlab])
+        for i, lab in zip(withlab, labels):
+            samples[i]['gt_sem_seg'] = dict(data=lab)
+    return data

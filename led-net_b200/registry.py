@@ -48,16 +48,19 @@ class Registry:
 
 MODELS = Registry('model')
 METRICS = Registry('metric')
+TRANSFORMS = Registry('transform')      # dataset pipeline steps (mmseg/registry/registry.py TRANSFORMS)
 
 
 def register_into_mmseg():
     """Register the B200 modules in a real mmseg install (returns False if mmseg is absent)."""
     try:
-        from mmseg.registry import MODELS as MM, METRICS as MT
+        from mmseg.registry import MODELS as MM, METRICS as MT, TRANSFORMS as TR
     except Exception:
         return False
     for k, v in MODELS._table.items():
         MM.register_module(name=k, force=True, module=v)
     for k, v in METRICS._table.items():
         MT.register_module(name=k, force=True, module=v)
+    for k, v in TRANSFORMS._table.items():
+        TR.register_module(name=k, force=True, module=v)
     return True

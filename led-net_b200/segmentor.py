@@ -13,6 +13,7 @@ import torch.nn.functional as F
 from .engine import Engine, MEAN, STD
 from .registry import MODELS
 from . import ops
+from .png_feed import decode_batch
 
 
 def _meta(sample):
@@ -75,6 +76,7 @@ class SegDataPreProcessor(nn.Module):
         return mh, mw
 
     def forward(self, data, training=False):
+        decode_batch(data)
         inputs = data['inputs']
         samples = data.get('data_samples', None)
         inputs = list(inputs) if isinstance(inputs, (list, tuple)) else list(inputs.unbind(0))

@@ -14,6 +14,7 @@ import torch
 import torch.nn as nn
 
 from .augment import device_images, parse_tta_transforms, view_meta, view_size
+from .png_feed import decode_batch
 from .registry import MODELS
 from .segmentor import SegDataPreProcessor, _meta, _view_geometry
 from . import ops
@@ -225,6 +226,7 @@ class SegTTAModel(nn.Module):
     def _test_step_device_views(self, data):
         if isinstance(data, (list, tuple)):
             data = dict(zip(('inputs', 'data_samples'), data))
+        decode_batch(data)
         images = self._images(data['inputs'])
         n = len(images)
         samples = data.get('data_samples') or [{} for _ in range(n)]
