@@ -579,6 +579,50 @@ int ledb200_png_decode(const ledb200_png_file* files, int32_t n, int32_t mode, c
                        int32_t* status, void* stream);
 int ledb200_png_decode_host(const ledb200_png_file* files, int32_t n, int32_t mode, const uint8_t* lut, int32_t* status);
 
+/* ---- baseline JPEG files -> decoded images (csrc/jpeg_decode.cu) ---------------------------------------------------------
+ * LoadImageFromFile (mmcv imfrombytes, cv2 backend, flag 'color') on the device for JPEG files: out [3,h,w] uint8 BGR,
+ * bit-identical to cv2.imdecode(buf, IMREAD_COLOR) transposed to CHW (libjpeg-turbo, JDCT_ISLOW, fancy upsampling).
+ * Supported: SOF0 / SOF1, 8-bit precision, Huffman coding, one interleaved scan carrying every component; 1 component
+ * (grey, replicated) or 3 that libjpeg treats as YCbCr, with luma sampling factors in {1, 2} x {1, 2} and chroma 1 x 1
+ * (4:4:4, 4:2:2, 4:2:0, 4:4:0); any restart interval.  The caller walks the markers to the first SOS and refuses the
+ * rest before the call (lednet_b200.ops.jpeg_info); the device refuses them too, with LEDB200_JPEG_EUNSUPPORTED.
+ * Unlike libjpeg, which warns and fills the rest of the image with grey, corrupt entropy-coded data is an error.
+ * One descriptor per file (HOST array): data / size = the whole file (device, size < 2^28), out = its output (device),
+ * h / w / components as the frame header states them (the device checks that they do).  status: device int32 [n], one
+ * LEDB200_JPEG_* code per file; a file with a non-zero status leaves its output undefined.  Every file of a call is
+ * decoded by one sequence of launches, and every stage but the header walk splits each file over many threads.  No
+ * file makes the kernels read outside it or write outside its output and its workspace slot, whatever its content.
+ * ledb200_jpeg_decode_workspace_bytes: device workspace of one ledb200_jpeg_decode call over these descriptors (a
+ *   bound that holds for every accepted sampling).
+ * ledb200_jpeg_decode_host: the same decoder on the CPU (diagnostics): every pointer of the descriptors and status is
+ *   HOST memory; the statuses equal the device's. */
+enum {
+  LEDB200_JPEG_OK = 0,
+  LEDB200_JPEG_EHEADER = 1,     /* no SOI, or the frame header's height, width or components differ from the
+                                   descriptor                                                                    */
+  LEDB200_JPEG_ESEGMENT = 2,    /* marker structure: a segment length past the end of the file or wrong for its
+                                   marker, a marker out of place (a second SOF, SOS before SOF, RSTn / EOI / DNL
+                                   before the scan, an unknown marker), the scan not followed by EOI, zero width   */
+  LEDB200_JPEG_EUNSUPPORTED = 3,/* progressive, lossless, hierarchical or arithmetic-coded, not 8-bit, 2 or 4
+                                   components, RGB colour space, other sampling factors, a non-interleaved scan,
+                                   height 0 (DNL), an Exif orientation other than 1 (cv2 would rotate)             */
+  LEDB200_JPEG_ETABLE = 4,      /* bad DQT / DHT (table class or id, length, over-subscribed or all-ones Huffman
+                                   code, DC symbol above 15), or a table the frame or scan refers to is missing  */
+  LEDB200_JPEG_EHUFF = 5,       /* a bit pattern that is no code of the Huffman table in use                     */
+  LEDB200_JPEG_ETRUNC = 6,      /* the entropy-coded data ends before the last MCU (of the scan or an interval) */
+  LEDB200_JPEG_ERESTART = 7,    /* an RSTn out of sequence, or more or fewer RSTn than the restart interval needs */
+  LEDB200_JPEG_EZZ = 8          /* an AC run that takes the coefficient index past 63                            */
+};
+typedef struct {
+  const uint8_t* data;
+  int64_t size;
+  uint8_t* out;
+  int32_t h, w, components;
+} ledb200_jpeg_file;
+int64_t ledb200_jpeg_decode_workspace_bytes(const ledb200_jpeg_file* files, int32_t n);
+int ledb200_jpeg_decode(const ledb200_jpeg_file* files, int32_t n, void* workspace, int32_t* status, void* stream);
+int ledb200_jpeg_decode_host(const ledb200_jpeg_file* files, int32_t n, int32_t* status);
+
 /* ---- layer-level operators for module compositions outside the R0 plan (the LED wiring, led_variant.py) ---------------
  * A conv layer handle is ONE mmcv ConvModule (mmcv/cnn/bricks/conv_module.py; conv k = 1 | 3, stride 1 | 2, padding k/2)
  * whose BatchNorm the caller folded into `weight` (OIHW, HOST fp32) / `bias` (nullable); `pre_scale` / `pre_shift`

@@ -1,6 +1,6 @@
 """led-net_b200: the LED-Net data-parallel hot path as hand-written sm_100a CUDA kernels behind
 the reference's mmseg registry surface (MODELS: LEDNet, LEDHead, OhemCrossEntropy, EncoderDecoder,
-SegDataPreProcessor, DeviceAugSegDataPreProcessor, SegTTAModel; METRICS: IoUMetric; TRANSFORMS: PackSegPNGFiles).  Host code is Python/PyTorch plumbing over the C ABI in
+SegDataPreProcessor, DeviceAugSegDataPreProcessor, SegTTAModel; METRICS: IoUMetric; TRANSFORMS: PackSegFiles, PackSegPNGFiles).  Host code is Python/PyTorch plumbing over the C ABI in
 include/ledb200.h; there is no CPU fallback."""
 __version__ = '0.1.0'
 
@@ -12,7 +12,7 @@ from .metrics import IoUMetric  # noqa: F401
 from .segmentor import EncoderDecoder, SegDataPreProcessor  # noqa: F401
 from .tta import SegTTAModel  # noqa: F401
 from .augment import DeviceAugSegDataPreProcessor  # noqa: F401
-from .png_feed import PackSegPNGFiles, decode_batch  # noqa: F401
+from .png_feed import PackSegFiles, PackSegPNGFiles, decode_batch  # noqa: F401
 from .engine import Engine  # noqa: F401
 from .sesp import SESP  # noqa: F401
 from .mfaf import Muti_AFF  # noqa: F401

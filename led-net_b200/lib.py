@@ -39,6 +39,7 @@ SYMBOLS = [
     'ledb200_tta_merge', 'ledb200_crop_select', 'ledb200_train_augment', 'ledb200_view_resize',
     'ledb200_png_bound', 'ledb200_png_workspace_bytes', 'ledb200_png_encode',
     'ledb200_png_decode_workspace_bytes', 'ledb200_png_decode', 'ledb200_png_decode_host',
+    'ledb200_jpeg_decode_workspace_bytes', 'ledb200_jpeg_decode', 'ledb200_jpeg_decode_host',
     'ledb200_seam_param_floats', 'ledb200_seam_workspace_bytes', 'ledb200_seam_forward',
     'ledb200_conv_layer_create', 'ledb200_conv_layer_forward', 'ledb200_conv_layer_destroy',
     'ledb200_avgpool2d', 'ledb200_resize_bilinear', 'ledb200_add_relu', 'ledb200_conv_layer_forward_image',
@@ -101,6 +102,26 @@ PNG_STATUS = {
     9: 'wrong number of decompressed bytes for the image size',
     10: 'Adler-32 mismatch of the decompressed data',
     11: 'invalid scanline filter type',
+}
+
+
+class JpegFile(C.Structure):
+    """ledb200_jpeg_file: one baseline JPEG file (its bytes and size), its output and the frame's h, w, components."""
+    _fields_ = [('data', C.c_void_p), ('size', C.c_int64), ('out', C.c_void_p), ('h', C.c_int32), ('w', C.c_int32),
+                ('components', C.c_int32)]
+
+
+# ledb200_jpeg_decode's per-file status codes (include/ledb200.h LEDB200_JPEG_*)
+JPEG_STATUS = {
+    1: 'no SOI, or the frame header does not match the descriptor',
+    2: 'malformed marker structure (a segment past the end of the file or of the wrong length, a marker out of '
+       'place, or the scan not followed by EOI)',
+    3: 'unsupported: not a baseline 8-bit interleaved YCbCr / grey file, or an Exif orientation other than 1',
+    4: 'invalid or missing quantisation / Huffman table',
+    5: 'invalid Huffman code in the entropy-coded data',
+    6: 'the entropy-coded data ends early',
+    7: 'restart marker out of sequence or missing',
+    8: 'coefficient index past 63',
 }
 
 
@@ -219,6 +240,10 @@ def get():
     lib.ledb200_png_decode_workspace_bytes.restype = i64
     lib.ledb200_png_decode.argtypes = [C.POINTER(PngFile), i32, i32, vp, vp, vp, vp]
     lib.ledb200_png_decode_host.argtypes = [C.POINTER(PngFile), i32, i32, vp, vp]
+    lib.ledb200_jpeg_decode_workspace_bytes.argtypes = [C.POINTER(JpegFile), i32]
+    lib.ledb200_jpeg_decode_workspace_bytes.restype = i64
+    lib.ledb200_jpeg_decode.argtypes = [C.POINTER(JpegFile), i32, vp, vp, vp]
+    lib.ledb200_jpeg_decode_host.argtypes = [C.POINTER(JpegFile), i32, vp]
     lib.ledb200_conv_layer_create.argtypes = [vp, vp, vp, vp] + [i32] * 5 + [C.POINTER(vp)]
     lib.ledb200_conv_layer_forward.argtypes = [vp, vp, vp, vp] + [i32] * 9 + [vp]
     lib.ledb200_conv_layer_destroy.argtypes = [vp]

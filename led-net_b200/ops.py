@@ -387,7 +387,7 @@ def _head(f, n):
     """the first n bytes of a file given as bytes-like or a 1-D uint8 tensor (a device tensor costs one small copy)"""
     if isinstance(f, torch.Tensor):
         if f.dtype != torch.uint8 or f.dim() != 1:
-            raise L.LedB200Error('PNG files are bytes or 1-D uint8 tensors')
+            raise L.LedB200Error('files are bytes or 1-D uint8 tensors')
         return f[:n].cpu().numpy().tobytes()
     return bytes(memoryview(f)[:n])
 
@@ -443,41 +443,22 @@ def label_lut(reduce_zero_label=False, label_map=None):
     return v
 
 
-def png_decode(files, kind='color', reduce_zero_label=False, label_map=None, names=None, device=None):
-    """PNG files -> CUDA uint8 tensors, decoded on the device (csrc/png_decode.cu).
-
-    files: bytes-like objects or 1-D uint8 tensors (host or device), bit depth 8, not interlaced.
-    kind='color': each result is [3, h, w] BGR, bit-identical to cv2.imdecode(buf, cv2.IMREAD_COLOR).transpose(2, 0, 1)
-      (what LoadImageFromFile gives): grey replicated, palettes expanded, alpha dropped, ancillary chunks ignored.
-    kind='label': grey or palette files; each result is [1, h, w], the stored values (palette indices, not colours: what
-      np.array(Image.open(f)) gives) through label_lut(reduce_zero_label, label_map), as LoadAnnotations gives them.
-    The host reads each IHDR (png_info), packs the host files into one pinned buffer and uploads it with one copy; one
-    decode call covers every file and one small copy brings the statuses back.  A file that fails raises LedB200Error
-    naming it (names[i], default 'file i') and the reason."""
-    if kind not in ('color', 'label'):
-        raise ValueError(f"kind must be 'color' or 'label', not {kind!r}")
-    files = list(files)
+def _decode_files(files, names, infos, ch, device, who, launch, status_names):
+    """The host side shared by png_decode and jpeg_decode: files (bytes-like or 1-D uint8 tensors, host or device) are
+    staged, the host ones packed into one pinned buffer and uploaded with one copy; one [ch, h, w] uint8 output per
+    file (infos[i] starts with h, w) is carved from one allocation; launch(arr_args) runs the decode call, given the
+    device copies of the files, their sizes and the outputs, and returns the int32 status tensor, read back with one
+    copy.  A file with a non-zero status raises LedB200Error naming it and status_names' reason."""
     n = len(files)
-    if n == 0:
-        return []
-    names = list(names) if names is not None else [f'file {i}' for i in range(n)]
-    infos = []
-    for f, name in zip(files, names):
-        try:
-            infos.append(png_info(f, kind))
-        except NotImplementedError as e:
-            raise NotImplementedError(f'{name}: {e}') from None
-        except L.LedB200Error as e:
-            raise L.LedB200Error(f'{name}: {e}') from None
     if device is None:
         device = next((f.device for f in files if isinstance(f, torch.Tensor) and f.is_cuda), None)
     if device is None:
         if not torch.cuda.is_available():
-            raise L.LedB200Error('png_decode decodes on a CUDA device (no CPU fallback)')
+            raise L.LedB200Error(f'{who} decodes on a CUDA device (no CPU fallback)')
         device = torch.device('cuda', torch.cuda.current_device())
     dev = torch.device(device)
     if dev.type != 'cuda':
-        raise L.LedB200Error('png_decode decodes on a CUDA device (no CPU fallback)')
+        raise L.LedB200Error(f'{who} decodes on a CUDA device (no CPU fallback)')
     # host files: one pinned staging buffer, one host-to-device copy
     host = [i for i, f in enumerate(files) if not (isinstance(f, torch.Tensor) and f.is_cuda)]
     sizes = [f.numel() if isinstance(f, torch.Tensor) else memoryview(f).nbytes for f in files]
@@ -496,27 +477,212 @@ def png_decode(files, kind='color', reduce_zero_label=False, label_map=None, nam
     for i, f in enumerate(files):
         if data[i] is None:
             data[i] = f.to(dev).contiguous()
-    ch = 3 if kind == 'color' else 1
-    numel = [ch * h * w for h, w, _ in infos]
+    numel = [ch * info[0] * info[1] for info in infos]
     flat = torch.empty(sum(numel), dtype=torch.uint8, device=dev)
     outs, at = [], 0
-    for (h, w, _), m in zip(infos, numel):
-        outs.append(flat[at:at + m].view(ch, h, w))
+    for info, m in zip(infos, numel):
+        outs.append(flat[at:at + m].view(ch, info[0], info[1]))
         at += m
-    arr = (L.PngFile * n)()
-    for d, t, o, (h, w, ct), sz in zip(arr, data, outs, infos, sizes):
-        d.data, d.size, d.out, d.h, d.w, d.color_type = t.data_ptr(), sz, o.data_ptr(), h, w, ct
-    lib = L.get()
-    ws = torch.empty(max(1, L.check(lib.ledb200_png_decode_workspace_bytes(arr, n), 'ledb200_png_decode_workspace_bytes')),
-                     dtype=torch.uint8, device=dev)
-    status = torch.empty(n, dtype=torch.int32, device=dev)
-    lut = None
-    if kind == 'label':
-        lut = (C.c_uint8 * 256)(*label_lut(reduce_zero_label, label_map).tolist())
-    L.check(lib.ledb200_png_decode(arr, n, L.PNG_LABEL if kind == 'label' else L.PNG_COLOR, lut, _p(ws), _p(status),
-                                   L.stream_ptr(dev)), 'ledb200_png_decode')
-    st = status.cpu().tolist()
-    bad = [(names[i], L.PNG_STATUS.get(c, f'status {c}')) for i, c in enumerate(st) if c]
+    st = launch(data, sizes, outs, dev).cpu().tolist()
+    bad = [(names[i], status_names.get(c, f'status {c}')) for i, c in enumerate(st) if c]
     if bad:
-        raise L.LedB200Error('png_decode: ' + '; '.join(f'{nm}: {why}' for nm, why in bad))
+        raise L.LedB200Error(f'{who}: ' + '; '.join(f'{nm}: {why}' for nm, why in bad))
     return outs
+
+
+def _infos(files, names, parse):
+    """parse(f) for every file, its errors prefixed with the file's name"""
+    infos = []
+    for f, name in zip(files, names):
+        try:
+            infos.append(parse(f))
+        except NotImplementedError as e:
+            raise NotImplementedError(f'{name}: {e}') from None
+        except L.LedB200Error as e:
+            raise L.LedB200Error(f'{name}: {e}') from None
+    return infos
+
+
+def png_decode(files, kind='color', reduce_zero_label=False, label_map=None, names=None, device=None):
+    """PNG files -> CUDA uint8 tensors, decoded on the device (csrc/png_decode.cu).
+
+    files: bytes-like objects or 1-D uint8 tensors (host or device), bit depth 8, not interlaced.
+    kind='color': each result is [3, h, w] BGR, bit-identical to cv2.imdecode(buf, cv2.IMREAD_COLOR).transpose(2, 0, 1)
+      (what LoadImageFromFile gives): grey replicated, palettes expanded, alpha dropped, ancillary chunks ignored.
+    kind='label': grey or palette files; each result is [1, h, w], the stored values (palette indices, not colours: what
+      np.array(Image.open(f)) gives) through label_lut(reduce_zero_label, label_map), as LoadAnnotations gives them.
+    The host reads each IHDR (png_info), packs the host files into one pinned buffer and uploads it with one copy; one
+    decode call covers every file and one small copy brings the statuses back.  A file that fails raises LedB200Error
+    naming it (names[i], default 'file i') and the reason."""
+    if kind not in ('color', 'label'):
+        raise ValueError(f"kind must be 'color' or 'label', not {kind!r}")
+    files = list(files)
+    n = len(files)
+    if n == 0:
+        return []
+    names = list(names) if names is not None else [f'file {i}' for i in range(n)]
+    infos = _infos(files, names, lambda f: png_info(f, kind))
+
+    def launch(data, sizes, outs, dev):
+        arr = (L.PngFile * n)()
+        for d, t, o, (h, w, ct), sz in zip(arr, data, outs, infos, sizes):
+            d.data, d.size, d.out, d.h, d.w, d.color_type = t.data_ptr(), sz, o.data_ptr(), h, w, ct
+        lib = L.get()
+        ws = torch.empty(max(1, L.check(lib.ledb200_png_decode_workspace_bytes(arr, n),
+                                        'ledb200_png_decode_workspace_bytes')), dtype=torch.uint8, device=dev)
+        status = torch.empty(n, dtype=torch.int32, device=dev)
+        lut = None
+        if kind == 'label':
+            lut = (C.c_uint8 * 256)(*label_lut(reduce_zero_label, label_map).tolist())
+        L.check(lib.ledb200_png_decode(arr, n, L.PNG_LABEL if kind == 'label' else L.PNG_COLOR, lut, _p(ws),
+                                       _p(status), L.stream_ptr(dev)), 'ledb200_png_decode')
+        return status
+
+    return _decode_files(files, names, infos, 3 if kind == 'color' else 1, device, 'png_decode', launch, L.PNG_STATUS)
+
+
+JPEG_SOI = b'\xff\xd8'
+_JPEG_SOF_REFUSED = {0xC2: 'progressive', 0xC3: 'lossless', 0xC5: 'hierarchical', 0xC6: 'hierarchical progressive',
+                     0xC7: 'hierarchical lossless', 0xC9: 'arithmetic-coded', 0xCA: 'arithmetic-coded progressive',
+                     0xCB: 'arithmetic-coded lossless', 0xCD: 'hierarchical arithmetic-coded',
+                     0xCE: 'hierarchical arithmetic-coded progressive', 0xCF: 'hierarchical arithmetic-coded lossless'}
+
+
+def _exif_orientation(d):
+    """the orientation tag of an APP1 Exif payload (IFD0), 0 when there is none"""
+    if len(d) < 14 or d[:6] != b'Exif\x00\x00':
+        return 0
+    t = d[6:]
+    if t[:2] not in (b'II', b'MM'):
+        return 0
+    e = '<' if t[:2] == b'II' else '>'
+    if struct.unpack(e + 'H', t[2:4])[0] != 42:
+        return 0
+    ifd = struct.unpack(e + 'I', t[4:8])[0]
+    if ifd > len(t) - 2:
+        return 0
+    for i in range(struct.unpack(e + 'H', t[ifd:ifd + 2])[0]):
+        at = ifd + 2 + 12 * i
+        if at + 12 > len(t):
+            break
+        if struct.unpack(e + 'H', t[at:at + 2])[0] == 0x0112:
+            return struct.unpack(e + 'H', t[at + 8:at + 10])[0]
+    return 0
+
+
+def _jpeg_markers(b):
+    """(h, w, components) from a JPEG header prefix b; None when b ends before the first SOS"""
+    if len(b) < 2 or b[:2] != JPEG_SOI:
+        raise L.LedB200Error('not a JPEG file (no SOI marker)')
+    p, frame, jfif, adobe, transform, orient = 2, None, False, False, 0, 0
+    while True:
+        if p >= len(b):
+            return None
+        if b[p] != 0xFF:
+            raise L.LedB200Error(f'no marker at byte {p}')
+        while p < len(b) and b[p] == 0xFF:
+            p += 1
+        if p + 3 > len(b):
+            return None
+        m, n = b[p], (b[p + 1] << 8 | b[p + 2]) - 2
+        p += 3
+        if n < 0:
+            raise L.LedB200Error(f'marker 0x{m:02X}: segment length {n + 2}')
+        if p + n > len(b):
+            return None
+        s = b[p:p + n]
+        p += n
+        if m in _JPEG_SOF_REFUSED or m == 0xCC:
+            raise NotImplementedError(f'{_JPEG_SOF_REFUSED.get(m, "arithmetic-coded")} JPEG files (baseline only)')
+        if m in (0xC0, 0xC1):
+            if frame is not None:
+                raise L.LedB200Error('a second frame header')
+            if n < 6 or n != 6 + 3 * s[5]:
+                raise L.LedB200Error('frame header length')
+            prec, h, w, nf = s[0], s[1] << 8 | s[2], s[3] << 8 | s[4], s[5]
+            if prec != 8:
+                raise NotImplementedError(f'{prec}-bit JPEG files (8-bit only)')
+            if h == 0:
+                raise NotImplementedError('JPEG files whose height is given by a DNL marker')
+            if w == 0:
+                raise L.LedB200Error('frame width 0')
+            if nf not in (1, 3):
+                raise NotImplementedError(f'JPEG files of {nf} components (grey or YCbCr only)')
+            comps = [(s[6 + 3 * c], s[7 + 3 * c] >> 4, s[7 + 3 * c] & 15) for c in range(nf)]
+            if any(not (1 <= hs <= 4 and 1 <= vs <= 4) for _, hs, vs in comps):
+                raise L.LedB200Error('invalid sampling factors')
+            if nf == 3 and not (comps[0][1] <= 2 and comps[0][2] <= 2 and all(c[1:] == (1, 1) for c in comps[1:])):
+                raise NotImplementedError('sampling factors ' + ', '.join(f'{hs}x{vs}' for _, hs, vs in comps) +
+                                          ' (4:4:4, 4:2:2, 4:2:0 and 4:4:0 only)')
+            frame = (h, w, nf, [c[0] for c in comps])
+        elif m == 0xDA:
+            if frame is None:
+                raise L.LedB200Error('SOS before the frame header')
+            h, w, nf, ids = frame
+            if n < 1 or s[0] != nf:
+                raise NotImplementedError('non-interleaved (multi-scan) JPEG files')
+            if [s[1 + 2 * c] for c in range(nf)] != ids:
+                raise NotImplementedError('a scan whose components are not in frame order')
+            if nf == 3 and (False if jfif else transform == 0 if adobe else ids == [82, 71, 66]):
+                raise NotImplementedError('RGB JPEG files (YCbCr or grey only)')
+            if 2 <= orient <= 8:
+                raise NotImplementedError(f'Exif orientation {orient} (cv2.imdecode would rotate the image)')
+            if h * w > MAX_PNG_PIXELS:
+                raise L.LedB200Error(f'{w} x {h} is more than {MAX_PNG_PIXELS} pixels')
+            return h, w, nf
+        elif m == 0xE0:
+            jfif |= n >= 14 and s[:5] == b'JFIF\x00'
+        elif m == 0xE1:
+            orient = orient or _exif_orientation(s)
+        elif m == 0xEE and n >= 12 and s[:5] == b'Adobe':
+            adobe, transform = True, s[11]
+        elif m == 0xDC:
+            raise NotImplementedError('JPEG files whose height is given by a DNL marker')
+        elif not (m in (0xC4, 0xDB, 0xDD, 0xFE) or 0xE0 <= m <= 0xEF):
+            raise L.LedB200Error(f'unexpected marker 0x{m:02X} before the scan')
+
+
+def jpeg_info(f):
+    """(h, w, components) of a JPEG file (bytes-like or 1-D uint8 tensor), from its markers up to the first SOS (a device
+    tensor costs small copies of the header prefix).  A malformed header raises LedB200Error; a valid JPEG outside what
+    jpeg_decode supports raises NotImplementedError: progressive, lossless, hierarchical or arithmetic-coded files,
+    precision other than 8 bits, 2 or 4 components, RGB colour space, sampling other than 4:4:4 / 4:2:2 / 4:2:0 /
+    4:4:0, non-interleaved scans, a DNL height and an Exif orientation other than 1."""
+    size = f.numel() if isinstance(f, torch.Tensor) else memoryview(f).nbytes
+    n = 1 << 16
+    while True:
+        info = _jpeg_markers(_head(f, n))
+        if info is not None:
+            return info
+        if n >= size:
+            raise L.LedB200Error('the file ends before the first SOS')
+        n *= 4
+
+
+def jpeg_decode(files, names=None, device=None):
+    """Baseline JPEG files -> CUDA [3, h, w] uint8 BGR tensors decoded on the device (csrc/jpeg_decode.cu),
+    bit-identical to cv2.imdecode(buf, cv2.IMREAD_COLOR).transpose(2, 0, 1) (what LoadImageFromFile gives).
+
+    files: bytes-like objects or 1-D uint8 tensors (host or device).  The host walks each file's markers (jpeg_info),
+    packs the host files into one pinned buffer and uploads it with one copy; one decode call covers every file and
+    one small copy brings the statuses back.  A file that fails raises LedB200Error naming it (names[i], default
+    'file i') and the reason: corrupt entropy-coded data is an error, where libjpeg would warn and fill with grey."""
+    files = list(files)
+    n = len(files)
+    if n == 0:
+        return []
+    names = list(names) if names is not None else [f'file {i}' for i in range(n)]
+    infos = _infos(files, names, jpeg_info)
+
+    def launch(data, sizes, outs, dev):
+        arr = (L.JpegFile * n)()
+        for d, t, o, (h, w, nc), sz in zip(arr, data, outs, infos, sizes):
+            d.data, d.size, d.out, d.h, d.w, d.components = t.data_ptr(), sz, o.data_ptr(), h, w, nc
+        lib = L.get()
+        ws = torch.empty(L.check(lib.ledb200_jpeg_decode_workspace_bytes(arr, n), 'ledb200_jpeg_decode_workspace_bytes'),
+                         dtype=torch.uint8, device=dev)
+        status = torch.empty(n, dtype=torch.int32, device=dev)
+        L.check(lib.ledb200_jpeg_decode(arr, n, _p(ws), _p(status), L.stream_ptr(dev)), 'ledb200_jpeg_decode')
+        return status
+
+    return _decode_files(files, names, infos, 3, device, 'jpeg_decode', launch, L.JPEG_STATUS)
