@@ -528,11 +528,19 @@ int ledb200_view_resize(const ledb200_view_desc* views, int32_t n, int32_t Hp, i
  * ledb200_png_workspace_bytes: device workspace of ledb200_png_encode for N maps of H x W.
  * ledb200_png_encode: labels [N,H,W] contiguous, dtype LEDB200_U8 | LEDB200_I64, add 0 | 1.  out (capacity N * bound)
  *   receives the files back to back, file i at out[offsets[i] : offsets[i + 1]]; offsets: device int64 [N + 1].  The
- *   host reads offsets, then offsets[N] bytes of out. */
+ *   host reads offsets, then offsets[N] bytes of out.
+ * ledb200_png_encode_lut: the same with pixels lut[label & 255] (lut: HOST 256 bytes; ledb200_png_encode is the table
+ *   (i + add) & 255).  palette 1 writes colour type 3 and, before the IDAT, the 256-entry grey PLTE (entry i = (i, i, i))
+ *   that PIL's Image.convert('P') gives a grayscale image (CityscapesMetric's labelId files); out then holds
+ *   N * ledb200_png_lut_bound(H, W, 1) bytes.
+ * ledb200_png_lut_bound: ledb200_png_bound plus the PLTE chunk when palette is 1. */
 int64_t ledb200_png_bound(int32_t H, int32_t W);
+int64_t ledb200_png_lut_bound(int32_t H, int32_t W, int32_t palette);
 int64_t ledb200_png_workspace_bytes(int32_t N, int32_t H, int32_t W);
 int ledb200_png_encode(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, int32_t add, uint8_t* out,
                        int64_t* offsets, void* workspace, void* stream);
+int ledb200_png_encode_lut(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, const uint8_t* lut,
+                           int32_t palette, uint8_t* out, int64_t* offsets, void* workspace, void* stream);
 
 /* ---- PNG files -> decoded images and label maps (csrc/png_decode.cu) -----------------------------------------------------
  * The dataset feed of LoadImageFromFile (mmcv imfrombytes, cv2 backend, flag 'color') and LoadAnnotations (pillow backend,
@@ -542,15 +550,18 @@ int ledb200_png_encode(const void* labels, int32_t dtype, int32_t N, int32_t H, 
  *     replicated, palette expanded through PLTE, alpha dropped, tRNS / gAMA / other ancillary chunks ignored).
  *   LEDB200_PNG_LABEL: colour types 0 and 3 only; out [1,h,w] uint8 = lut[grey value or palette index] (lut: HOST 256
  *     bytes, NULL = identity), i.e. np.array(Image.open(f)) through the table.
+ *   LEDB200_PNG_GREY16: bit depth 16, colour type 0 only (Cityscapes' *_gtFine_instanceIds.png); out [1,h,w] int32 =
+ *     np.array(Image.open(f)), the big-endian 16-bit samples; lut is ignored.  The other modes read bit depth 8.
  * One descriptor per file (HOST array): data / size = the whole file (device), out = its output (device), h / w /
  * color_type as the IHDR states them (the device checks that they do).  status: device int32 [n], one LEDB200_PNG_*
  * code per file; a file with a non-zero status leaves its output undefined.  Every file is decoded at once (one warp
  * inflates each file; a block per file undoes the filters).  No file makes the kernels read outside it or write
  * outside its output and its workspace slot, whatever its content.
- * ledb200_png_decode_workspace_bytes: device workspace of one ledb200_png_decode call over these descriptors.
+ * ledb200_png_decode_workspace_bytes: device workspace of one ledb200_png_decode call over these descriptors in the
+ *   colour or label mode; ledb200_png_decode_mode_workspace_bytes: the same for any mode.
  * ledb200_png_decode_host: the same decoder on the CPU (diagnostics, like ledb200_debug_fetch): every pointer of the
  *   descriptors, status and lut are HOST memory; the statuses equal the device's. */
-enum { LEDB200_PNG_COLOR = 0, LEDB200_PNG_LABEL = 1 };
+enum { LEDB200_PNG_COLOR = 0, LEDB200_PNG_LABEL = 1, LEDB200_PNG_GREY16 = 16 };
 enum {
   LEDB200_PNG_OK = 0,
   LEDB200_PNG_EHEADER = 1,      /* signature or IHDR differs from the descriptor                                 */
@@ -575,9 +586,29 @@ typedef struct {
   int32_t h, w, color_type;
 } ledb200_png_file;
 int64_t ledb200_png_decode_workspace_bytes(const ledb200_png_file* files, int32_t n);
+int64_t ledb200_png_decode_mode_workspace_bytes(const ledb200_png_file* files, int32_t n, int32_t mode);
 int ledb200_png_decode(const ledb200_png_file* files, int32_t n, int32_t mode, const uint8_t* lut, void* workspace,
                        int32_t* status, void* stream);
 int ledb200_png_decode_host(const ledb200_png_file* files, int32_t n, int32_t mode, const uint8_t* lut, int32_t* status);
+
+/* ---- Cityscapes pixel-level statistics (csrc/cityscapes.cu) --------------------------------------------------------------
+ * CityscapesMetric's evaluation (cityscapesscripts evalPixelLevelSemanticLabeling.evaluatePair, evalInstLevelScore) for N
+ * same-shape images: pred [N,H,W] trainIds (LEDB200_U8 | LEDB200_I64), gt [N,H,W] uint8 labelIds, inst [N,H,W] int32
+ * instanceIds, all device and contiguous.  Tables (HOST): train_to_id[256] maps a trainId to its labelId; category[34]
+ * is each labelId's instance category (-1: none); inst_rule[34] says what an instance id id > 1000 of class id / 1000
+ * does: 0 error, 1 skipped (ignoreInEval), 2 counted (only ids 24 .. 33 of a category).
+ * cm_inout: device int64 [34,34] (rows GT, columns prediction), accumulated; cm_last_out (device int64 [34,34] or NULL)
+ * receives the matrix of image N - 1 alone.  out: device int32 of ledb200_cityscapes_out_ints(N): statuses [N] (bits:
+ * 1 a GT labelId above 33, 2 a predicted labelId outside 0 .. 33, 4 an instance id of a class neither counted nor
+ * skipped or above 33, 8 an int64 prediction outside 0 .. 255), record counts [N], then the records (instId, size, tp,
+ * catTp) of every counted instance, image after image, in ascending instId.  workspace: device,
+ * ledb200_cityscapes_workspace_bytes(N).  Every count is an exact integer. */
+int64_t ledb200_cityscapes_out_ints(int32_t N);
+int64_t ledb200_cityscapes_workspace_bytes(int32_t N);
+int ledb200_cityscapes_accumulate(const void* pred, int32_t pred_dtype, const uint8_t* gt, const int32_t* inst,
+                                  int32_t N, int32_t H, int32_t W, const int32_t* train_to_id, const int8_t* category,
+                                  const int8_t* inst_rule, int64_t* cm_inout, int64_t* cm_last_out, int32_t* out,
+                                  void* workspace, void* stream);
 
 /* ---- baseline JPEG files -> decoded images (csrc/jpeg_decode.cu) ---------------------------------------------------------
  * LoadImageFromFile (mmcv imfrombytes, cv2 backend, flag 'color') on the device for JPEG files: out [3,h,w] uint8 BGR,

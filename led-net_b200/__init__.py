@@ -1,6 +1,6 @@
 """led-net_b200: the LED-Net data-parallel hot path as hand-written sm_100a CUDA kernels behind
 the reference's mmseg registry surface (MODELS: LEDNet, LEDHead, OhemCrossEntropy, EncoderDecoder,
-SegDataPreProcessor, DeviceAugSegDataPreProcessor, SegTTAModel; METRICS: IoUMetric; TRANSFORMS: PackSegFiles, PackSegPNGFiles).  Host code is Python/PyTorch plumbing over the C ABI in
+SegDataPreProcessor, DeviceAugSegDataPreProcessor, SegTTAModel; METRICS: IoUMetric, CityscapesMetric; TRANSFORMS: PackSegFiles, PackSegPNGFiles).  Host code is Python/PyTorch plumbing over the C ABI in
 include/ledb200.h; there is no CPU fallback."""
 __version__ = '0.1.0'
 
@@ -9,6 +9,7 @@ from .lib import LedB200Error  # noqa: F401
 from .losses import OhemCrossEntropy, accuracy  # noqa: F401
 from .modules import LEDNet, LEDHead  # noqa: F401
 from .metrics import IoUMetric  # noqa: F401
+from .cityscapes import CityscapesMetric  # noqa: F401
 from .segmentor import EncoderDecoder, SegDataPreProcessor  # noqa: F401
 from .tta import SegTTAModel  # noqa: F401
 from .augment import DeviceAugSegDataPreProcessor  # noqa: F401

@@ -1,8 +1,10 @@
 // Label maps -> PNG files on the device (IoUMetric's output_dir / format_only, mmseg's `tools/test.py --out`).
 //
-// Every image becomes an 8-bit grayscale PNG (IHDR colour type 0, no interlace) whose pixels are (label + add) mod 256,
-// what `Image.fromarray((pred + reduce_zero_label).astype(np.uint8))` saves.  The file is the signature, IHDR, one IDAT
-// holding one zlib stream (header 78 01, deflate, big-endian Adler-32) and IEND.  Every scanline has filter type 0.
+// Every image becomes an 8-bit PNG (no interlace) whose pixels are lut[label & 255]: (label + add) mod 256 for
+// IoUMetric, what `Image.fromarray((pred + reduce_zero_label).astype(np.uint8))` saves, or CityscapesMetric's trainId ->
+// labelId table.  The file is the signature, IHDR, one IDAT holding one zlib stream (header 78 01, deflate, big-endian
+// Adler-32) and IEND: grayscale (colour type 0), or with `palette` colour type 3 and, before the IDAT, the 256-entry grey
+// PLTE that PIL's `.convert('P')` writes for a grayscale image.  Every scanline has filter type 0.
 //
 //  * png_filter_kernel   : the filtered scanline stream (a 0 filter byte, then W pixels, per row) into the workspace.
 //  * png_band_kernel     : one warp per band of R rows (R * (W + 1) <= 65535 bytes where a row allows it).  The band is
@@ -33,7 +35,10 @@ constexpr int64_t kStoredMax = 65535;
 // file bytes outside the zlib data: signature 8, IHDR 25, IDAT length + type 8, zlib header 2, Adler-32 4, IDAT CRC 4,
 // IEND 12
 constexpr int64_t kFileOverhead = 8 + 25 + 8 + 2 + 4 + 4 + 12;
-constexpr int64_t kIdatData = 8 + 25 + 8;    // offset of the zlib header within the file
+constexpr int64_t kIdatData = 8 + 25 + 8;    // offset of the zlib header within the file (no palette)
+constexpr int64_t kPlteChunk = 12 + 768;     // the grey PLTE chunk of a palette file, between IHDR and IDAT
+
+struct Lut { uint8_t v[256]; };
 
 struct Plan {
   int64_t S, n, R, nb, band_cap;              // row bytes, stream bytes, rows per band, bands, slot bytes per band
@@ -67,13 +72,16 @@ int64_t bound_of(const Plan& p) {
 
 // ---- filtered scanlines --------------------------------------------------------------------------------------------
 template <typename T>
-__global__ void __launch_bounds__(256) png_filter_kernel(const T* __restrict__ labels, int W, int64_t S, int add,
-                                                        uint8_t* __restrict__ raw) {
+__global__ void __launch_bounds__(256) png_filter_kernel(const T* __restrict__ labels, int W, int64_t S,
+                                                        const __grid_constant__ Lut lut, uint8_t* __restrict__ raw) {
+  __shared__ uint8_t tab[256];
+  tab[threadIdx.x] = lut.v[threadIdx.x];
+  __syncthreads();
   const int64_t row = blockIdx.x;
   const T* src = labels + row * W;
   uint8_t* dst = raw + row * S;
   for (int c = threadIdx.x; c <= W; c += blockDim.x)
-    dst[c] = c == 0 ? (uint8_t)0 : (uint8_t)((int64_t)src[c - 1] + add);
+    dst[c] = c == 0 ? (uint8_t)0 : tab[(uint8_t)src[c - 1]];
 }
 
 // ---- deflate symbols -------------------------------------------------------------------------------------------------
@@ -429,8 +437,8 @@ __global__ void __launch_bounds__(32) png_band_kernel(const uint8_t* __restrict_
 }
 
 // Per image: band offsets within the zlib data (info[.][3]), the file size into sizes[img + 1], the Adler-32.
-__global__ void __launch_bounds__(32) png_size_kernel(Plan p, int64_t* __restrict__ info, int64_t* __restrict__ sizes,
-                                                      uint32_t* __restrict__ adler) {
+__global__ void __launch_bounds__(32) png_size_kernel(Plan p, int64_t extra, int64_t* __restrict__ info,
+                                                      int64_t* __restrict__ sizes, uint32_t* __restrict__ adler) {
   const int lane = threadIdx.x;
   const int64_t img = blockIdx.x;
   int64_t* inf = info + img * p.nb * 4;
@@ -462,7 +470,7 @@ __global__ void __launch_bounds__(32) png_size_kernel(Plan p, int64_t* __restric
   if (lane == 0) {
     const uint64_t s1 = (1 + A) % kAdlerMod, s2 = ((uint64_t)p.n % kAdlerMod + B) % kAdlerMod;
     adler[img] = (uint32_t)(s2 << 16 | s1);
-    sizes[img + 1] = carry - 2 + kFileOverhead;
+    sizes[img + 1] = carry - 2 + kFileOverhead + extra;
   }
 }
 
@@ -503,7 +511,9 @@ __device__ __forceinline__ void put_be32(uint8_t* p, uint32_t v) {
   p[0] = (uint8_t)(v >> 24); p[1] = (uint8_t)(v >> 16); p[2] = (uint8_t)(v >> 8); p[3] = (uint8_t)v;
 }
 
-__global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W, const uint8_t* __restrict__ slots,
+// palette_crc: the CRC-32 of the grey PLTE chunk (type and data), 0 for a grayscale file
+__global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W, uint32_t palette_crc,
+                                                           const uint8_t* __restrict__ slots,
                                                            const int64_t* __restrict__ info,
                                                            const uint32_t* __restrict__ adler,
                                                            const int64_t* __restrict__ offsets, uint8_t* __restrict__ out) {
@@ -511,27 +521,40 @@ __global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W,
   __shared__ int64_t len_s[256];
   const int t = threadIdx.x;
   const int64_t img = blockIdx.x;
+  const int64_t pre = palette_crc ? kPlteChunk : 0;        // bytes before the IDAT chunk move by the PLTE chunk
   uint8_t* f = out + offsets[img];
   const int64_t size = offsets[img + 1] - offsets[img];
-  const int64_t idat_len = size - kFileOverhead + 2 + 4;   // zlib header + deflate data + Adler-32
+  const int64_t idat_len = size - pre - kFileOverhead + 2 + 4;   // zlib header + deflate data + Adler-32
   tab[t] = crc_table_entry((uint32_t)t);
+  if (pre) {
+    uint8_t* c = f + 33;
+    if (t == 0) {
+      put_be32(c, 768);
+      c[4] = 'P'; c[5] = 'L'; c[6] = 'T'; c[7] = 'E';
+      put_be32(c + 8 + 768, palette_crc);
+    }
+    for (int k = 0; k < 3; ++k) c[8 + 3 * t + k] = (uint8_t)t;
+  }
+  f += pre;                                                // from here on f is the file shifted by the PLTE chunk
   __syncthreads();
   if (t == 0) {
     crc_x2n_table(x2n);
+    uint8_t* f0 = f - pre;
     const uint8_t sig[8] = {0x89, 'P', 'N', 'G', 0x0d, 0x0a, 0x1a, 0x0a};
-    for (int k = 0; k < 8; ++k) f[k] = sig[k];
-    uint8_t* h = f + 8;
+    for (int k = 0; k < 8; ++k) f0[k] = sig[k];
+    uint8_t* h = f0 + 8;
     put_be32(h, 13);
     h[4] = 'I'; h[5] = 'H'; h[6] = 'D'; h[7] = 'R';
     put_be32(h + 8, (uint32_t)W); put_be32(h + 12, (uint32_t)H);
-    h[16] = 8; h[17] = 0; h[18] = 0; h[19] = 0; h[20] = 0;   // bit depth 8, grayscale, deflate, filter 0, no interlace
+    // bit depth 8, grayscale (0) or palette (3), deflate, filter 0, no interlace
+    h[16] = 8; h[17] = pre ? 3 : 0; h[18] = 0; h[19] = 0; h[20] = 0;
     put_be32(h + 21, ~crc_update(tab, 0xffffffffu, h + 4, 17));
     uint8_t* d = f + 33;
     put_be32(d, (uint32_t)idat_len);
     d[4] = 'I'; d[5] = 'D'; d[6] = 'A'; d[7] = 'T';
     d[8] = 0x78; d[9] = 0x01;
     put_be32(f + kIdatData + idat_len - 4, adler[img]);
-    uint8_t* e = f + size - 12;
+    uint8_t* e = f + size - pre - 12;
     put_be32(e, 0);
     e[4] = 'I'; e[5] = 'E'; e[6] = 'N'; e[7] = 'D';
     put_be32(e + 8, 0xae426082u);
@@ -574,38 +597,62 @@ int64_t ledb200_png_bound(int32_t H, int32_t W) {
   return b;
 }
 
+int64_t ledb200_png_lut_bound(int32_t H, int32_t W, int32_t palette) {
+  if (palette != 0 && palette != 1) return fail(LEDB200_EINVAL, "png_lut_bound: palette must be 0 or 1");
+  const int64_t b = ledb200_png_bound(H, W);
+  return b < 0 ? b : b + (palette ? kPlteChunk : 0);
+}
+
 int64_t ledb200_png_workspace_bytes(int32_t N, int32_t H, int32_t W) {
   if (N < 1 || H < 1 || W < 1) return fail(LEDB200_EINVAL, "png_workspace_bytes: N, H and W must be at least 1");
   return make_plan(N, H, W).total;
 }
 
-int ledb200_png_encode(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, int32_t add, uint8_t* out,
-                       int64_t* offsets, void* workspace, void* stream) {
+int ledb200_png_encode_lut(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, const uint8_t* lut,
+                           int32_t palette, uint8_t* out, int64_t* offsets, void* workspace, void* stream) {
   if (N < 1 || H < 1 || W < 1) return fail(LEDB200_EINVAL, "png_encode: N, H and W must be at least 1");
   if (dtype != LEDB200_U8 && dtype != LEDB200_I64) return fail(LEDB200_EINVAL, "png_encode: labels must be U8 or I64");
-  if (add != 0 && add != 1) return fail(LEDB200_EINVAL, "png_encode: add must be 0 or 1");
-  if (!labels || !out || !offsets || !workspace) return fail(LEDB200_EINVAL, "png_encode: null buffer");
+  if (palette != 0 && palette != 1) return fail(LEDB200_EINVAL, "png_encode: palette must be 0 or 1");
+  if (!labels || !lut || !out || !offsets || !workspace) return fail(LEDB200_EINVAL, "png_encode: null buffer");
   if (ledb200_png_bound(H, W) < 0) return LEDB200_EINVAL;
   const Plan p = make_plan(N, H, W);
   if ((int64_t)N * p.nb > INT32_MAX) return fail(LEDB200_EINVAL, "png_encode: too many bands in one call");
+  // the grey palette's CRC is the same for every file: computed here once
+  static const uint32_t palette_crc = [] {
+    uint32_t tab[256];
+    for (uint32_t i = 0; i < 256; ++i) tab[i] = crc_table_entry(i);
+    uint8_t chunk[4 + 768] = {'P', 'L', 'T', 'E'};
+    for (int i = 0; i < 768; ++i) chunk[4 + i] = (uint8_t)(i / 3);
+    return ~crc_update(tab, 0xffffffffu, chunk, sizeof chunk);
+  }();
+  Lut tab;
+  for (int i = 0; i < 256; ++i) tab.v[i] = lut[i];
   cudaStream_t st = (cudaStream_t)stream;
   uint8_t* ws = (uint8_t*)workspace;
   uint8_t* slots = ws + p.slot_off;
   int64_t* info = (int64_t*)(ws + p.info_off);
   uint32_t* adler = (uint32_t*)(ws + p.adler_off);
   const unsigned rows = (unsigned)((int64_t)N * H);
-  if (dtype == LEDB200_I64) png_filter_kernel<int64_t><<<rows, 256, 0, st>>>((const int64_t*)labels, W, p.S, add, ws);
-  else png_filter_kernel<uint8_t><<<rows, 256, 0, st>>>((const uint8_t*)labels, W, p.S, add, ws);
+  if (dtype == LEDB200_I64) png_filter_kernel<int64_t><<<rows, 256, 0, st>>>((const int64_t*)labels, W, p.S, tab, ws);
+  else png_filter_kernel<uint8_t><<<rows, 256, 0, st>>>((const uint8_t*)labels, W, p.S, tab, ws);
   LEDB_LAUNCH_OK("png_filter_kernel");
   png_band_kernel<<<(unsigned)(N * p.nb), 32, 0, st>>>(ws, p, slots, info, (uint32_t*)(ws + p.bm_off));
   LEDB_LAUNCH_OK("png_band_kernel");
-  png_size_kernel<<<(unsigned)N, 32, 0, st>>>(p, info, offsets, adler);
+  png_size_kernel<<<(unsigned)N, 32, 0, st>>>(p, palette ? kPlteChunk : 0, info, offsets, adler);
   LEDB_LAUNCH_OK("png_size_kernel");
   png_scan_kernel<<<1, 1024, 0, st>>>(offsets, N);
   LEDB_LAUNCH_OK("png_scan_kernel");
-  png_assemble_kernel<<<(unsigned)N, 256, 0, st>>>(p, H, W, slots, info, adler, offsets, out);
+  png_assemble_kernel<<<(unsigned)N, 256, 0, st>>>(p, H, W, palette ? palette_crc : 0u, slots, info, adler, offsets, out);
   LEDB_LAUNCH_OK("png_assemble_kernel");
   return LEDB200_OK;
+}
+
+int ledb200_png_encode(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, int32_t add, uint8_t* out,
+                       int64_t* offsets, void* workspace, void* stream) {
+  if (add != 0 && add != 1) return fail(LEDB200_EINVAL, "png_encode: add must be 0 or 1");
+  uint8_t lut[256];
+  for (int i = 0; i < 256; ++i) lut[i] = (uint8_t)(i + add);
+  return ledb200_png_encode_lut(labels, dtype, N, H, W, lut, 0, out, offsets, workspace, stream);
 }
 
 }  // extern "C"

@@ -1,10 +1,12 @@
 // PNG files -> decoded images and label maps on the device (the dataset feed: LoadImageFromFile / LoadAnnotations).
 //
-// Supported: bit depth 8, colour types 0 / 2 / 3 / 4 / 6, no interlace (the caller read the IHDR and rejected the rest).
+// Supported: bit depth 8, colour types 0 / 2 / 3 / 4 / 6, and bit depth 16 grey in the grey16 mode; no interlace (the
+// caller read the IHDR and rejected the rest).
 // Colour mode writes [3, h, w] uint8 BGR, what cv2.imdecode(buf, IMREAD_COLOR) returns transposed to CHW: grey
 // replicated, palette expanded through PLTE (indices past its end read black, as libpng's zero-filled palette does),
 // alpha dropped, tRNS / gAMA and every other ancillary chunk ignored.  Label mode (colour types 0 and 3) writes [1, h, w]
-// uint8: the grey value or the palette index through a 256-entry lookup table.
+// uint8: the grey value or the palette index through a 256-entry lookup table.  Grey16 mode (bit depth 16, colour type 0
+// only: Cityscapes' instanceIds maps) writes [1, h, w] int32, the big-endian samples as np.array(Image.open(f)) reads them.
 //
 //  * png_inflate_kernel  : one warp per file.  Lane 0 walks the chunks (order and lengths; ChunkWalk), the warp checks
 //      the CRC of every critical chunk (per-lane CRCs merged with crc_combine) and gathers the IDAT payloads into one
@@ -42,17 +44,20 @@ constexpr int kUnfilterThreads = 256;
 HD uint32_t be32(const uint8_t* p) {
   return (uint32_t)p[0] << 24 | (uint32_t)p[1] << 16 | (uint32_t)p[2] << 8 | (uint32_t)p[3];
 }
-HD int bytes_per_pixel(int ct) { return ct == 2 ? 3 : ct == 4 ? 2 : ct == 6 ? 4 : 1; }
+HD int bytes_per_pixel(int ct, int mode) {
+  return mode == LEDB200_PNG_GREY16 ? 2 : ct == 2 ? 3 : ct == 4 ? 2 : ct == 6 ? 4 : 1;
+}
+HD int bit_depth(int mode) { return mode == LEDB200_PNG_GREY16 ? 16 : 8; }
 
 // ---- signature and IHDR against the descriptor ----------------------------------------------------------------------
-HD int check_header(const uint8_t* f, int64_t size, int h, int w, int ct) {
+HD int check_header(const uint8_t* f, int64_t size, int h, int w, int ct, int depth) {
   const uint8_t sig[8] = {0x89, 'P', 'N', 'G', 0x0d, 0x0a, 0x1a, 0x0a};
   if (size < 33) return LEDB200_PNG_EHEADER;
   for (int k = 0; k < 8; ++k)
     if (f[k] != sig[k]) return LEDB200_PNG_EHEADER;
   const uint8_t* c = f + 8;
   if (be32(c) != 13 || be32(c + 4) != 0x49484452u) return LEDB200_PNG_EHEADER;   // "IHDR"
-  if (be32(c + 8) != (uint32_t)w || be32(c + 12) != (uint32_t)h || c[16] != 8 || c[17] != (uint8_t)ct || c[18] || c[19] ||
+  if (be32(c + 8) != (uint32_t)w || be32(c + 12) != (uint32_t)h || c[16] != depth || c[17] != (uint8_t)ct || c[18] || c[19] ||
       c[20])
     return LEDB200_PNG_EHEADER;
   return LEDB200_PNG_OK;
@@ -366,9 +371,15 @@ HD void unfilter_span(uint8_t* cur, const uint8_t* prev, int ft, int bpp, int64_
   }
 }
 
-// pixels [x0, x1) of reconstructed row y into the output: colour [3, h, w] BGR, label [1, h, w] through lut
+// pixels [x0, x1) of reconstructed row y into the output: colour [3, h, w] BGR, label [1, h, w] through lut, grey16
+// [1, h, w] int32
 HD void emit_pixels(const uint8_t* d, int ct, int mode, const uint8_t* plte, const uint8_t* lut, uint8_t* out,
                     int64_t plane, int64_t y, int64_t w, int64_t x0, int64_t x1) {
+  if (mode == LEDB200_PNG_GREY16) {
+    int32_t* o = reinterpret_cast<int32_t*>(out) + y * w;
+    for (int64_t x = x0; x < x1; ++x) o[x] = (int32_t)d[2 * x] << 8 | d[2 * x + 1];
+    return;
+  }
   uint8_t* o = out + y * w;
   for (int64_t x = x0; x < x1; ++x) {
     if (mode == LEDB200_PNG_LABEL) { o[x] = lut[d[x]]; continue; }
@@ -455,7 +466,7 @@ __global__ void __launch_bounds__(32) png_inflate_kernel(const __grid_constant__
   for (int i = lane; i < 768; i += 32) f.plte[i] = 0;
   if (lane == 0) crc_x2n_table(x2n);
   __syncwarp();
-  int st = lane == 0 ? check_header(f.data, f.size, f.h, f.w, f.ct) : 0;
+  int st = lane == 0 ? check_header(f.data, f.size, f.h, f.w, f.ct, bit_depth(a.mode)) : 0;
   st = __shfl_sync(0xffffffffu, st, 0);
 
   // chunks: lane 0 walks, the warp checks CRCs and gathers the IDAT payloads
@@ -557,7 +568,8 @@ int check_files(const ledb200_png_file* files, int n, int mode, const char* who)
   const std::string w(who);
   if (!files) return fail(LEDB200_EINVAL, w + ": null file descriptors");
   if (n < 1) return fail(LEDB200_EINVAL, w + ": at least one file");
-  if (mode != LEDB200_PNG_COLOR && mode != LEDB200_PNG_LABEL) return fail(LEDB200_EINVAL, w + ": mode must be colour or label");
+  if (mode != LEDB200_PNG_COLOR && mode != LEDB200_PNG_LABEL && mode != LEDB200_PNG_GREY16)
+    return fail(LEDB200_EINVAL, w + ": mode must be colour, label or grey16");
   for (int i = 0; i < n; ++i) {
     const ledb200_png_file& d = files[i];
     const std::string at = w + ": file " + std::to_string(i) + ": ";
@@ -569,14 +581,15 @@ int check_files(const ledb200_png_file* files, int n, int mode, const char* who)
       return fail(LEDB200_EINVAL, at + "colour type must be 0, 2, 3, 4 or 6");
     if (mode == LEDB200_PNG_LABEL && d.color_type != 0 && d.color_type != 3)
       return fail(LEDB200_EINVAL, at + "label maps must be grey or palette images");
+    if (mode == LEDB200_PNG_GREY16 && d.color_type != 0) return fail(LEDB200_EINVAL, at + "grey16 files must be grey images");
   }
   return LEDB200_OK;
 }
 
-Slot slot_of(const ledb200_png_file& d, int64_t& at) {
+Slot slot_of(const ledb200_png_file& d, int mode, int64_t& at) {
   Slot s;
   s.zbuf = at; at += align16(d.size);
-  s.raw = at; at += align16((int64_t)d.h * (1 + (int64_t)d.w * bytes_per_pixel(d.color_type)));
+  s.raw = at; at += align16((int64_t)d.h * (1 + (int64_t)d.w * bytes_per_pixel(d.color_type, mode)));
   s.plte = at; at += 768;
   return s;
 }
@@ -587,7 +600,7 @@ int decode_host(DecFile f, int mode, const uint8_t* lut) {
   for (uint32_t i = 0; i < 256; ++i) tab[i] = crc_table_entry(i);
   crc_x2n_table(x2n.data());
   std::memset(f.plte, 0, 768);
-  int st = check_header(f.data, f.size, f.h, f.w, f.ct);
+  int st = check_header(f.data, f.size, f.h, f.w, f.ct, bit_depth(mode));
   ChunkWalk w;
   int64_t zlen = 0;
   while (st == LEDB200_PNG_OK) {
@@ -643,11 +656,15 @@ using namespace ledb;
 
 extern "C" {
 
-int64_t ledb200_png_decode_workspace_bytes(const ledb200_png_file* files, int32_t n) {
+int64_t ledb200_png_decode_mode_workspace_bytes(const ledb200_png_file* files, int32_t n, int32_t mode) {
   if (!files || n < 1) return fail(LEDB200_EINVAL, "png_decode_workspace_bytes: need at least one file descriptor");
   int64_t at = 0;
-  for (int i = 0; i < n; ++i) slot_of(files[i], at);
+  for (int i = 0; i < n; ++i) slot_of(files[i], mode, at);
   return at;
+}
+
+int64_t ledb200_png_decode_workspace_bytes(const ledb200_png_file* files, int32_t n) {
+  return ledb200_png_decode_mode_workspace_bytes(files, n, LEDB200_PNG_COLOR);
 }
 
 int ledb200_png_decode(const ledb200_png_file* files, int32_t n, int32_t mode, const uint8_t* lut, void* workspace,
@@ -665,11 +682,11 @@ int ledb200_png_decode(const ledb200_png_file* files, int32_t n, int32_t mode, c
     for (int k = 0; k < 256; ++k) a.lut[k] = lut ? lut[k] : (uint8_t)k;
     for (int i = 0; i < a.n; ++i) {
       const ledb200_png_file& d = files[i0 + i];
-      const Slot s = slot_of(d, at);
+      const Slot s = slot_of(d, mode, at);
       DecFile& f = a.f[i];
       f.data = d.data; f.size = d.size; f.out = d.out;
       f.zbuf = ws + s.zbuf; f.raw = ws + s.raw; f.plte = ws + s.plte;
-      f.h = d.h; f.w = d.w; f.ct = d.color_type; f.bpp = bytes_per_pixel(d.color_type);
+      f.h = d.h; f.w = d.w; f.ct = d.color_type; f.bpp = bytes_per_pixel(d.color_type, mode);
     }
     png_inflate_kernel<<<a.n, 32, 0, st>>>(a);
     LEDB_LAUNCH_OK("png_inflate_kernel");
@@ -687,12 +704,12 @@ int ledb200_png_decode_host(const ledb200_png_file* files, int32_t n, int32_t mo
   for (int i = 0; i < n; ++i) {
     const ledb200_png_file& d = files[i];
     int64_t at = 0;
-    const Slot s = slot_of(d, at);
+    const Slot s = slot_of(d, mode, at);
     std::vector<uint8_t> ws((size_t)at);
     DecFile f;
     f.data = d.data; f.size = d.size; f.out = d.out;
     f.zbuf = ws.data() + s.zbuf; f.raw = ws.data() + s.raw; f.plte = ws.data() + s.plte;
-    f.h = d.h; f.w = d.w; f.ct = d.color_type; f.bpp = bytes_per_pixel(d.color_type);
+    f.h = d.h; f.w = d.w; f.ct = d.color_type; f.bpp = bytes_per_pixel(d.color_type, mode);
     status[i] = decode_host(f, mode, lut ? lut : ident);
   }
   return LEDB200_OK;

@@ -38,7 +38,10 @@ SYMBOLS = [
     'ledb200_postprocess', 'ledb200_slide_accumulate', 'ledb200_slide_finalize', 'ledb200_slide_merge', 'ledb200_stack_pad',
     'ledb200_tta_merge', 'ledb200_crop_select', 'ledb200_train_augment', 'ledb200_view_resize',
     'ledb200_png_bound', 'ledb200_png_workspace_bytes', 'ledb200_png_encode',
+    'ledb200_png_lut_bound', 'ledb200_png_encode_lut',
     'ledb200_png_decode_workspace_bytes', 'ledb200_png_decode', 'ledb200_png_decode_host',
+    'ledb200_png_decode_mode_workspace_bytes',
+    'ledb200_cityscapes_out_ints', 'ledb200_cityscapes_workspace_bytes', 'ledb200_cityscapes_accumulate',
     'ledb200_jpeg_decode_workspace_bytes', 'ledb200_jpeg_decode', 'ledb200_jpeg_decode_host',
     'ledb200_seam_param_floats', 'ledb200_seam_workspace_bytes', 'ledb200_seam_forward',
     'ledb200_conv_layer_create', 'ledb200_conv_layer_forward', 'ledb200_conv_layer_destroy',
@@ -87,7 +90,7 @@ class PngFile(C.Structure):
                 ('color_type', C.c_int32)]
 
 
-PNG_COLOR, PNG_LABEL = 0, 1
+PNG_COLOR, PNG_LABEL, PNG_GREY16 = 0, 1, 16
 # ledb200_png_decode's per-file status codes (include/ledb200.h LEDB200_PNG_*)
 PNG_STATUS = {
     1: 'signature or IHDR does not match the descriptor',
@@ -102,6 +105,15 @@ PNG_STATUS = {
     9: 'wrong number of decompressed bytes for the image size',
     10: 'Adler-32 mismatch of the decompressed data',
     11: 'invalid scanline filter type',
+}
+
+
+# ledb200_cityscapes_accumulate's per-image status bits (include/ledb200.h)
+CITYSCAPES_STATUS = {
+    1: 'a ground-truth labelId above 33 (unknown label)',
+    2: 'a predicted labelId outside 0 .. 33 (unknown label)',
+    4: 'an instance id whose class is not an instance class of the evaluation (cityscapesscripts raises KeyError)',
+    8: 'an int64 prediction outside 0 .. 255',
 }
 
 
@@ -236,6 +248,16 @@ def get():
     lib.ledb200_png_workspace_bytes.argtypes = [i32, i32, i32]
     lib.ledb200_png_workspace_bytes.restype = i64
     lib.ledb200_png_encode.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp]
+    lib.ledb200_png_lut_bound.argtypes = [i32, i32, i32]
+    lib.ledb200_png_lut_bound.restype = i64
+    lib.ledb200_png_encode_lut.argtypes = [vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp]
+    lib.ledb200_png_decode_mode_workspace_bytes.argtypes = [C.POINTER(PngFile), i32, i32]
+    lib.ledb200_png_decode_mode_workspace_bytes.restype = i64
+    lib.ledb200_cityscapes_out_ints.argtypes = [i32]
+    lib.ledb200_cityscapes_out_ints.restype = i64
+    lib.ledb200_cityscapes_workspace_bytes.argtypes = [i32]
+    lib.ledb200_cityscapes_workspace_bytes.restype = i64
+    lib.ledb200_cityscapes_accumulate.argtypes = [vp, i32, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.ledb200_png_decode_workspace_bytes.argtypes = [C.POINTER(PngFile), i32]
     lib.ledb200_png_decode_workspace_bytes.restype = i64
     lib.ledb200_png_decode.argtypes = [C.POINTER(PngFile), i32, i32, vp, vp, vp, vp]

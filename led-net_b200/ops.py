@@ -352,12 +352,16 @@ def view_resize(imgs, resized_hw, out=None, out_flip=None, swap_rb=False, mean=N
     return out, out_flip
 
 
-def png_encode(labels, add=0):
+def png_encode(labels, add=0, lut=None, palette=False):
     """Label maps -> PNG files on the device: labels [H,W], [1,H,W] or [N,H,W], CUDA uint8 or int64.  Returns N `bytes`,
     each an 8-bit grayscale PNG of (label + add) mod 256 (add 0 or 1: mmseg's reduce_zero_label), which decodes to the
-    pixels of `Image.fromarray((label + add).astype(np.uint8))`.  One launch sequence, then two copies back: the offsets
-    and the files."""
+    pixels of `Image.fromarray((label + add).astype(np.uint8))`.  With `lut` (256 values in 0 .. 255) the pixels are
+    lut[label mod 256] instead; `add` and `lut` do not go together.  palette=True writes a palette file (colour type 3)
+    with PIL's 256-entry grey palette, what `Image.fromarray(x).convert('P').save(f)` writes: the same pixel values, read
+    back in mode 'P'.  One launch sequence, then two copies back: the offsets and the files."""
     _need_cuda(labels)
+    if lut is not None and add:
+        raise L.LedB200Error('png_encode: give either add or lut, not both')
     if labels.dtype not in (torch.uint8, torch.int64):
         raise L.LedB200Error('png_encode: labels must be uint8 or int64')
     if labels.dim() == 2:
@@ -367,16 +371,81 @@ def png_encode(labels, add=0):
     labels = labels.contiguous()
     N, H, W = labels.shape
     lib, dev = L.get(), labels.device
-    bound = L.check(lib.ledb200_png_bound(H, W), 'ledb200_png_bound')
+    table = None
+    if lut is not None:
+        lut = np.asarray(lut)
+        if lut.shape != (256,) or lut.min() < 0 or lut.max() > 255:
+            raise L.LedB200Error('png_encode: lut must hold 256 values in 0 .. 255')
+        table = (C.c_uint8 * 256)(*lut.astype(np.uint8).tolist())
+    bound = L.check(lib.ledb200_png_lut_bound(H, W, int(bool(palette))), 'ledb200_png_lut_bound')
     ws = torch.empty(L.check(lib.ledb200_png_workspace_bytes(N, H, W), 'ledb200_png_workspace_bytes'),
                      dtype=torch.uint8, device=dev)
     out = torch.empty(N * bound, dtype=torch.uint8, device=dev)
     offsets = torch.empty(N + 1, dtype=torch.int64, device=dev)
-    L.check(lib.ledb200_png_encode(_p(labels), L.torch_dtype_code(labels), N, H, W, int(add), _p(out), _p(offsets),
-                                   _p(ws), L.stream_ptr(dev)), 'ledb200_png_encode')
+    if table is None and not palette:
+        L.check(lib.ledb200_png_encode(_p(labels), L.torch_dtype_code(labels), N, H, W, int(add), _p(out), _p(offsets),
+                                       _p(ws), L.stream_ptr(dev)), 'ledb200_png_encode')
+    else:
+        if table is None:
+            if add not in (0, 1):
+                raise L.LedB200Error('png_encode: add must be 0 or 1')
+            table = (C.c_uint8 * 256)(*[(i + int(add)) & 255 for i in range(256)])
+        L.check(lib.ledb200_png_encode_lut(_p(labels), L.torch_dtype_code(labels), N, H, W, table, int(bool(palette)),
+                                           _p(out), _p(offsets), _p(ws), L.stream_ptr(dev)), 'ledb200_png_encode_lut')
     offs = offsets.cpu().tolist()
     data = out[:offs[-1]].cpu().numpy().tobytes()
     return [data[offs[i]:offs[i + 1]] for i in range(N)]
+
+
+CITYSCAPES_RECORDS_PER_COPY = 256   # records per image fetched with the statuses; a batch with more costs a second copy
+
+
+def cityscapes_accumulate(pred, gt, inst, train_to_id, category, inst_rule, cm=None, cm_last=None):
+    """cityscapesscripts' evaluatePair statistics for N same-shape images in one call (csrc/cityscapes.cu).
+
+    pred [N,H,W] (or [H,W]) uint8 / int64 trainIds, gt uint8 labelIds, inst int32 instanceIds, all CUDA.  Tables:
+    train_to_id (256 labelIds), category (34 instance categories, -1 none), inst_rule (34: 0 error, 1 skip, 2 count).
+    cm: int64 [34, 34] CUDA matrix accumulated (allocated when None); cm_last: when given, receives the matrix of the
+    batch's last image alone.  Returns (cm, statuses, records): statuses an int32 numpy [N] of LEDB200 bit flags
+    (lib.CITYSCAPES_STATUS), records one int64 numpy [k, 4] per image of (instId, size, tp, catTp) in ascending instId.
+    One small copy brings statuses, counts and records back (a second one when a batch holds more than
+    CITYSCAPES_RECORDS_PER_COPY instances per image)."""
+    _need_cuda(pred, gt, inst, cm, cm_last)
+    if pred.dim() == 2:
+        pred, gt, inst = pred[None], gt[None], inst[None]
+    if pred.dtype not in (torch.uint8, torch.int64) or gt.dtype != torch.uint8 or inst.dtype != torch.int32:
+        raise L.LedB200Error('cityscapes_accumulate: predictions uint8 / int64, labelIds uint8, instanceIds int32')
+    if pred.dim() != 3 or pred.shape != gt.shape or pred.shape != inst.shape:
+        raise L.LedB200Error(f'cityscapes_accumulate: shapes differ ({tuple(pred.shape)}, {tuple(gt.shape)}, '
+                             f'{tuple(inst.shape)})')
+    pred, gt, inst = pred.contiguous(), gt.contiguous(), inst.contiguous()
+    N, H, W = pred.shape
+    dev, lib = pred.device, L.get()
+    if cm is None:
+        cm = torch.zeros((34, 34), dtype=torch.int64, device=dev)
+    assert cm.dtype == torch.int64 and cm.is_contiguous() and cm.numel() == 34 * 34
+    if cm_last is not None:
+        assert cm_last.dtype == torch.int64 and cm_last.is_contiguous() and cm_last.numel() == 34 * 34
+    out = torch.empty(L.check(lib.ledb200_cityscapes_out_ints(N), 'ledb200_cityscapes_out_ints'), dtype=torch.int32,
+                      device=dev)
+    ws = torch.empty(L.check(lib.ledb200_cityscapes_workspace_bytes(N), 'ledb200_cityscapes_workspace_bytes'),
+                     dtype=torch.uint8, device=dev)
+    t2i = (C.c_int32 * 256)(*[int(v) for v in train_to_id])
+    cat = (C.c_int8 * 34)(*[int(v) for v in category])
+    rule = (C.c_int8 * 34)(*[int(v) for v in inst_rule])
+    L.check(lib.ledb200_cityscapes_accumulate(_p(pred), L.torch_dtype_code(pred), _p(gt), _p(inst), N, H, W, t2i, cat,
+                                              rule, _p(cm), _p(cm_last), _p(out), _p(ws), L.stream_ptr(dev)),
+            'ledb200_cityscapes_accumulate')
+    cap = N * CITYSCAPES_RECORDS_PER_COPY
+    head = out[:2 * N + 4 * cap].cpu().numpy()
+    statuses, counts = head[:N].copy(), head[N:2 * N].astype(np.int64)
+    total = int(counts.sum())
+    rec = head[2 * N:2 * N + 4 * min(total, cap)]
+    if total > cap:
+        rec = np.concatenate([rec, out[2 * N + 4 * cap:2 * N + 4 * total].cpu().numpy()])
+    rec = rec.astype(np.int64).reshape(-1, 4)
+    ends = np.cumsum(counts)
+    return cm, statuses, [rec[e - c:e] for c, e in zip(counts, ends)]
 
 
 PNG_SIGNATURE = b'\x89PNG\r\n\x1a\n'
@@ -395,8 +464,9 @@ def _head(f, n):
 def png_info(f, kind='color'):
     """(h, w, colour type) from the IHDR of a PNG file (bytes-like or 1-D uint8 tensor), which sits at a fixed offset
     after the signature.  Checks the signature, the IHDR's length, name and CRC, and the sizes; a malformed header raises
-    LedB200Error, a valid PNG outside what png_decode supports raises NotImplementedError: bit depths other than 8,
-    interlaced (Adam7) files and, for kind='label', colour types 2 / 4 / 6."""
+    LedB200Error, a valid PNG outside what png_decode supports raises NotImplementedError: bit depths other than 8
+    (kind 'color' and 'label') or 16 (kind 'grey16'), interlaced (Adam7) files, for kind='label' colour types 2 / 4 / 6
+    and for kind='grey16' every colour type but 0."""
     b = _head(f, 33)
     if len(b) < 33 or b[:8] != PNG_SIGNATURE:
         raise L.LedB200Error('not a PNG file (no PNG signature)')
@@ -410,8 +480,11 @@ def png_info(f, kind='color'):
     if ct not in (0, 2, 3, 4, 6) or depth not in (1, 2, 4, 8, 16) or comp or filt or interlace > 1:
         raise L.LedB200Error(f'IHDR: invalid header (bit depth {depth}, colour type {ct}, compression {comp}, '
                              f'filter {filt}, interlace {interlace})')
-    if depth != 8:
-        raise NotImplementedError(f'{depth}-bit PNG files (png_decode reads bit depth 8)')
+    if kind == 'grey16':
+        if depth != 16 or ct != 0:
+            raise NotImplementedError(f'{depth}-bit PNG files of colour type {ct} as grey16 (16-bit grey only)')
+    elif depth != 8:
+        raise NotImplementedError(f'{depth}-bit PNG files (png_decode reads bit depth 8, 16 for kind grey16)')
     if interlace:
         raise NotImplementedError('interlaced (Adam7) PNG files')
     if kind == 'label' and ct not in (0, 3):
@@ -443,9 +516,9 @@ def label_lut(reduce_zero_label=False, label_map=None):
     return v
 
 
-def _decode_files(files, names, infos, ch, device, who, launch, status_names):
+def _decode_files(files, names, infos, ch, device, who, launch, status_names, dtype=torch.uint8):
     """The host side shared by png_decode and jpeg_decode: files (bytes-like or 1-D uint8 tensors, host or device) are
-    staged, the host ones packed into one pinned buffer and uploaded with one copy; one [ch, h, w] uint8 output per
+    staged, the host ones packed into one pinned buffer and uploaded with one copy; one [ch, h, w] output of `dtype` per
     file (infos[i] starts with h, w) is carved from one allocation; launch(arr_args) runs the decode call, given the
     device copies of the files, their sizes and the outputs, and returns the int32 status tensor, read back with one
     copy.  A file with a non-zero status raises LedB200Error naming it and status_names' reason."""
@@ -478,7 +551,7 @@ def _decode_files(files, names, infos, ch, device, who, launch, status_names):
         if data[i] is None:
             data[i] = f.to(dev).contiguous()
     numel = [ch * info[0] * info[1] for info in infos]
-    flat = torch.empty(sum(numel), dtype=torch.uint8, device=dev)
+    flat = torch.empty(sum(numel), dtype=dtype, device=dev)
     outs, at = [], 0
     for info, m in zip(infos, numel):
         outs.append(flat[at:at + m].view(ch, info[0], info[1]))
@@ -511,11 +584,13 @@ def png_decode(files, kind='color', reduce_zero_label=False, label_map=None, nam
       (what LoadImageFromFile gives): grey replicated, palettes expanded, alpha dropped, ancillary chunks ignored.
     kind='label': grey or palette files; each result is [1, h, w], the stored values (palette indices, not colours: what
       np.array(Image.open(f)) gives) through label_lut(reduce_zero_label, label_map), as LoadAnnotations gives them.
+    kind='grey16': 16-bit grey files only (Cityscapes' *_instanceIds.png); each result is [1, h, w] int32, the values
+      np.array(Image.open(f)) gives.
     The host reads each IHDR (png_info), packs the host files into one pinned buffer and uploads it with one copy; one
     decode call covers every file and one small copy brings the statuses back.  A file that fails raises LedB200Error
     naming it (names[i], default 'file i') and the reason."""
-    if kind not in ('color', 'label'):
-        raise ValueError(f"kind must be 'color' or 'label', not {kind!r}")
+    if kind not in ('color', 'label', 'grey16'):
+        raise ValueError(f"kind must be 'color', 'label' or 'grey16', not {kind!r}")
     files = list(files)
     n = len(files)
     if n == 0:
@@ -528,17 +603,18 @@ def png_decode(files, kind='color', reduce_zero_label=False, label_map=None, nam
         for d, t, o, (h, w, ct), sz in zip(arr, data, outs, infos, sizes):
             d.data, d.size, d.out, d.h, d.w, d.color_type = t.data_ptr(), sz, o.data_ptr(), h, w, ct
         lib = L.get()
-        ws = torch.empty(max(1, L.check(lib.ledb200_png_decode_workspace_bytes(arr, n),
-                                        'ledb200_png_decode_workspace_bytes')), dtype=torch.uint8, device=dev)
+        mode = {'color': L.PNG_COLOR, 'label': L.PNG_LABEL, 'grey16': L.PNG_GREY16}[kind]
+        ws = torch.empty(max(1, L.check(lib.ledb200_png_decode_mode_workspace_bytes(arr, n, mode),
+                                        'ledb200_png_decode_mode_workspace_bytes')), dtype=torch.uint8, device=dev)
         status = torch.empty(n, dtype=torch.int32, device=dev)
         lut = None
         if kind == 'label':
             lut = (C.c_uint8 * 256)(*label_lut(reduce_zero_label, label_map).tolist())
-        L.check(lib.ledb200_png_decode(arr, n, L.PNG_LABEL if kind == 'label' else L.PNG_COLOR, lut, _p(ws),
-                                       _p(status), L.stream_ptr(dev)), 'ledb200_png_decode')
+        L.check(lib.ledb200_png_decode(arr, n, mode, lut, _p(ws), _p(status), L.stream_ptr(dev)), 'ledb200_png_decode')
         return status
 
-    return _decode_files(files, names, infos, 3 if kind == 'color' else 1, device, 'png_decode', launch, L.PNG_STATUS)
+    return _decode_files(files, names, infos, 3 if kind == 'color' else 1, device, 'png_decode', launch, L.PNG_STATUS,
+                         torch.int32 if kind == 'grey16' else torch.uint8)
 
 
 JPEG_SOI = b'\xff\xd8'
