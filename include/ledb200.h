@@ -533,7 +533,11 @@ int ledb200_view_resize(const ledb200_view_desc* views, int32_t n, int32_t Hp, i
  *   (i + add) & 255).  palette 1 writes colour type 3 and, before the IDAT, the 256-entry grey PLTE (entry i = (i, i, i))
  *   that PIL's Image.convert('P') gives a grayscale image (CityscapesMetric's labelId files); out then holds
  *   N * ledb200_png_lut_bound(H, W, 1) bytes.
- * ledb200_png_lut_bound: ledb200_png_bound plus the PLTE chunk when palette is 1. */
+ * ledb200_png_lut_bound: ledb200_png_bound plus the PLTE chunk when palette is 1.
+ * ledb200_png_encode_rgb: rgb [N,H,W,3] uint8 contiguous (device) -> 8-bit RGB files (colour type 2), the drawn
+ *   pictures of SegLocalVisualizer.  Each scanline takes the filter (None, Sub, Up, Average, Paeth) with the least sum
+ *   of |signed residual| (libpng's heuristic).  ledb200_png_rgb_bound / ledb200_png_rgb_workspace_bytes size it; out
+ *   and offsets as for ledb200_png_encode. */
 int64_t ledb200_png_bound(int32_t H, int32_t W);
 int64_t ledb200_png_lut_bound(int32_t H, int32_t W, int32_t palette);
 int64_t ledb200_png_workspace_bytes(int32_t N, int32_t H, int32_t W);
@@ -541,6 +545,37 @@ int ledb200_png_encode(const void* labels, int32_t dtype, int32_t N, int32_t H, 
                        int64_t* offsets, void* workspace, void* stream);
 int ledb200_png_encode_lut(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, const uint8_t* lut,
                            int32_t palette, uint8_t* out, int64_t* offsets, void* workspace, void* stream);
+int64_t ledb200_png_rgb_bound(int32_t H, int32_t W);
+int64_t ledb200_png_rgb_workspace_bytes(int32_t N, int32_t H, int32_t W);
+int ledb200_png_encode_rgb(const uint8_t* rgb, int32_t N, int32_t H, int32_t W, uint8_t* out, int64_t* offsets,
+                           void* workspace, void* stream);
+
+/* ---- segmentation overlays (csrc/visualize.cu) ---------------------------------------------------------------------------
+ * mmseg's SegLocalVisualizer._draw_sem_seg on the device.
+ * ledb200_seg_label_locations: labels [N,H,W] (LEDB200_U8 | LEDB200_I64, device, contiguous), 1 <= K <= 255.  out: device
+ *   int32 [N,K,3] = (present, x, y) per class k < K: the row holding the most pixels of k (the first on a tie) and the
+ *   pixel at index count / 2 of that row in x order (mmseg's _get_center_loc); (0, 0, 0) for an absent class.  Labels
+ *   outside 0 .. K - 1 are not counted.  workspace: device, ledb200_seg_locate_workspace_bytes(N, H, K).
+ * ledb200_seg_overlay: images [N,3,H,W] uint8 BGR (the decoders' layout), gt / pred [N,H,W] label maps of their own
+ *   dtype (LEDB200_U8 | LEDB200_I64) or NULL (not both).  out [N,H,P*W,3] uint8 RGB, P = the number of non-NULL maps,
+ *   gt panel first.  Pixel (y, x) of a panel is table[i * 256 + c] per channel, i the image's channel and c: the colour
+ *   of the last stamp of that panel touching the pixel, else palette[label] for 0 <= label < K, else 0.  palette: device
+ *   K x 3 RGB; table: device 256 x 256 (the caller's blend, e.g. uint8(i * (1 - alpha) + c * alpha) in float64).
+ *   stamps: device array of num_stamps descriptors, drawn in array order; stamp_data: device bytes, 4 per stamp pixel
+ *   (R, G, B, touched), row-major over the stamp's w x h box, stamp_bytes in all.  A descriptor whose box leaves its
+ *   panel, the batch or stamp_data is skipped. */
+typedef struct {
+  int32_t image, panel;       /* batch index, panel 0 .. P - 1 */
+  int32_t x0, y0, w, h;       /* the box in panel coordinates */
+  int64_t offset;             /* byte offset of the box's pixels in stamp_data */
+} ledb200_seg_stamp;
+int64_t ledb200_seg_locate_workspace_bytes(int32_t N, int32_t H, int32_t K);
+int ledb200_seg_label_locations(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, int32_t K,
+                                int32_t* out, void* workspace, void* stream);
+int ledb200_seg_overlay(const uint8_t* images, const void* gt, int32_t gt_dtype, const void* pred, int32_t pred_dtype,
+                        int32_t N, int32_t H, int32_t W, int32_t K, const uint8_t* palette, const uint8_t* table,
+                        const ledb200_seg_stamp* stamps, int32_t num_stamps, const uint8_t* stamp_data,
+                        int64_t stamp_bytes, uint8_t* out, void* stream);
 
 /* ---- PNG files -> decoded images and label maps (csrc/png_decode.cu) -----------------------------------------------------
  * The dataset feed of LoadImageFromFile (mmcv imfrombytes, cv2 backend, flag 'color') and LoadAnnotations (pillow backend,

@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, 'csrc')
 OUT = os.path.join(HERE, 'libledb200.so')
 SOURCES = ['engine.cu', 'api.cu', 'packed_conv.cu', 'conv_direct.cu', 'conv_tc.cu', 'ladder_tc.cu', 'dappm.cu', 'stem_tc.cu', 'elementwise.cu', 'tail.cu',
            'metrics.cu', 'ohem.cu', 'train.cu', 'wgrad_tc.cu', 'sesp.cu', 'mfaf.cu', 'getb.cu', 'postprocess.cu', 'seam.cu', 'glue.cu', 'augment.cu', 'png.cu',
-           'png_decode.cu', 'jpeg_decode.cu', 'cityscapes.cu']
+           'png_decode.cu', 'jpeg_decode.cu', 'cityscapes.cu', 'visualize.cu']
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
          '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr', '-Xptxas', '-v']

@@ -1,16 +1,21 @@
-// Label maps -> PNG files on the device (IoUMetric's output_dir / format_only, mmseg's `tools/test.py --out`).
+// Label maps and drawn pictures -> PNG files on the device (IoUMetric's output_dir / format_only, mmseg's
+// `tools/test.py --out` and `--show-dir`).
 //
-// Every image becomes an 8-bit PNG (no interlace) whose pixels are lut[label & 255]: (label + add) mod 256 for
+// A label map becomes an 8-bit PNG (no interlace) whose pixels are lut[label & 255]: (label + add) mod 256 for
 // IoUMetric, what `Image.fromarray((pred + reduce_zero_label).astype(np.uint8))` saves, or CityscapesMetric's trainId ->
 // labelId table.  The file is the signature, IHDR, one IDAT holding one zlib stream (header 78 01, deflate, big-endian
 // Adler-32) and IEND: grayscale (colour type 0), or with `palette` colour type 3 and, before the IDAT, the 256-entry grey
-// PLTE that PIL's `.convert('P')` writes for a grayscale image.  Every scanline has filter type 0.
+// PLTE that PIL's `.convert('P')` writes for a grayscale image.  Every scanline of these has filter type 0.  An RGB image
+// ([H,W,3] uint8, SegLocalVisualizer's pictures) becomes colour type 2, each scanline with the filter libpng's heuristic
+// picks.  S = C * W + 1 is the bytes of one filtered scanline (C = 1 or 3 bytes per pixel).
 //
 //  * png_filter_kernel   : the filtered scanline stream (a 0 filter byte, then W pixels, per row) into the workspace.
-//  * png_band_kernel     : one warp per band of R rows (R * (W + 1) <= 65535 bytes where a row allows it).  The band is
+//  * png_filter_rgb_kernel : the same for RGB rows, each with the filter whose residuals have the least sum of
+//      |signed byte| (None, Sub, Up, Average, Paeth; the first on a tie).
+//  * png_band_kernel     : one warp per band of R rows (R * S <= 65535 bytes where a row allows it).  The band is
 //      one dynamic-Huffman deflate block, or stored blocks when that is smaller.  Matches take the longer of distance 1
-//      (a run) and W + 1 (the pixel one row up) when W + 1 <= 32768; they may reach back into the previous band, since
-//      the image is one zlib stream.  The warp first writes two bitmaps of the band (byte equals the byte 1 / W + 1
+//      (a run) and S (the byte one row up) when S <= 32768; they may reach back into the previous band, since
+//      the image is one zlib stream.  The warp first writes two bitmaps of the band (byte equals the byte 1 / S
 //      back), so a match length is a search for the next clear bit, a few words per 258 bytes.  The greedy parse is split over the 32 lanes: lane k parses from where lane k - 1's
 //      last match ended, found by re-parsing until no lane's start moves (lane k's start is final after k + 1 rounds,
 //      typically two in all), so the tokens are exactly those of one sequential greedy parse of the band.  The parse
@@ -48,9 +53,9 @@ struct Plan {
 
 __host__ __device__ inline int64_t stored_bytes(int64_t L) { return L + 5 * ((L + kStoredMax - 1) / kStoredMax); }
 
-Plan make_plan(int N, int H, int W) {
+Plan make_plan(int N, int H, int W, int C) {
   Plan p;
-  p.S = (int64_t)W + 1;
+  p.S = (int64_t)C * W + 1;
   p.n = (int64_t)H * p.S;
   p.R = std::max<int64_t>(1, std::min<int64_t>(H, kStoredMax / p.S));
   p.nb = (H + p.R - 1) / p.R;
@@ -82,6 +87,75 @@ __global__ void __launch_bounds__(256) png_filter_kernel(const T* __restrict__ l
   uint8_t* dst = raw + row * S;
   for (int c = threadIdx.x; c <= W; c += blockDim.x)
     dst[c] = c == 0 ? (uint8_t)0 : tab[(uint8_t)src[c - 1]];
+}
+
+// libpng's filter heuristic: the residual byte v costs min(v, 256 - v), its magnitude as a signed byte
+__device__ __forceinline__ uint32_t sad(uint32_t v) { v &= 255u; return v < 128u ? v : 256u - v; }
+
+__device__ __forceinline__ uint32_t paeth(int a, int b, int c) {
+  const int p = a + b - c, pa = abs(p - a), pb = abs(p - b), pc = abs(p - c);
+  return (uint32_t)(pa <= pb && pa <= pc ? a : pb <= pc ? b : c);
+}
+
+// residual of byte j (j >= 0) of a row under filter f, x the byte, a / b / c the bytes left, up and up-left
+__device__ __forceinline__ uint32_t residual(int f, uint32_t x, uint32_t a, uint32_t b, uint32_t c) {
+  switch (f) {
+    case 0: return x;
+    case 1: return x - a;
+    case 2: return x - b;
+    case 3: return x - ((a + b) >> 1);
+    default: return x - paeth((int)a, (int)b, (int)c);
+  }
+}
+
+// One block per row of rgb [N*H, W*3]: the five filters' costs, a block reduction, then the chosen filter's row.
+__global__ void __launch_bounds__(256) png_filter_rgb_kernel(const uint8_t* __restrict__ rgb, int H, int W, int64_t S,
+                                                            uint8_t* __restrict__ raw) {
+  __shared__ unsigned long long part[8][5];
+  __shared__ int best_s;
+  const int64_t row = blockIdx.x;
+  const int64_t B = 3 * (int64_t)W;
+  const uint8_t* cur = rgb + row * B;
+  const uint8_t* up = row % H ? cur - B : nullptr;
+  auto bytes = [&](int64_t j, uint32_t& x, uint32_t& a, uint32_t& b, uint32_t& c) {
+    x = cur[j];
+    a = j >= 3 ? cur[j - 3] : 0u;
+    b = up ? up[j] : 0u;
+    c = up && j >= 3 ? up[j - 3] : 0u;
+  };
+  unsigned long long cost[5] = {0, 0, 0, 0, 0};
+  for (int64_t j = threadIdx.x; j < B; j += blockDim.x) {
+    uint32_t x, a, b, c;
+    bytes(j, x, a, b, c);
+#pragma unroll
+    for (int f = 0; f < 5; ++f) cost[f] += sad(residual(f, x, a, b, c));
+  }
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+  for (int f = 0; f < 5; ++f) {
+    for (int o = 16; o; o >>= 1) cost[f] += __shfl_xor_sync(0xffffffffu, cost[f], o);
+    if (lane == 0) part[wid][f] = cost[f];
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int best = 0;
+    unsigned long long mins = 0;
+    for (int f = 0; f < 5; ++f) {
+      unsigned long long s = 0;
+      for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += part[w][f];
+      if (f == 0 || s < mins) { mins = s; best = f; }
+    }
+    best_s = best;
+  }
+  __syncthreads();
+  const int f = best_s;
+  uint8_t* dst = raw + row * S;
+  if (threadIdx.x == 0) dst[0] = (uint8_t)f;
+  for (int64_t j = threadIdx.x; j < B; j += blockDim.x) {
+    uint32_t x, a, b, c;
+    bytes(j, x, a, b, c);
+    dst[1 + j] = (uint8_t)residual(f, x, a, b, c);
+  }
 }
 
 // ---- deflate symbols -------------------------------------------------------------------------------------------------
@@ -511,8 +585,8 @@ __device__ __forceinline__ void put_be32(uint8_t* p, uint32_t v) {
   p[0] = (uint8_t)(v >> 24); p[1] = (uint8_t)(v >> 16); p[2] = (uint8_t)(v >> 8); p[3] = (uint8_t)v;
 }
 
-// palette_crc: the CRC-32 of the grey PLTE chunk (type and data), 0 for a grayscale file
-__global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W, uint32_t palette_crc,
+// palette_crc: the CRC-32 of the grey PLTE chunk (type and data), 0 for a file without one
+__global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W, int color_type, uint32_t palette_crc,
                                                            const uint8_t* __restrict__ slots,
                                                            const int64_t* __restrict__ info,
                                                            const uint32_t* __restrict__ adler,
@@ -546,8 +620,8 @@ __global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W,
     put_be32(h, 13);
     h[4] = 'I'; h[5] = 'H'; h[6] = 'D'; h[7] = 'R';
     put_be32(h + 8, (uint32_t)W); put_be32(h + 12, (uint32_t)H);
-    // bit depth 8, grayscale (0) or palette (3), deflate, filter 0, no interlace
-    h[16] = 8; h[17] = pre ? 3 : 0; h[18] = 0; h[19] = 0; h[20] = 0;
+    // bit depth 8, grayscale (0), RGB (2) or palette (3), deflate, filter method 0, no interlace
+    h[16] = 8; h[17] = (uint8_t)color_type; h[18] = 0; h[19] = 0; h[20] = 0;
     put_be32(h + 21, ~crc_update(tab, 0xffffffffu, h + 4, 17));
     uint8_t* d = f + 33;
     put_be32(d, (uint32_t)idat_len);
@@ -583,6 +657,31 @@ __global__ void __launch_bounds__(256) png_assemble_kernel(Plan p, int H, int W,
   if (t == 0) put_be32(f + 37 + clen, crc_s[0]);
 }
 
+// Everything after the filter kernel, which the caller has launched into the workspace.
+int encode_filtered(const Plan& p, int N, int H, int W, int color_type, uint32_t palette_crc, uint8_t* out,
+                    int64_t* offsets, uint8_t* ws, cudaStream_t st) {
+  uint8_t* slots = ws + p.slot_off;
+  int64_t* info = (int64_t*)(ws + p.info_off);
+  uint32_t* adler = (uint32_t*)(ws + p.adler_off);
+  png_band_kernel<<<(unsigned)(N * p.nb), 32, 0, st>>>(ws, p, slots, info, (uint32_t*)(ws + p.bm_off));
+  LEDB_LAUNCH_OK("png_band_kernel");
+  png_size_kernel<<<(unsigned)N, 32, 0, st>>>(p, palette_crc ? kPlteChunk : 0, info, offsets, adler);
+  LEDB_LAUNCH_OK("png_size_kernel");
+  png_scan_kernel<<<1, 1024, 0, st>>>(offsets, N);
+  LEDB_LAUNCH_OK("png_scan_kernel");
+  png_assemble_kernel<<<(unsigned)N, 256, 0, st>>>(p, H, W, color_type, palette_crc, slots, info, adler, offsets, out);
+  LEDB_LAUNCH_OK("png_assemble_kernel");
+  return LEDB200_OK;
+}
+
+int64_t checked_bound(int32_t H, int32_t W, int C, const char* who) {
+  if (H < 1 || W < 1) return fail(LEDB200_EINVAL, std::string(who) + ": H and W must be at least 1");
+  const int64_t b = bound_of(make_plan(1, H, W, C));
+  if (b - 8 - 25 - 12 - 12 > INT32_MAX)
+    return fail(LEDB200_EINVAL, std::string(who) + ": the image is too large for one IDAT chunk");
+  return b;
+}
+
 }  // namespace
 }  // namespace ledb
 
@@ -590,12 +689,9 @@ using namespace ledb;
 
 extern "C" {
 
-int64_t ledb200_png_bound(int32_t H, int32_t W) {
-  if (H < 1 || W < 1) return fail(LEDB200_EINVAL, "png_bound: H and W must be at least 1");
-  const int64_t b = bound_of(make_plan(1, H, W));
-  if (b - 8 - 25 - 12 - 12 > INT32_MAX) return fail(LEDB200_EINVAL, "png_bound: the image is too large for one IDAT chunk");
-  return b;
-}
+int64_t ledb200_png_bound(int32_t H, int32_t W) { return checked_bound(H, W, 1, "png_bound"); }
+
+int64_t ledb200_png_rgb_bound(int32_t H, int32_t W) { return checked_bound(H, W, 3, "png_rgb_bound"); }
 
 int64_t ledb200_png_lut_bound(int32_t H, int32_t W, int32_t palette) {
   if (palette != 0 && palette != 1) return fail(LEDB200_EINVAL, "png_lut_bound: palette must be 0 or 1");
@@ -605,7 +701,12 @@ int64_t ledb200_png_lut_bound(int32_t H, int32_t W, int32_t palette) {
 
 int64_t ledb200_png_workspace_bytes(int32_t N, int32_t H, int32_t W) {
   if (N < 1 || H < 1 || W < 1) return fail(LEDB200_EINVAL, "png_workspace_bytes: N, H and W must be at least 1");
-  return make_plan(N, H, W).total;
+  return make_plan(N, H, W, 1).total;
+}
+
+int64_t ledb200_png_rgb_workspace_bytes(int32_t N, int32_t H, int32_t W) {
+  if (N < 1 || H < 1 || W < 1) return fail(LEDB200_EINVAL, "png_rgb_workspace_bytes: N, H and W must be at least 1");
+  return make_plan(N, H, W, 3).total;
 }
 
 int ledb200_png_encode_lut(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, const uint8_t* lut,
@@ -615,7 +716,7 @@ int ledb200_png_encode_lut(const void* labels, int32_t dtype, int32_t N, int32_t
   if (palette != 0 && palette != 1) return fail(LEDB200_EINVAL, "png_encode: palette must be 0 or 1");
   if (!labels || !lut || !out || !offsets || !workspace) return fail(LEDB200_EINVAL, "png_encode: null buffer");
   if (ledb200_png_bound(H, W) < 0) return LEDB200_EINVAL;
-  const Plan p = make_plan(N, H, W);
+  const Plan p = make_plan(N, H, W, 1);
   if ((int64_t)N * p.nb > INT32_MAX) return fail(LEDB200_EINVAL, "png_encode: too many bands in one call");
   // the grey palette's CRC is the same for every file: computed here once
   static const uint32_t palette_crc = [] {
@@ -629,22 +730,25 @@ int ledb200_png_encode_lut(const void* labels, int32_t dtype, int32_t N, int32_t
   for (int i = 0; i < 256; ++i) tab.v[i] = lut[i];
   cudaStream_t st = (cudaStream_t)stream;
   uint8_t* ws = (uint8_t*)workspace;
-  uint8_t* slots = ws + p.slot_off;
-  int64_t* info = (int64_t*)(ws + p.info_off);
-  uint32_t* adler = (uint32_t*)(ws + p.adler_off);
   const unsigned rows = (unsigned)((int64_t)N * H);
   if (dtype == LEDB200_I64) png_filter_kernel<int64_t><<<rows, 256, 0, st>>>((const int64_t*)labels, W, p.S, tab, ws);
   else png_filter_kernel<uint8_t><<<rows, 256, 0, st>>>((const uint8_t*)labels, W, p.S, tab, ws);
   LEDB_LAUNCH_OK("png_filter_kernel");
-  png_band_kernel<<<(unsigned)(N * p.nb), 32, 0, st>>>(ws, p, slots, info, (uint32_t*)(ws + p.bm_off));
-  LEDB_LAUNCH_OK("png_band_kernel");
-  png_size_kernel<<<(unsigned)N, 32, 0, st>>>(p, palette ? kPlteChunk : 0, info, offsets, adler);
-  LEDB_LAUNCH_OK("png_size_kernel");
-  png_scan_kernel<<<1, 1024, 0, st>>>(offsets, N);
-  LEDB_LAUNCH_OK("png_scan_kernel");
-  png_assemble_kernel<<<(unsigned)N, 256, 0, st>>>(p, H, W, palette ? palette_crc : 0u, slots, info, adler, offsets, out);
-  LEDB_LAUNCH_OK("png_assemble_kernel");
-  return LEDB200_OK;
+  return encode_filtered(p, N, H, W, palette ? 3 : 0, palette ? palette_crc : 0u, out, offsets, ws, st);
+}
+
+int ledb200_png_encode_rgb(const uint8_t* rgb, int32_t N, int32_t H, int32_t W, uint8_t* out, int64_t* offsets,
+                           void* workspace, void* stream) {
+  if (N < 1 || H < 1 || W < 1) return fail(LEDB200_EINVAL, "png_encode_rgb: N, H and W must be at least 1");
+  if (!rgb || !out || !offsets || !workspace) return fail(LEDB200_EINVAL, "png_encode_rgb: null buffer");
+  if (ledb200_png_rgb_bound(H, W) < 0) return LEDB200_EINVAL;
+  const Plan p = make_plan(N, H, W, 3);
+  if ((int64_t)N * p.nb > INT32_MAX) return fail(LEDB200_EINVAL, "png_encode_rgb: too many bands in one call");
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* ws = (uint8_t*)workspace;
+  png_filter_rgb_kernel<<<(unsigned)((int64_t)N * H), 256, 0, st>>>(rgb, H, W, p.S, ws);
+  LEDB_LAUNCH_OK("png_filter_rgb_kernel");
+  return encode_filtered(p, N, H, W, 2, 0u, out, offsets, ws, st);
 }
 
 int ledb200_png_encode(const void* labels, int32_t dtype, int32_t N, int32_t H, int32_t W, int32_t add, uint8_t* out,

@@ -39,6 +39,8 @@ SYMBOLS = [
     'ledb200_tta_merge', 'ledb200_crop_select', 'ledb200_train_augment', 'ledb200_view_resize',
     'ledb200_png_bound', 'ledb200_png_workspace_bytes', 'ledb200_png_encode',
     'ledb200_png_lut_bound', 'ledb200_png_encode_lut',
+    'ledb200_png_rgb_bound', 'ledb200_png_rgb_workspace_bytes', 'ledb200_png_encode_rgb',
+    'ledb200_seg_locate_workspace_bytes', 'ledb200_seg_label_locations', 'ledb200_seg_overlay',
     'ledb200_png_decode_workspace_bytes', 'ledb200_png_decode', 'ledb200_png_decode_host',
     'ledb200_png_decode_mode_workspace_bytes',
     'ledb200_cityscapes_out_ints', 'ledb200_cityscapes_workspace_bytes', 'ledb200_cityscapes_accumulate',
@@ -88,6 +90,12 @@ class PngFile(C.Structure):
     """ledb200_png_file: one PNG file (its bytes and size), its output and the IHDR's h, w and colour type."""
     _fields_ = [('data', C.c_void_p), ('size', C.c_int64), ('out', C.c_void_p), ('h', C.c_int32), ('w', C.c_int32),
                 ('color_type', C.c_int32)]
+
+
+class SegStamp(C.Structure):
+    """ledb200_seg_stamp: one label stamp's image, panel, box in panel coordinates and byte offset of its pixels."""
+    _fields_ = [('image', C.c_int32), ('panel', C.c_int32), ('x0', C.c_int32), ('y0', C.c_int32), ('w', C.c_int32),
+                ('h', C.c_int32), ('offset', C.c_int64)]
 
 
 PNG_COLOR, PNG_LABEL, PNG_GREY16 = 0, 1, 16
@@ -251,6 +259,15 @@ def get():
     lib.ledb200_png_lut_bound.argtypes = [i32, i32, i32]
     lib.ledb200_png_lut_bound.restype = i64
     lib.ledb200_png_encode_lut.argtypes = [vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp]
+    lib.ledb200_png_rgb_bound.argtypes = [i32, i32]
+    lib.ledb200_png_rgb_bound.restype = i64
+    lib.ledb200_png_rgb_workspace_bytes.argtypes = [i32, i32, i32]
+    lib.ledb200_png_rgb_workspace_bytes.restype = i64
+    lib.ledb200_png_encode_rgb.argtypes = [vp, i32, i32, i32, vp, vp, vp, vp]
+    lib.ledb200_seg_locate_workspace_bytes.argtypes = [i32, i32, i32]
+    lib.ledb200_seg_locate_workspace_bytes.restype = i64
+    lib.ledb200_seg_label_locations.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp]
+    lib.ledb200_seg_overlay.argtypes = [vp, vp, i32, vp, i32] + [i32] * 4 + [vp, vp, vp, i32, vp, i64, vp, vp]
     lib.ledb200_png_decode_mode_workspace_bytes.argtypes = [C.POINTER(PngFile), i32, i32]
     lib.ledb200_png_decode_mode_workspace_bytes.restype = i64
     lib.ledb200_cityscapes_out_ints.argtypes = [i32]

@@ -353,7 +353,11 @@ def view_resize(imgs, resized_hw, out=None, out_flip=None, swap_rb=False, mean=N
 
 
 def png_encode(labels, add=0, lut=None, palette=False):
-    """Label maps -> PNG files on the device: labels [H,W], [1,H,W] or [N,H,W], CUDA uint8 or int64.  Returns N `bytes`,
+    """Label maps or RGB images -> PNG files on the device.
+
+    A [N,H,W,3] uint8 tensor is N RGB images: each file is an 8-bit RGB PNG (colour type 2) that decodes to exactly
+    those pixels (cv2.imdecode gives them in BGR order); add / lut / palette do not apply.
+    Otherwise labels [H,W], [1,H,W] or [N,H,W], CUDA uint8 or int64.  Returns N `bytes`,
     each an 8-bit grayscale PNG of (label + add) mod 256 (add 0 or 1: mmseg's reduce_zero_label), which decodes to the
     pixels of `Image.fromarray((label + add).astype(np.uint8))`.  With `lut` (256 values in 0 .. 255) the pixels are
     lut[label mod 256] instead; `add` and `lut` do not go together.  palette=True writes a palette file (colour type 3)
@@ -362,6 +366,8 @@ def png_encode(labels, add=0, lut=None, palette=False):
     _need_cuda(labels)
     if lut is not None and add:
         raise L.LedB200Error('png_encode: give either add or lut, not both')
+    if labels.dim() == 4:
+        return _png_encode_rgb(labels, add, lut, palette)
     if labels.dtype not in (torch.uint8, torch.int64):
         raise L.LedB200Error('png_encode: labels must be uint8 or int64')
     if labels.dim() == 2:
@@ -392,9 +398,104 @@ def png_encode(labels, add=0, lut=None, palette=False):
             table = (C.c_uint8 * 256)(*[(i + int(add)) & 255 for i in range(256)])
         L.check(lib.ledb200_png_encode_lut(_p(labels), L.torch_dtype_code(labels), N, H, W, table, int(bool(palette)),
                                            _p(out), _p(offsets), _p(ws), L.stream_ptr(dev)), 'ledb200_png_encode_lut')
+    return _fetch_files(out, offsets)
+
+
+def _fetch_files(out, offsets):
     offs = offsets.cpu().tolist()
     data = out[:offs[-1]].cpu().numpy().tobytes()
-    return [data[offs[i]:offs[i + 1]] for i in range(N)]
+    return [data[offs[i]:offs[i + 1]] for i in range(len(offs) - 1)]
+
+
+def _png_encode_rgb(rgb, add, lut, palette):
+    if add or lut is not None or palette:
+        raise L.LedB200Error('png_encode: add, lut and palette apply to label maps, not to RGB images')
+    if rgb.dtype != torch.uint8 or rgb.shape[-1] != 3:
+        raise L.LedB200Error('png_encode: RGB images are [N, H, W, 3] uint8')
+    rgb = rgb.contiguous()
+    N, H, W, _ = rgb.shape
+    lib, dev = L.get(), rgb.device
+    bound = L.check(lib.ledb200_png_rgb_bound(H, W), 'ledb200_png_rgb_bound')
+    ws = torch.empty(L.check(lib.ledb200_png_rgb_workspace_bytes(N, H, W), 'ledb200_png_rgb_workspace_bytes'),
+                     dtype=torch.uint8, device=dev)
+    out = torch.empty(N * bound, dtype=torch.uint8, device=dev)
+    offsets = torch.empty(N + 1, dtype=torch.int64, device=dev)
+    L.check(lib.ledb200_png_encode_rgb(_p(rgb), N, H, W, _p(out), _p(offsets), _p(ws), L.stream_ptr(dev)),
+            'ledb200_png_encode_rgb')
+    return _fetch_files(out, offsets)
+
+
+def blend_table(alpha):
+    """The 256 x 256 uint8 table of mmseg's blend `(image * (1 - alpha) + mask * alpha).astype(np.uint8)`: entry
+    [i, c] for image value i and mask value c, computed with numpy's own float64 expression (a float32 or fused
+    multiply-add restatement truncates differently for some pairs)."""
+    v = np.arange(256, dtype=np.uint8)
+    return (v[:, None] * (1 - alpha) + v[None, :] * alpha).astype(np.uint8)
+
+
+def _label_map(t, who):
+    _need_cuda(t)
+    if t.dim() == 2:
+        t = t[None]
+    if t.dim() != 3 or t.dtype not in (torch.uint8, torch.int64):
+        raise L.LedB200Error(f'{who}: label maps are [N, H, W] (or [H, W]) uint8 or int64')
+    return t.contiguous()
+
+
+def seg_label_locations(labels, num_classes):
+    """mmseg's SegLocalVisualizer._get_center_loc for every class of N label maps in one launch sequence.
+
+    labels [N,H,W] (or [H,W]) CUDA uint8 / int64, 1 <= num_classes <= 255.  Returns int32 [N, K, 3] on the device:
+    (present, x, y) per class k < K, where y is the first row holding the most pixels of k and x the pixel at index
+    count // 2 of that row in x order; (0, 0, 0) when k is absent.  Labels outside 0 .. K - 1 are not counted."""
+    labels = _label_map(labels, 'seg_label_locations')
+    N, H, W = labels.shape
+    K = int(num_classes)
+    lib, dev = L.get(), labels.device
+    ws = torch.empty(L.check(lib.ledb200_seg_locate_workspace_bytes(N, H, K), 'ledb200_seg_locate_workspace_bytes'),
+                     dtype=torch.uint8, device=dev)
+    out = torch.empty((N, K, 3), dtype=torch.int32, device=dev)
+    L.check(lib.ledb200_seg_label_locations(_p(labels), L.torch_dtype_code(labels), N, H, W, K, _p(out), _p(ws),
+                                            L.stream_ptr(dev)), 'ledb200_seg_label_locations')
+    return out
+
+
+STAMP_DTYPE = np.dtype([('image', '<i4'), ('panel', '<i4'), ('x0', '<i4'), ('y0', '<i4'), ('w', '<i4'), ('h', '<i4'),
+                        ('offset', '<i8')])        # ledb200_seg_stamp
+
+
+def seg_overlay(images, gt, pred, palette, table, stamps=None, stamp_data=None):
+    """mmseg's _draw_sem_seg blend for N same-shape images, with the gt | pred panels side by side, in one call.
+
+    images [N,3,H,W] CUDA uint8 BGR (what the decoders give); gt / pred [N,H,W] label maps (uint8 / int64), either may
+    be None.  palette: CUDA uint8 [K, 3] RGB (K <= 255); table: CUDA uint8 [256, 256] (blend_table(alpha)).  stamps:
+    an optional CUDA tensor holding a STAMP_DTYPE array as bytes (drawn in order: the last one touching a pixel wins),
+    stamp_data its CUDA uint8 pixels, 4 bytes (R, G, B, touched) each.  Returns CUDA uint8 [N, H, P*W, 3] RGB."""
+    _need_cuda(images, palette, table, stamps, stamp_data)
+    if gt is None and pred is None:
+        raise L.LedB200Error('seg_overlay: neither a gt nor a pred label map')
+    if images.dim() != 4 or images.shape[1] != 3 or images.dtype != torch.uint8:
+        raise L.LedB200Error('seg_overlay: images are [N, 3, H, W] uint8')
+    images = images.contiguous()
+    N, _, H, W = images.shape
+    maps = [None if m is None else _label_map(m, 'seg_overlay') for m in (gt, pred)]
+    for m in maps:
+        if m is not None and tuple(m.shape) != (N, H, W):
+            raise L.LedB200Error(f'seg_overlay: a label map of {tuple(m.shape)} for images of {(N, H, W)}')
+    palette = palette.contiguous()
+    if palette.dtype != torch.uint8 or palette.dim() != 2 or palette.shape[1] != 3:
+        raise L.LedB200Error('seg_overlay: palette is [K, 3] uint8')
+    if table.dtype != torch.uint8 or table.numel() != 65536:
+        raise L.LedB200Error('seg_overlay: table is [256, 256] uint8')
+    P = sum(m is not None for m in maps)
+    out = torch.empty((N, H, P * W, 3), dtype=torch.uint8, device=images.device)
+    ns = 0 if stamps is None else stamps.numel() // STAMP_DTYPE.itemsize
+    codes = [L.torch_dtype_code(m) if m is not None else L.U8 for m in maps]
+    L.check(L.get().ledb200_seg_overlay(_p(images), _p(maps[0]), codes[0], _p(maps[1]), codes[1], N, H, W,
+                                        palette.shape[0], _p(palette), _p(table.contiguous()), _p(stamps), ns,
+                                        _p(stamp_data), 0 if stamp_data is None else stamp_data.numel(), _p(out),
+                                        L.stream_ptr(images.device)), 'ledb200_seg_overlay')
+    return out
 
 
 CITYSCAPES_RECORDS_PER_COPY = 256   # records per image fetched with the statuses; a batch with more costs a second copy

@@ -87,6 +87,11 @@ def _meta(s):
     return s.get('metainfo', s) if isinstance(s, dict) else {}
 
 
+class DecodedFiles(list):
+    """The images decode_batch decoded from a batch's files: the files' pixels by construction, so
+    SegVisualizationHook draws on them without reading the files again."""
+
+
 def decode_batch(data):
     """Decodes a batch of PackSegFiles outputs in place: data['inputs'] becomes the [3, h, w] uint8 BGR images (one
     png_decode call for the PNG images and one jpeg_decode call for the JPEG ones, back in batch order) and each
@@ -105,7 +110,7 @@ def decode_batch(data):
         if idx:
             for i, img in zip(idx, decode([inputs[i] for i in idx], names=[names[i] for i in idx])):
                 images[i] = img
-    data['inputs'] = images
+    data['inputs'] = DecodedFiles(images)
     withlab = [i for i, s in enumerate(samples or []) if isinstance(s, dict) and 'gt_seg_map_file' in s]
     if withlab:
         rzl = {bool(metas[i].get('reduce_zero_label', False)) for i in withlab}

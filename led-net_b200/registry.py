@@ -49,12 +49,14 @@ class Registry:
 MODELS = Registry('model')
 METRICS = Registry('metric')
 TRANSFORMS = Registry('transform')      # dataset pipeline steps (mmseg/registry/registry.py TRANSFORMS)
+VISUALIZERS = Registry('visualizer')    # SegLocalVisualizer (mmseg/registry/registry.py VISUALIZERS)
+HOOKS = Registry('hook')                # SegVisualizationHook (mmseg/registry/registry.py HOOKS)
 
 
 def register_into_mmseg():
     """Register the B200 modules in a real mmseg install (returns False if mmseg is absent)."""
     try:
-        from mmseg.registry import MODELS as MM, METRICS as MT, TRANSFORMS as TR
+        from mmseg.registry import MODELS as MM, METRICS as MT, TRANSFORMS as TR, VISUALIZERS as VI, HOOKS as HK
     except Exception:
         return False
     for k, v in MODELS._table.items():
@@ -63,4 +65,12 @@ def register_into_mmseg():
         MT.register_module(name=k, force=True, module=v)
     for k, v in TRANSFORMS._table.items():
         TR.register_module(name=k, force=True, module=v)
+    for k, v in VISUALIZERS._table.items():
+        VI.register_module(name=k, force=True, module=v)
+    try:                                # mmengine's runner calls every Hook method: give the hooks its base class
+        from mmengine.hooks import Hook
+    except Exception:
+        Hook = None
+    for k, v in HOOKS._table.items():
+        HK.register_module(name=k, force=True, module=type(k, (v, Hook), {}) if Hook is not None else v)
     return True
